@@ -4,6 +4,7 @@ K=4096, T=100, 7-DoF, 256^3 SDF, at 1/2/4/8 GPUs).
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path through the C ABI
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 
 A "step" is one STOMP iteration (Stomp::runSingleIteration): generate K rollouts, cost them, weight them,
 update the trajectory, cost the noise-less rollout.  One JSON line is printed by rank 0.
@@ -142,6 +143,43 @@ def broadcast_bytes(dist, payload, local):
         return payload
     from motion_planners_b200 import sharding
     return sharding.broadcast_bytes(dist, payload, 128, f"cuda:{local}")
+
+
+# what a caller of stomp_b200_run reads back after a step: the trajectory, its update and noise levels, the noise-less
+# rollout's costs, and the rollout-indexed tables of the step (probabilities as full_probabilities: with cumulative costs
+# the per-time-step table repeats that value along T)
+DUMP_TENSORS = ("parameters", "updates", "stddevs", "noiseless_state_costs", "noiseless_control_costs", "total_cost",
+                "cumulative_costs", "full_probabilities", "state_costs", "verdicts", "rollouts")
+DUMP_LIMIT_BYTES = 60 << 20          # array data; with the .npy headers the directory stays below 64 MB (64e6 bytes)
+
+
+def read_outputs(eng):
+    """The engine's DUMP_TENSORS as numpy arrays.  In rollout sharding a read-back is collective: every rank calls this,
+    and rollouts / state_costs / verdicts are the calling rank's share of the rollouts (their shapes depend on N)."""
+    return {name: eng.tensor(name) for name in DUMP_TENSORS}
+
+
+def dump_outputs(outputs, out_dir):
+    """Writes every array as out_dir/<name>.npy (float64; the 0 / 1 verdicts as float32), within DUMP_LIMIT_BYTES in all.
+    Smallest first, each array may use an equal share of what the ones before it left; one larger than that keeps a fixed
+    sample of its rows (leading two axes flattened, rows drawn with seed 0 and kept in order), so that two builds given
+    the same arguments store the same elements.  Returns {name: {"shape", "stored"}}."""
+    os.makedirs(out_dir, exist_ok=True)
+    left, info = DUMP_LIMIT_BYTES, {}
+    for i, name in enumerate(sorted(outputs, key=lambda k: outputs[k].size)):
+        a = outputs[name].astype(np.float32 if outputs[name].dtype == np.uint8 else np.float64)
+        share = left // (len(outputs) - i)
+        full_shape = list(a.shape)
+        if a.nbytes > share:
+            lead = 2 if a.ndim > 2 else 1
+            rows = a.reshape((-1,) + a.shape[lead:])
+            keep = max(1, share // (rows[0].nbytes or 1))
+            pick = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=min(keep, rows.shape[0]), replace=False))
+            a = rows[pick]
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+        left -= a.nbytes
+        info[name] = {"shape": full_shape, "stored": list(a.shape)}
+    return {name: info[name] for name in outputs}
 
 
 class L2Flusher:
@@ -358,6 +396,7 @@ def run_ours(args):
             total_ms += eng.timer_end()
             it += 1
     launches = eng.launch_count() - launches0
+    outputs = read_outputs(eng) if args.dump_outputs else None       # the last timed step's results, before anything else runs
     replays0 = eng.graph_replays()
     dist_barrier(dist, local)
     total_ms = dist_max(dist, total_ms, local)
@@ -539,6 +578,9 @@ def run_ours(args):
         "kernel_ms_per_step": {k: v[0] / args.steps for k, v in stats.items()},
         "cpu_baseline": cb,
     }
+    if outputs is not None:
+        line["dump_outputs"] = {"dir": args.dump_outputs, "what": "results of the last timed step, read from rank 0's engine",
+                                "arrays": dump_outputs(outputs, args.dump_outputs)}
     print(json.dumps(line), flush=True)
     eng.close()
 
@@ -555,7 +597,15 @@ def main():
     ap.add_argument("--reference-sample", type=int, default=1024, dest="reference_sample")
     ap.add_argument("--skip-cpu-baseline", action="store_true", dest="skip_cpu_baseline")
     ap.add_argument("--skip-c4", action="store_true", dest="skip_c4")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (64 MB at most); with "
+                         "rollout sharding (--gpus N > 1) rollouts, state_costs and verdicts hold rank 0's share of the "
+                         "rollouts, so their shapes depend on N")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

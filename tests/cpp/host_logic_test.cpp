@@ -25,8 +25,8 @@ using namespace motion_planners;
 
 int main(int argc, char** argv)
 {
-    CHECK(argc == 2);
-    const std::string test_dir = argv[1];
+    CHECK(argc == 3);
+    const std::string test_dir = argv[1], scratch = argv[2];   // scratch: a directory of this run's own for the files it writes
 
     // ---- YAML subset + StompConfig (reference HandleStompConfig.cpp:7-63, test/config/stomp.yml) ----
     YAML::Node cfg;
@@ -110,7 +110,7 @@ int main(int argc, char** argv)
         const double bc[3] = {0.02, -0.01, 0.3}, bh[3] = {0.05, 0.07, 0.3};
         robot_model::appendBoxMesh(bc, bh, box);
         CHECK(box.size() == 12u * 9u);
-        const std::string bin = "/tmp/stomp_b200_host_test_box.stl", asc = "/tmp/stomp_b200_host_test_box_ascii.stl";
+        const std::string bin = scratch + "/box.stl", asc = scratch + "/box_ascii.stl";
         {
             FILE* f = std::fopen(bin.c_str(), "wb");
             char header[80] = "solid binary box";     // a binary file that starts with "solid": recognised by its size
@@ -142,7 +142,7 @@ int main(int argc, char** argv)
             CHECK(std::fabs(from_asc[i] - (box[i] * scale[i % 3] + shift[i % 3])) < 1e-6);
         }
         std::vector<double> none;
-        CHECK(!robot_model::loadStl("/tmp/stomp_b200_no_such_file.stl", none) && none.empty());
+        CHECK(!robot_model::loadStl(scratch + "/no_such_file.stl", none) && none.empty());
         // sphere fit: slabs along the long (z) axis, every vertex covered, radii close to the slab's half diagonal
         const auto fit = robot_model::fitSpheres(box, 8, 0.0);
         CHECK(fit.size() >= 3 && fit.size() <= 8);

@@ -25,8 +25,8 @@ static base::samples::Joints joints(const std::vector<std::string>& names, const
 
 int main(int argc, char** argv)
 {
-    if (argc != 2) return 2;
-    const std::string dir = argv[1];
+    if (argc != 3) return 2;
+    const std::string dir = argv[1], scratch = argv[2];   // scratch: a directory of this run's own for the files it writes
     Config config;
     config.planner_config.robot_model_config.urdf_file = dir + "/data/iiwa_chain.urdf";
     config.planner_config.robot_model_config.planning_group_name = "manipulator";
@@ -154,7 +154,7 @@ int main(int argc, char** argv)
         std::vector<double> crate;
         const double zero[3] = {0, 0, 0}, half[3] = {0.9, 0.9, 0.9};
         robot_model::appendBoxMesh(zero, half, crate);         // a crate that swallows most of the workspace above the base
-        const std::string stl = "/tmp/stomp_b200_scene_test_crate.stl";
+        const std::string stl = scratch + "/crate.stl";
         {
             FILE* f = std::fopen(stl.c_str(), "wb");
             char header[80] = "crate"; std::fwrite(header, 1, 80, f);

@@ -21,7 +21,7 @@ def test_host_logic_cpp(tmp_path):
                     os.path.join(ROOT, "tests", "cpp", "host_logic_test.cpp"), "-o", exe,
                     "-L" + os.path.join(ROOT, "motion_planners_b200"), "-lmotion_planners_b200", "-lstomp_b200",
                     "-Wl,-rpath," + os.path.join(ROOT, "motion_planners_b200")], check=True)
-    out = subprocess.run([exe, os.path.join(ROOT, "test")], capture_output=True, text=True)
+    out = subprocess.run([exe, os.path.join(ROOT, "test"), str(tmp_path)], capture_output=True, text=True)
     assert out.returncode == 0, out.stdout + out.stderr
     for name in ("yaml_and_stomp_config", "robot_model", "meshes", "planner_api", "policy"):
         assert f"ok {name}" in out.stdout
@@ -60,7 +60,7 @@ def test_requests_by_joint_name_and_late_scene_changes(tmp_path):
                     os.path.join(ROOT, "tests", "cpp", "scene_and_request_test.cpp"), "-o", exe,
                     "-L" + os.path.join(ROOT, "motion_planners_b200"), "-lmotion_planners_b200", "-lstomp_b200",
                     "-Wl,-rpath," + os.path.join(ROOT, "motion_planners_b200")], check=True)
-    out = subprocess.run([exe, os.path.join(ROOT, "test")], capture_output=True, text=True, timeout=300)
+    out = subprocess.run([exe, os.path.join(ROOT, "test"), str(tmp_path)], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout + out.stderr
     for name in ("request_by_name", "refused_requests", "scene_change_reaches_the_validity_checks",
                  "scene_change_reaches_the_next_solve", "world_objects_meshes_octomap_grasp"):

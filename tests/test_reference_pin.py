@@ -1,11 +1,16 @@
-"""The CPU restatement (oracle/stomp_oracle.cpp) against the REFERENCE'S OWN CODE: /root/reference/src/planners/stomp/
-src/{Stomp,PolicyImprovement,CovariantMovementPrimitive,StompUtils}.cpp compiled unmodified against the Eigen / Boost
+"""The CPU restatement (oracle/stomp_oracle.cpp) against the REFERENCE'S OWN CODE: the reference project's
+src/planners/stomp/src/{Stomp,PolicyImprovement,CovariantMovementPrimitive,StompUtils}.cpp compiled unmodified against the Eigen / Boost
 stand-ins of oracle/ref/shim (oracle/ref/Makefile -> oracle/_ref/libstomp_ref.so).  Both sides are fed the same
 standard normals; every field of every rollout, the update, the parameters, the adapted noise and the noise-less
 rollout must agree to 1e-12 relative over whole solves — in practice they agree bit for bit.
 
-Runs wherever the library is (this container; the GPU box gets the prebuilt .so with the snapshot) and is skipped
-elsewhere; tests/test_golden_vectors.py holds the same comparison against committed vectors."""
+Where the reference's sources are absent, the reference's side is replayed from tests/golden/reference_pin/<test>.npz,
+which tests/golden/make_pin_golden.py records from the reference build: every value the test takes from it, including
+the unit noise L·eps the reference formed, which the oracle is then fed.  Arrays of more than FULL elements are kept as
+their shape, 64 elements at fixed positions, and their plain, position-weighted and absolute sums.  A test with neither
+the reference build nor its recording skips."""
+import os
+
 import numpy as np
 import pytest
 
@@ -13,7 +18,118 @@ from motion_planners_b200 import problems as P
 from oracle.binding import Oracle
 from oracle import ref_binding
 
-pytestmark = pytest.mark.skipif(not ref_binding.available(), reason="oracle/_ref/libstomp_ref.so needs /root/reference to build")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+RECORDINGS = os.path.join(ROOT, "tests", "golden", "reference_pin")
+LIVE = ref_binding.available()
+FULL = 256
+_RECORD = None      # {key: array} while tests/golden/make_pin_golden.py records the running test
+_CURRENT = [""]     # name of the running test
+
+
+@pytest.fixture(autouse=True)
+def _test_name(request):
+    _CURRENT[0] = request.node.name
+
+
+def _recording():
+    return os.path.join(RECORDINGS, _CURRENT[0] + ".npz")
+
+
+class _Print:
+    """What the recording keeps of a large array."""
+
+    def __init__(self, shape, sums, sample):
+        self.shape, self.sums, self.sample = tuple(int(n) for n in shape), np.asarray(sums, dtype=np.float64), sample
+
+
+def _print(a):
+    flat = a.reshape(-1)
+    rng = np.random.default_rng(flat.size)
+    weights = np.arange(1, flat.size + 1, dtype=np.float64) / flat.size
+    sums = [np.abs(flat).sum(), flat.sum(), (weights * flat).sum()]      # the absolute sum bounds the others' rounding
+    return _Print(a.shape, sums, flat[np.sort(rng.choice(flat.size, 64, replace=False))])
+
+
+def _store(key, v, out):
+    if v is None:
+        out[key + "~"] = np.zeros(0)
+    elif isinstance(v, dict):
+        for k, x in v.items():
+            _store(f"{key}.{k}", x, out)
+    elif isinstance(v, tuple):
+        for i, x in enumerate(v):
+            _store(f"{key}.{i}", x, out)
+        out[key + "()"] = np.array(len(v))
+    elif isinstance(v, np.ndarray) and v.size > FULL:
+        p = _print(v)
+        out[key + "#"] = np.concatenate([[len(p.shape)], p.shape, p.sums, p.sample])     # one entry: ndim, shape, sums, sample
+    else:
+        out[key] = np.array(v)
+
+
+def _load(key, g):
+    if key + "~" in g:
+        return None
+    if key in g:
+        return g[key][()] if g[key].ndim == 0 else g[key]
+    if key + "()" in g:
+        return tuple(_load(f"{key}.{i}", g) for i in range(int(g[key + "()"])))
+    if key + "#" in g:
+        p = g[key + "#"]
+        nd = int(p[0])
+        return _Print(p[1:1 + nd], p[1 + nd:4 + nd], p[4 + nd:])
+    names = sorted({k[len(key) + 1:].split(".")[0].rstrip("#~") for k in g.files if k.startswith(key + ".")})
+    assert names, f"{key} is not in {_recording()}: record it again with tests/golden/make_pin_golden.py"
+    return {n: _load(f"{key}.{n}", g) for n in names}
+
+
+class _Recorded:
+    """Answers the reference's calls in the order the test makes them: recorded from the reference build while
+    make_pin_golden.py runs, else replayed from the test's recording.  iterate's unit noise is kept whole: it is the
+    oracle's input."""
+
+    def __init__(self, reference=None, stored=None):
+        self.reference, self.stored, self.n = reference, stored, 0
+
+    def _call(self, name, *args):
+        key = f"{self.n:03d}.{name}"
+        self.n += 1
+        if self.stored is None:
+            v = getattr(self.reference, name)(*args)
+            if name == "iterate":
+                _RECORD[key + ".stop"], _RECORD[key + ".unit"] = np.array(v[0]), v[1]
+            else:
+                _store(key, v, _RECORD)
+            return v
+        if name == "iterate":
+            return bool(self.stored[key + ".stop"]), self.stored[key + ".unit"]
+        return _load(key, self.stored)
+
+    def __getattr__(self, name):
+        return lambda *args: self._call(name, *args)
+
+
+def _as_print(a, like):
+    return _print(a) if isinstance(like, _Print) and isinstance(a, np.ndarray) else a
+
+
+def _same(a, b, what):
+    if isinstance(a, _Print) or isinstance(b, _Print):
+        a, b = _as_print(a, b), _as_print(b, a)
+        assert a.shape == b.shape, what
+        np.testing.assert_allclose(a.sample, b.sample, rtol=RTOL, atol=0.0, err_msg=what)
+        np.testing.assert_allclose(a.sums, b.sums, rtol=0.0, atol=RTOL * 4 * max(a.sums[0], b.sums[0]), err_msg=what)
+        return
+    assert a.shape == b.shape, what
+    np.testing.assert_allclose(a, b, rtol=RTOL, atol=0.0, err_msg=what)
+
+
+def _equal(a, b):
+    if isinstance(a, _Print) or isinstance(b, _Print):
+        a, b = _as_print(a, b), _as_print(b, a)
+        return a.shape == b.shape and np.array_equal(a.sample, b.sample) and np.array_equal(a.sums, b.sums)
+    return np.array_equal(a, b)
+
 
 FIELDS = ["parameters_noise", "noise", "noise_projected", "parameters_noise_projected", "state_costs", "control_costs",
           "total_costs", "cumulative_costs", "probabilities", "full_probabilities", "full_costs", "total_cost"]
@@ -25,14 +141,17 @@ def _pair(pb, min_r, max_r, per_it, **kw):
     o = Oracle(num_time_steps=T, num_dimensions=D, min_rollouts=min_r, max_rollouts=max_r, num_rollouts_per_iteration=per_it,
                noise_stddev=pb.noise_stddev, **kw)
     o.set_problem(pb)
-    r = ref_binding.Reference(o)
+    if _RECORD is not None:
+        r = _Recorded(reference=ref_binding.Reference(o))
+    elif LIVE:
+        r = ref_binding.Reference(o)
+    elif os.path.exists(_recording()):
+        r = _Recorded(stored=np.load(_recording()))
+    else:
+        pytest.skip("needs the reference's sources (oracle/ref/Makefile) or this test's recording of them "
+                    "(tests/golden/make_pin_golden.py)")
     r.set_start_goal(pb.start, pb.goal)
     return o, r
-
-
-def _same(a, b, what):
-    assert a.shape == b.shape, what
-    np.testing.assert_allclose(a, b, rtol=RTOL, atol=0.0, err_msg=what)
 
 
 def _run(o, r, iterations, seed, scale_at=None, cumulative=True, projection=False):
@@ -55,7 +174,7 @@ def _run(o, r, iterations, seed, scale_at=None, cumulative=True, projection=Fals
         for f in FIELDS:
             a, b = r.field(f), o.field(f)
             _same(a, b, f"iteration {it}: {f}")
-            exact = exact and np.array_equal(a, b)
+            exact = exact and _equal(a, b)
         if not cumulative:
             p = o.field("probabilities")
             assert not np.all(p == p[:, :, :1]), "per-time-step mode must give time-varying probabilities"
@@ -66,9 +185,9 @@ def _run(o, r, iterations, seed, scale_at=None, cumulative=True, projection=Fals
         assert nr["valid"] == no["valid"]
         np.testing.assert_allclose(nr["total_cost"], no["total_cost"], rtol=RTOL)
         np.testing.assert_allclose(nr["best_cost"], no["best_cost"], rtol=RTOL)
-        np.testing.assert_array_equal(nr["state_costs"], no["state_costs"])
+        assert _equal(nr["state_costs"], no["state_costs"]), "noise-less state costs"
         _same(nr["control_costs"], no["control_costs"], "noise-less control costs")
-        np.testing.assert_array_equal(r.rollout_validity(), o.rollout_validity())
+        assert _equal(r.rollout_validity(), o.rollout_validity()), "rollout validity"
         assert bool(stop_r) == bool(stop_o)
         counts.append(r.num_rollouts()[0])
     fr = r.finish_solve()

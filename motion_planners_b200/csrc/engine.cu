@@ -115,8 +115,6 @@ struct stomp_b200_engine {
     SdfParams sdf;
     float* d_sdf = nullptr;
     size_t sdf_count = 0;
-    float* d_bricks = nullptr;      // bricked copy of the grid (STOMP_B200_SDF_LAYOUT=brick), else null
-    size_t brick_count = 0;
     double sdf_origin[3] = {0, 0, 0}, sdf_voxel = 0;
     CostExtras extras;              // stomp_b200_set_cost_extras; all zero: the shipped 0 / 1 state cost
     bool extras_on = false;
@@ -382,17 +380,12 @@ void resolve_self_kernel(stomp_b200_engine* e)
     for (int d = 0; d < e->robot.num_joints; ++d)      // the FP32 bands rest on a bound of the centres that unclamped prismatic values can break
         if (e->robot.joint[d].prismatic) { e->spec_self_note = "prismatic joint"; return; }
     codegen::StateKernelOptions opt = state_kernel_options(e);
-    if (!opt.fold_identity || opt.brick_sdf || opt.stage_joints) { e->spec_self_note = "state kernel options without the pair rule"; return; }
     opt.self = &e->self_structure;
     opt.no_tail = true;          // the noise-less rollout of a pair-rule engine is a launch of its own (noiseless_tail_available)
-    opt.block_threads = 128;
-    if (const char* t = std::getenv("STOMP_B200_SELF_BLOCK")) { const int v = std::atoi(t); if (v >= 32 && v <= 256 && v % 32 == 0) opt.block_threads = v; }
     // the FP32 centres of the spheres that still have partners ahead stay in registers: left alone the dual arm's walk takes
     // 228 of them (8 warps per SM); bounded to 168 (12 warps per SM) a dozen values spill
     opt.rollout_lanes = true;
-    if (const char* t = std::getenv("STOMP_B200_SELF_LANES")) opt.rollout_lanes = std::strcmp(t, "time") != 0;
-    opt.min_blocks = std::max(1, 384 / opt.block_threads);
-    if (const char* t = std::getenv("STOMP_B200_SELF_MIN_BLOCKS")) opt.min_blocks = std::max(0, std::atoi(t));
+    opt.min_blocks = 384 / codegen::kStateThreads;
     std::string err;
     e->spec_self = codegen::specialised_state_kernel(e->robot, opt, err);
     e->spec_self_note = e->spec_self ? std::string() : err;
@@ -402,11 +395,10 @@ void launch_states_self_collision(stomp_b200_engine* e, const StateKernelArgs& a
 {
     resolve_self_kernel(e);
     if (e->spec_self && sane) {
-        const unsigned bt = (unsigned)e->spec_self->block_threads;
-        unsigned blocks = (unsigned)(((size_t)grid.x * 128 + bt - 1) / bt);     // the callers size their grids for 128-thread CTAs
-        if (e->spec_self->rollout_lanes) blocks = (unsigned)((a.num_gen + 31) / 32) * (unsigned)((a.T + (int)(bt / 32) - 1) / (int)(bt / 32));
+        constexpr int tw = codegen::kStateThreads / 32;      // time steps per CTA when the lanes of a warp are rollouts
+        const unsigned blocks = e->spec_self->rollout_lanes ? (unsigned)((a.num_gen + 31) / 32) * (unsigned)((a.T + tw - 1) / tw) : grid.x;
         void* args[] = {(void*)&a, &e->robot, &e->sdf, &e->self_pairs, e->self_bands.data()};
-        (void)cudaLaunchKernel((const void*)e->spec_self->kernel, dim3(blocks, grid.y), dim3(bt), args, 0, stream);
+        (void)cudaLaunchKernel((const void*)e->spec_self->kernel, dim3(blocks, grid.y), dim3(codegen::kStateThreads), args, 0, stream);
         return;
     }
     const int S = e->robot.num_spheres;
@@ -563,26 +555,15 @@ codegen::StateKernelOptions state_kernel_options(const stomp_b200_engine* e)
     bool has_prismatic = false;
     for (int d = 0; d < e->robot.num_joints; ++d) has_prismatic = has_prismatic || e->robot.joint[d].prismatic != 0;
     opt.magic_floor = !has_prismatic && codegen::magic_floor_is_safe(e->robot, e->sdf);
-    if (const char* f = std::getenv("STOMP_B200_STATES_FLOOR")) opt.magic_floor = opt.magic_floor && std::strcmp(f, "cvt") != 0;
     opt.inside_grid = !has_prismatic && codegen::reach_is_inside_grid(e->robot, e->sdf);
-    if (const char* c = std::getenv("STOMP_B200_STATES_CLAMP")) opt.inside_grid = opt.inside_grid && std::atoi(c) == 0;
-    if (const char* b = std::getenv("STOMP_B200_STATES_MIN_BLOCKS")) opt.min_blocks = std::atoi(b);   // tuning knobs
     // links between issuing a link's gathers and comparing them.  With the static spheres out of the walk the 7-joint arm is
     // fastest comparing one link later (16.1 against 16.9 us at lag 2 and 17.7 at lag 0, C3 in the loop; 16.9 / 17.8 / 18.4
     // isolated and flushed), the 14-joint dual arm two links later (41.5 against 44.0 us at lag 1): profiles/r5s_*
     opt.compare_lag = e->robot.num_joints > 8 ? 2 : 1;
-    if (const char* l = std::getenv("STOMP_B200_STATES_LAG")) opt.compare_lag = std::max(0, std::atoi(l));
-    if (const char* j = std::getenv("STOMP_B200_STATES_STAGE")) opt.stage_joints = std::atoi(j) != 0;
     // sines / cosines ahead of the chain walk: measured neutral on the 7-joint arm (15.5 vs 15.6 us at C3), a gain on the
     // 14-joint dual arm (46.8 -> 44.0 us at C5; profiles/r3i_state_kernel_variants*.txt)
     opt.batch_sincos = e->robot.num_joints > 8 ? e->robot.num_joints : 0;
-    if (const char* bs = std::getenv("STOMP_B200_STATES_BATCH")) opt.batch_sincos = std::max(0, std::atoi(bs));
-    if (const char* fo = std::getenv("STOMP_B200_STATES_FOLD")) opt.fold_identity = std::atoi(fo) != 0;
-    opt.brick_sdf = e->sdf.bricks != nullptr && opt.fold_identity;
-    if (const char* pf = std::getenv("STOMP_B200_STATES_PREFETCH")) opt.prefetch_joints = std::atoi(pf);
     if (const char* hs = std::getenv("STOMP_B200_STATES_STATIC")) opt.hoist_static = std::atoi(hs) != 0;     // A / B: 0 walks every sphere per state
-    if (const char* x = std::getenv("STOMP_B200_STATES_PER_THREAD")) opt.states_per_thread = std::atoi(x) == 2 ? 2 : 1;
-    if (const char* t = std::getenv("STOMP_B200_STATES_BLOCK")) { const int v = std::atoi(t); if (v >= 32 && v <= 256 && v % 32 == 0) opt.block_threads = v; }
     return opt;
 }
 
@@ -635,16 +616,13 @@ void finish_state_args(const stomp_b200_engine* e, StateKernelArgs& a)
     a.static_hit = (e->spec && e->spec->static_kernel) ? e->d_static_hit : nullptr;
     const unsigned long long T = (unsigned long long)std::max(a.T, 0), n = (unsigned long long)std::max(a.num_gen, 0);
     a.t_magic = (T >= 2 && n * T * T < (1ull << 32)) ? (uint32_t)((1ull << 32) / T + 1) : 0u;
-    static const bool divide = std::getenv("STOMP_B200_STATES_DIV") && std::atoi(std::getenv("STOMP_B200_STATES_DIV")) != 0;   // A / B: the division sequence
-    if (divide) a.t_magic = 0u;
 }
 
 // the noise-less rollout as a tail of the specialised state kernel (no self-collision pairs, 0 / 1 state costs)
 bool noiseless_tail_available(stomp_b200_engine* e)
 {
     resolve_state_kernel(e);
-    static const bool allowed = !(std::getenv("STOMP_B200_NL_TAIL") && std::strcmp(std::getenv("STOMP_B200_NL_TAIL"), "0") == 0);
-    return allowed && e->spec != nullptr && e->self_pairs.n == 0 && !e->extras_on;
+    return e->spec != nullptr && e->self_pairs.n == 0 && !e->extras_on;
 }
 
 void fill_noiseless_tail(const stomp_b200_engine* e, const LoopParams& lp, double* record, NoiselessTail& nl)
@@ -674,7 +652,7 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
         fill_noiseless_tail(e, lp, e->nl_sums2[e->nl_parity], a.nl);
         finish_state_args(e, a);
         void* args[] = {&a, &e->robot, &e->sdf};
-        const int bt = e->spec->block_threads;
+        constexpr int bt = codegen::kStateThreads;
         // at a join (the caller waits) the tail follows the update kernel on the main stream: as a programmatic dependent its
         // CTAs are resident and waiting when the update kernel's last CTA retires (bit 3 of STOMP_B200_PDL)
         if (on_main_stream) CUDA_TRY(e, launch_dependent(e, 3, (const void*)e->spec->kernel, dim3((lp.T + bt - 1) / bt, e->Q), dim3(bt), 0, st, args));
@@ -706,7 +684,7 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
         a.rollouts = lp.theta_all + kPad; a.state_costs = lp.nl_state; a.verdicts = lp.nl_verdict; a.validity = lp.nl_valid;
         a.sums = nullptr; a.s_compact = nullptr; a.stop = lp.stop; a.tile_counter = nullptr; a.timeline = nullptr;
         a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.num_gen = 1; a.gen_offset = 0;
-        a.honour_stop = lp.honour_stop; a.debug_skip = 0;
+        a.honour_stop = lp.honour_stop;
         a.row_stride = lp.N; a.rollout_stride = (int64_t)lp.D * lp.N;
         finish_state_args(e, a);
         if (e->self_pairs.n > 0) {
@@ -715,7 +693,7 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
             e->launch_count++;
         } else {
             void* args[] = {&a, &e->robot, &e->sdf};
-            const int bt = e->spec->block_threads;
+            constexpr int bt = codegen::kStateThreads;
             CUDA_TRY(e, cudaLaunchKernel((const void*)e->spec->kernel, dim3((lp.T + bt - 1) / bt, e->Q), dim3(bt), args, 0, nl_stream));
             e->launch_count++;
         }
@@ -825,8 +803,6 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     {
         const bool fuse_weights_ahead = e->fuse_weights_allowed && (world == 1 || peer) && !e->profiling && !e->reuse_possible && reused == 0 && c.use_cumulative_costs == 1;
         lp.noise_from_rollouts = (fused_rows && fuse_weights_ahead && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
-        static const bool lean_allowed = !(std::getenv("STOMP_B200_LEAN_NOISE") && std::strcmp(std::getenv("STOMP_B200_LEAN_NOISE"), "0") == 0);
-        if (!lean_allowed) lp.noise_from_rollouts = 0;
     }
     if (banded) {
         if (int rc = (mode == kNoisePhilox ? launch_sample_banded<true>(e, lp, fused_rows) : launch_sample_banded<false>(e, lp, fused_rows))) return rc;
@@ -845,9 +821,8 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     // ---- control costs + n^T R n of the generated rows (K5, K6) and the state costs (K4): independent of each
     // other (different columns of `sums`), both latency-bound at < 50 % occupancy -> run side by side on two
     // streams; serial on the main stream while per-kernel profiling is on ----
-    static const bool overlap_allowed = !(std::getenv("STOMP_B200_OVERLAP") && std::strcmp(std::getenv("STOMP_B200_OVERLAP"), "0") == 0);
     const bool rows_needed = !(fused_rows && !lp.control_costs);      // the fused sampler already left C_d and n^T R n
-    const bool overlap_rows = overlap_allowed && !e->profiling && e->rows_stream != nullptr && rows_needed;
+    const bool overlap_rows = !e->profiling && e->rows_stream != nullptr && rows_needed;
     cudaStream_t rows_stream = overlap_rows ? e->rows_stream : e->stream;
     if (overlap_rows) {
         CUDA_TRY(e, cudaEventRecord(e->ev_sampled, e->stream));
@@ -864,8 +839,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
                 for (int j = 0; j < rl.st_n; ++j) taps5 = taps5 && rl.st_off[j] > -3 && rl.st_off[j] < 3;
                 const bool rb4 = rl.rband_halfwidth <= 4;
                 const dim3 grid((rows + 7) / 8, e->Q);
-                static const bool tile_allowed = !(std::getenv("STOMP_B200_ROWS") && std::strcmp(std::getenv("STOMP_B200_ROWS"), "fast") == 0);
-                if (taps5 && rb4 && tile_allowed && launch_rows_tile(e, rl, rows, rows_stream, overlap_rows)) {
+                if (taps5 && rb4 && launch_rows_tile(e, rl, rows, rows_stream, overlap_rows)) {
                     // launched
                 } else if (taps5 && rb4) control_rows_fast_kernel<true, true><<<grid, 256, 0, rows_stream>>>(rl);
                 else control_rows_fast_kernel<false, false><<<grid, 256, 0, rows_stream>>>(rl);
@@ -915,7 +889,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
         a.sums = lp.sums; a.s_compact = lp.s_compact; a.stop = lp.stop; a.tile_counter = lp.tile_counter;
         a.timeline = lp.timeline ? lp.timeline + 2 * 1 : nullptr;
         a.T = lp.T; a.D = lp.D; a.slots = lp.slots; a.gslots = lp.gslots; a.sumw = lp.sumw; a.num_gen = lp.num_gen;
-        a.gen_offset = lp.gen_offset; a.honour_stop = lp.honour_stop; a.debug_skip = lp.debug_skip;
+        a.gen_offset = lp.gen_offset; a.honour_stop = lp.honour_stop;
         a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
         if (tail_in_state_kernel) fill_noiseless_tail(e, lp, lp.nl_sums, a.nl);
         finish_state_args(e, a);
@@ -923,9 +897,8 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
             launch_states_self_collision(e, a, dim3((states + 127) / 128, e->Q), e->stream);
         } else if (e->spec) {
             void* args[] = {&a, &e->robot, &e->sdf};
-            const int bt = e->spec->block_threads;
-            const int per_thread = e->spec->states_per_thread;
-            const int blocks = ((states + per_thread - 1) / per_thread + bt - 1) / bt + (tail_in_state_kernel ? (e->T + bt - 1) / bt : 0);    // main CTAs, then the tail's
+            constexpr int bt = codegen::kStateThreads;
+            const int blocks = (states + bt - 1) / bt + (tail_in_state_kernel ? (e->T + bt - 1) / bt : 0);    // main CTAs, then the tail's
             CUDA_TRY(e, launch_dependent(e, 1, (const void*)e->spec->kernel, dim3(blocks, e->Q), dim3(bt), 0, e->stream, args));
         } else if (e->robot.simple_chain) rollout_states_kernel<true><<<grid, 256, 0, e->stream>>>(lp, e->robot, e->sdf);
         else rollout_states_kernel<false><<<grid, 256, 0, e->stream>>>(lp, e->robot, e->sdf);
@@ -1450,11 +1423,6 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
     b.use_noise_adaptation = cfg->use_noise_adaptation;
     b.seed = cfg->seed;
     b.noiseless_slot = -1;
-#ifdef STOMP_B200_DEBUG_KNOBS      // measurement builds only: lets the cost kernels skip their work
-#ifdef STOMP_B200_DEBUG_KNOBS     // measurement builds only (add -DSTOMP_B200_DEBUG_KNOBS to NVFLAGS): a shipped library never skips work
-    if (const char* dbg = std::getenv("STOMP_B200_DEBUG_SKIP")) b.debug_skip = std::atoi(dbg);
-#endif
-#endif
 
     double* tmp = nullptr;
     CREATE_TRY(dev_alloc(e, &b.theta_all, Q * D * N));
@@ -1531,7 +1499,6 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
         e->num_sms = prop.multiProcessorCount;
         int chunk = 128;
         while (chunk > 32 && (long long)((S + chunk / 2 - 1) / (chunk / 2)) * (long long)D * (long long)Q <= 3LL * e->num_sms) chunk /= 2;
-        if (const char* ck = std::getenv("STOMP_B200_CHUNK")) { const int v = std::atoi(ck); if (v == 32 || v == 64 || v == 128) chunk = v; }
         b.chunk = chunk;
     }
     e->max_chunks = (int)((S + b.chunk - 1) / b.chunk);
@@ -1637,7 +1604,6 @@ int stomp_b200_destroy(stomp_b200_engine* e)
     if (e->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(e->comm);
     for (void* p : e->allocations) cudaFree(p);
     if (e->d_sdf) cudaFree(e->d_sdf);
-    if (e->d_bricks) cudaFree(e->d_bricks);
     for (void* p : e->self_pair_buffers) cudaFree(p);
     if (e->eval_theta) cudaFree(e->eval_theta);
     if (e->eval_cost) cudaFree(e->eval_cost);
@@ -1938,25 +1904,6 @@ static int adopt_sdf_geometry(stomp_b200_engine* e, const int32_t dims[3], const
     return STOMP_B200_OK;
 }
 
-// STOMP_B200_SDF_LAYOUT=brick: a second copy of the finished grid in 4 x 4 x 2 bricks for the specialised state kernel
-static int build_sdf_bricks(stomp_b200_engine* e)
-{
-    e->sdf.bricks = nullptr;
-    const char* layout = std::getenv("STOMP_B200_SDF_LAYOUT");
-    if (!layout || std::strcmp(layout, "brick") != 0) return STOMP_B200_OK;
-    const int nbx = (e->sdf.nx + 3) / 4, nby = (e->sdf.ny + 3) / 4, nbz = (e->sdf.nz + 1) / 2;
-    const size_t count = (size_t)nbx * nby * nbz * 32;
-    if (e->d_bricks && e->brick_count != count) { cudaFree(e->d_bricks); e->d_bricks = nullptr; }
-    if (!e->d_bricks) { CUDA_TRY(e, cudaMalloc(&e->d_bricks, count * sizeof(float))); e->brick_count = count; }
-    brick_sdf_kernel<<<(unsigned)((count + 255) / 256), 256, 0, e->stream>>>(e->d_sdf, e->d_bricks, e->sdf.nx, e->sdf.ny, e->sdf.nz, nbx, nby, count);
-    e->launch_count++;
-    if (int rc = check_launch(e, "brick_sdf_kernel")) return rc;
-    CUDA_TRY(e, cudaStreamSynchronize(e->stream));
-    e->sdf.bricks = e->d_bricks; e->sdf.nbx = nbx; e->sdf.nby = nby;
-    e->spec_resolved = false;
-    return STOMP_B200_OK;
-}
-
 int stomp_b200_set_sdf(stomp_b200_engine* e, const int32_t dims[3], const double origin[3], double voxel_size, const float* grid)
 {
     if (!e || !dims || !origin || !grid || !(voxel_size > 0.0)) return STOMP_B200_ERR_INVALID_ARGUMENT;
@@ -1964,7 +1911,7 @@ int stomp_b200_set_sdf(stomp_b200_engine* e, const int32_t dims[3], const double
     if (int rc = adopt_sdf_geometry(e, dims, origin, voxel_size)) return rc;
     CUDA_TRY(e, cudaMemcpy(e->d_sdf, grid, e->sdf_count * sizeof(float), cudaMemcpyHostToDevice));
     e->have_sdf = true;
-    return build_sdf_bricks(e);
+    return STOMP_B200_OK;
 }
 
 int stomp_b200_build_sdf_primitives(stomp_b200_engine* e, const int32_t dims[3], const double origin[3], double voxel_size,
@@ -1998,7 +1945,7 @@ int stomp_b200_build_sdf_primitives(stomp_b200_engine* e, const int32_t dims[3],
     cudaFree(d_list);
     if (err != cudaSuccess) { e->last_error = std::string("build_sdf_primitives: ") + cudaGetErrorString(err); return STOMP_B200_ERR_CUDA; }
     e->have_sdf = true;
-    return build_sdf_bricks(e);
+    return STOMP_B200_OK;
 }
 
 // exact signed Euclidean distance transform of a device occupancy grid into e->d_sdf (geometry already adopted)
@@ -2107,7 +2054,7 @@ int stomp_b200_build_sdf_scene(stomp_b200_engine* e, const int32_t dims[3], cons
     cleanup();
     if (rc) return rc;
     e->have_sdf = true;
-    return build_sdf_bricks(e);
+    return STOMP_B200_OK;
 }
 
 int stomp_b200_get_sdf(stomp_b200_engine* e, float* out, size_t count, int32_t dims_out[3], double origin_out[3], double* voxel_size_out)
@@ -2382,8 +2329,7 @@ int stomp_b200_run(stomp_b200_engine* e, int32_t first_iteration, int32_t num_it
     const bool allow_graph = num_iterations > 1;
     // the first call inside a timed region starts it: the stream is idle since stomp_b200_timer_begin, and what lies between
     // that call and this one is the caller's own time (the interpreter of bench.py), not a step's
-    static const bool region_in_run = !(std::getenv("STOMP_B200_TIMER_END") && std::strcmp(std::getenv("STOMP_B200_TIMER_END"), "host") == 0);
-    if (e->timer_armed && !e->timer_end_recorded && region_in_run) CUDA_TRY(e, cudaEventRecord(e->timer_a, e->stream));
+    if (e->timer_armed && !e->timer_end_recorded) CUDA_TRY(e, cudaEventRecord(e->timer_a, e->stream));
     for (int i = 0; i < num_iterations; ++i)
         if (int rc = iterate_async(e, first_iteration + i, kNoisePhilox, honour_stop ? 1 : 0, allow_graph)) return rc;
     if (int rc = join_side_stream(e)) return rc;
@@ -2652,14 +2598,14 @@ int stomp_b200_evaluate_states(stomp_b200_engine* e, const double* theta, int32_
         a.rollouts = d_theta; a.state_costs = d_cost; a.verdicts = d_verdict; a.validity = d_valid;
         a.sums = nullptr; a.s_compact = nullptr; a.stop = nullptr; a.tile_counter = nullptr; a.timeline = nullptr;
         a.T = num_steps; a.D = e->D; a.slots = num_trajectories; a.gslots = 1; a.sumw = 1; a.num_gen = num_trajectories;
-        a.gen_offset = 0; a.honour_stop = 0; a.debug_skip = 0;
+        a.gen_offset = 0; a.honour_stop = 0;
         a.row_stride = num_steps; a.rollout_stride = (int64_t)e->D * num_steps;
         finish_state_args(e, a);
         if (e->self_pairs.n > 0) {
             launch_states_self_collision(e, a, dim3((unsigned)((states + 127) / 128), 1), e->stream, sane);
         } else if (e->spec && sane) {
             void* args[] = {&a, &e->robot, &e->sdf};
-            const int bt = e->spec->block_threads;
+            constexpr int bt = codegen::kStateThreads;
             CUDA_TRY(e, cudaLaunchKernel((const void*)e->spec->kernel, dim3((unsigned)((states + bt - 1) / bt), 1), dim3(bt), args, 0, e->stream));
         } else {
             evaluate_states_kernel<<<(unsigned)((states + 127) / 128), 128, 0, e->stream>>>(e->robot, e->sdf, d_theta, num_trajectories, num_steps, d_cost, d_verdict, d_valid);
@@ -2832,8 +2778,7 @@ int stomp_b200_timer_end(stomp_b200_engine* e, double* elapsed_ms)
     if (int rc = join_side_stream(e)) return rc;
     // stomp_b200_run has put the end event behind its last kernel already (every call since timer_begin re-records it);
     // other call sequences (solve, iterate) end the region here
-    static const bool end_in_run = !(std::getenv("STOMP_B200_TIMER_END") && std::strcmp(std::getenv("STOMP_B200_TIMER_END"), "host") == 0);
-    if (!(e->timer_end_recorded && end_in_run)) CUDA_TRY(e, cudaEventRecord(e->timer_b, e->stream));
+    if (!e->timer_end_recorded) CUDA_TRY(e, cudaEventRecord(e->timer_b, e->stream));
     e->timer_armed = false;
     e->timer_end_recorded = false;
     CUDA_TRY(e, cudaEventSynchronize(e->timer_b));

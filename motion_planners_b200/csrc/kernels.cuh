@@ -51,7 +51,6 @@ struct LoopParams {
     double* fprob;            // [Q][gslots][D]
     double* fprob_sum;        // [Q][D]
     uint32_t* tile_counter;   // [4] work counters of sample_rollouts_dmma_kernel, one per slab of time steps
-    int32_t debug_skip;       // measurement only (STOMP_B200_DEBUG_SKIP): bit 0 skip the FK phase, bit 1 skip the control phase of the cost kernel
     unsigned long long* timeline;   // [kTimelineKernels][2] first-CTA-start / last-CTA-end %globaltimer stamps of this iteration, or null
     int32_t rband_halfwidth;  // largest o with R[t][t+o] != 0 (4 for the acceleration rule)
     int32_t r_toeplitz;       // R[t][t+o] does not depend on t (true for R built from the 7-tap rules)
@@ -1238,7 +1237,7 @@ control_rows_kernel(const __grid_constant__ LoopParams p)
     double* xs = smem + (size_t)warp * (XS + NS);   // xs[3 + i] = x_all[i]; zeros on both sides
     double* ns = xs + XS;                           // ns[t] = noise[t]; zeros beyond T
     const int row = blockIdx.x * kRowWarps + warp;
-    if (row < p.num_gen * D && !(p.debug_skip & 2)) {      // warp-uniform
+    if (row < p.num_gen * D) {      // warp-uniform
         const int k = row / D, d = row - k * D;
         const double* nz = p.rows_noise + (((size_t)q * p.slots + k) * D + d) * T;
         const double* th = p.theta_all + ((size_t)q * D + d) * N;
@@ -1383,7 +1382,7 @@ control_rows_fast_kernel(const __grid_constant__ LoopParams p)
     const int T = p.T, D = p.D, N = p.N;
     const int lane = threadIdx.x & 31;
     const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (row < p.num_gen * D && !(p.debug_skip & 2)) {      // warp-uniform
+    if (row < p.num_gen * D) {      // warp-uniform
         const int k = row / D, d = row - k * D;
         const double* nz = p.rows_noise + (((size_t)q * p.slots + k) * D + d) * T;
         const double* th = p.theta_all + ((size_t)q * D + d) * N;
@@ -1491,7 +1490,7 @@ control_rows_tile_kernel(const __grid_constant__ LoopParams p)
     const int nrows = p.num_gen * D;
     const int c0 = (blockIdx.x * kTileWarps + warp) * 8;      // first row of this warp
 
-    if (c0 < nrows && !(p.debug_skip & 2)) {
+    if (c0 < nrows) {
         // ---- stage: rows c0 .. c0+7 are contiguous in `noise` ----
         const double* src = p.rows_noise + ((size_t)q * p.slots * D + c0) * T;
         // cp.async (16 bytes, zero-filled outside the row): all ~24 copies of a lane are in flight at once.  As a
@@ -1518,7 +1517,7 @@ control_rows_tile_kernel(const __grid_constant__ LoopParams p)
     __syncwarp();
     const int r = lane >> 2, kq = lane & 3;
     const int c = c0 + r;
-    if (c0 < nrows && !(p.debug_skip & 2)) {          // warp-uniform
+    if (c0 < nrows) {          // warp-uniform
         const bool live = c < nrows;
         const int k = live ? c / D : 0, d = live ? c - k * D : 0;
         const double dtw = p.dt * p.control_cost_weight;
@@ -1646,7 +1645,7 @@ rollout_states_kernel(const __grid_constant__ LoopParams p, const __grid_constan
     TimelineScope tls(p, 1);
     const int T = p.T, D = p.D;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx < p.num_gen * T && !(p.debug_skip & 1)) {
+    if (idx < p.num_gen * T) {
         const int k = idx / T, t = idx - k * T;
         const double* xq = p.rollouts + ((size_t)q * p.slots + k) * D * T + t;
         const bool hit = state_collides<kSimple>(robot, sdf, [&](int d) { return xq[(size_t)d * T]; });
@@ -1829,7 +1828,7 @@ states_self_collision_kernel(const __grid_constant__ StateKernelArgs a, const __
     }
     const int T = a.T;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx < a.num_gen * T && !(a.debug_skip & 1)) {
+    if (idx < a.num_gen * T) {
         const int k = idx / T, t = idx - k * T;
         const double* xq = a.rollouts + ((size_t)q * a.slots + k) * a.rollout_stride + t;
         const size_t rs = (size_t)a.row_stride;

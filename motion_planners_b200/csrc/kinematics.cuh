@@ -69,11 +69,6 @@ struct SdfParams {
     int32_t wide_index;        // 1 when nx*ny*nz does not fit 31 bits
     double offx, offy, offz;   // -(origin * inv_h)
     double inv_h;
-    // optional second copy of the grid in 4 x 4 x 2-voxel bricks of 128 bytes (one L2 line per brick; measurement of
-    // DESIGN.md 4 "SDF staging", STOMP_B200_SDF_LAYOUT=brick): voxel (x, y, z) lives at
-    //   (((z >> 1) * nby + (y >> 2)) * nbx + (x >> 2)) * 32 + (z & 1) * 16 + (y & 3) * 4 + (x & 3);  null: not built
-    const float* bricks;
-    int32_t nbx, nby;
 };
 
 // Deterministic sin/cos (also run on the host for the fixed rpy rotations of stomp_b200_set_chain, so
@@ -247,18 +242,14 @@ __device__ __forceinline__ size_t sdf_index(const SdfParams& g, double cx, doubl
 // ---------------------------------------------------------------------------------------------------
 // Compile-time structured variants for the run-time specialised state kernel (state_codegen.hpp): the same
 // operations in the same order as apply_joint / sphere_centre / sdf_index above, with every structural
-// decision (axis kind, zero masks, fixed rotation, prismatic, chain restart, index width) a template
+// decision (axis kind, zero masks, fixed rotation, prismatic, index width) a template
 // argument, so that the instantiated code is straight-line and every constant a direct constant-bank operand.
 // ---------------------------------------------------------------------------------------------------
-template <int kKind>
-__device__ __forceinline__ void rotate_joint_static(Frame& f, const JointParams& j, double s, double c);
-
-// everything of a joint that comes before its rotation: chain restart, origin, fixed rotation; for a prismatic joint
-// also the translation along its axis (the joint is then complete)
-template <int kOMask, bool kFixedRot, bool kPrismatic, bool kRestart>
+// everything of a joint that comes before its rotation: origin, fixed rotation; for a prismatic joint also the translation
+// along its axis (the joint is then complete).  A chain restart is the caller's: it materialises the identity frame first.
+template <int kOMask, bool kFixedRot, bool kPrismatic>
 __device__ __forceinline__ void place_joint_static(Frame& f, const JointParams& j, double q)
 {
-    if (kRestart) frame_identity(f);
     if (kOMask & 1) { f.px = fma(f.r00, j.o[0], f.px); f.py = fma(f.r10, j.o[0], f.py); f.pz = fma(f.r20, j.o[0], f.pz); }
     if (kOMask & 2) { f.px = fma(f.r01, j.o[1], f.px); f.py = fma(f.r11, j.o[1], f.py); f.pz = fma(f.r21, j.o[1], f.pz); }
     if (kOMask & 4) { f.px = fma(f.r02, j.o[2], f.px); f.py = fma(f.r12, j.o[2], f.py); f.pz = fma(f.r22, j.o[2], f.pz); }
@@ -286,18 +277,8 @@ __device__ __forceinline__ void place_joint_static(Frame& f, const JointParams& 
     }
 }
 
-template <int kKind, int kOMask, bool kFixedRot, bool kPrismatic, bool kRestart>
-__device__ __forceinline__ void apply_joint_static(Frame& f, const JointParams& j, double q)
-{
-    place_joint_static<kOMask, kFixedRot, kPrismatic, kRestart>(f, j, q);
-    if (kPrismatic) return;
-    double s, c;
-    det_sincos(q, s, c);
-    rotate_joint_static<kKind>(f, j, s, c);
-}
-
-// the rotation of a revolute joint from the sine / cosine of its value: the tail of apply_joint_static, also called on
-// its own by the generated kernel when it evaluates all sines and cosines of a state up front (state_codegen.hpp:
+// the rotation of a revolute joint from the sine / cosine of its value (the tail of apply_joint); the generated kernel
+// evaluates the sines and cosines itself, inside each joint or a batch of joints up front (state_codegen.hpp:
 // StateKernelOptions::batch_sincos) — the same operations on the same operands either way
 template <int kKind>
 __device__ __forceinline__ void rotate_joint_static(Frame& f, const JointParams& j, double s, double c)
@@ -348,24 +329,11 @@ __device__ __forceinline__ void rotate_joint_static(Frame& f, const JointParams&
 // reach of the chain (state_codegen.hpp: magic_floor_is_safe).
 __device__ __forceinline__ int voxel_floor_magic(double v) { return __double2loint(__dadd_rd(v, 6755399441055744.0)); }
 
-// kInside: the host has proved that no sphere centre can leave the grid (state_codegen.hpp: reach_is_inside_grid), so
-// the clamps — six VIMNMX per sphere, an eighth of the kernel's instructions — are identities and are left out.
-template <bool kWide, bool kMagic, bool kInside, bool kBrick = false>
-__device__ __forceinline__ const float* voxel_of_centre(double cx, double cy, double cz, const SdfParams& g);
-
-template <int kMask, bool kWide, bool kMagic, bool kInside>
-__device__ __forceinline__ const float* sphere_voxel_static(const Frame& f, const SphereParams& sp, const SdfParams& g)
-{
-    double cx = f.px, cy = f.py, cz = f.pz;
-    if (kMask & 1) { cx = fma(f.r00, sp.l[0], cx); cy = fma(f.r10, sp.l[0], cy); cz = fma(f.r20, sp.l[0], cz); }
-    if (kMask & 2) { cx = fma(f.r01, sp.l[1], cx); cy = fma(f.r11, sp.l[1], cy); cz = fma(f.r21, sp.l[1], cz); }
-    if (kMask & 4) { cx = fma(f.r02, sp.l[2], cx); cy = fma(f.r12, sp.l[2], cy); cz = fma(f.r22, sp.l[2], cz); }
-    return voxel_of_centre<kWide, kMagic, kInside>(cx, cy, cz, g);
-}
-
-// address of the voxel under a centre (the tail of sphere_voxel_static; the generated kernel calls it directly when it
-// has formed the centre itself, state_codegen.hpp: fold_identity)
-template <bool kWide, bool kMagic, bool kInside, bool kBrick>
+// address of the voxel under a sphere centre that the generated kernel has formed itself (state_codegen.hpp:
+// FoldingEmitter::centre).  kInside: the host has proved that no sphere centre can leave the grid (state_codegen.hpp:
+// reach_is_inside_grid), so the clamps — six VIMNMX per sphere, an eighth of the kernel's instructions — are identities
+// and are left out.
+template <bool kWide, bool kMagic, bool kInside>
 __device__ __forceinline__ const float* voxel_of_centre(double cx, double cy, double cz, const SdfParams& g)
 {
     const double vx = fma(cx, g.inv_h, g.offx), vy = fma(cy, g.inv_h, g.offy), vz = fma(cz, g.inv_h, g.offz);
@@ -376,11 +344,6 @@ __device__ __forceinline__ const float* voxel_of_centre(double cx, double cy, do
         ix = min(max(ix, 0), g.nx - 1);
         iy = min(max(iy, 0), g.ny - 1);
         iz = min(max(iz, 0), g.nz - 1);
-    }
-    if (kBrick) {
-        const unsigned in = (unsigned)(((iz & 1) << 4) | ((iy & 3) << 2) | (ix & 3));
-        if (kWide) return g.bricks + ((((size_t)(iz >> 1) * (size_t)g.nby + (size_t)(iy >> 2)) * (size_t)g.nbx + (size_t)(ix >> 2)) * 32 + in);
-        return g.bricks + ((unsigned)(((iz >> 1) * g.nby + (iy >> 2)) * g.nbx + (ix >> 2)) * 32u + in);
     }
     if (kWide) return g.grid + (((size_t)iz * (size_t)g.ny + (size_t)iy) * (size_t)g.nx + (size_t)ix);
     return g.grid + (unsigned)((iz * g.ny + iy) * g.nx + ix);
@@ -432,7 +395,7 @@ struct StateKernelArgs {
     const int32_t* stop;           // [Q]
     uint32_t* tile_counter;        // [4]
     unsigned long long* timeline;  // first-start / last-end stamps of this kernel, or null
-    int32_t T, D, slots, gslots, sumw, num_gen, gen_offset, honour_stop, debug_skip;
+    int32_t T, D, slots, gslots, sumw, num_gen, gen_offset, honour_stop;
     int32_t row_stride;            // doubles between consecutive joints of one rollout (T; N for the padded policy rows)
     int64_t rollout_stride;        // doubles between consecutive rollouts (D * T)
     NoiselessTail nl;

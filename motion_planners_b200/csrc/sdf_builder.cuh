@@ -258,19 +258,4 @@ __global__ void flood_fill_kernel(uint8_t* __restrict__ occ, const uint8_t* __re
     if (i < count && !outside[i]) occ[i] = 1;
 }
 
-// copy of the grid in 4 x 4 x 2-voxel bricks (SdfParams::bricks); one thread per brick voxel, padding voxels repeat the
-// nearest grid voxel
-__global__ void brick_sdf_kernel(const float* __restrict__ grid, float* __restrict__ bricks, int nx, int ny, int nz, int nbx, int nby, size_t count)
-{
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= count) return;
-    const unsigned in = (unsigned)(i & 31);
-    size_t b = i >> 5;
-    const int bx = (int)(b % (size_t)nbx); b /= (size_t)nbx;
-    const int by = (int)(b % (size_t)nby);
-    const int bz = (int)(b / (size_t)nby);
-    const int x = min(bx * 4 + (int)(in & 3), nx - 1), y = min(by * 4 + (int)((in >> 2) & 3), ny - 1), z = min(bz * 2 + (int)(in >> 4), nz - 1);
-    bricks[i] = grid[((size_t)z * ny + y) * nx + x];
-}
-
 }  // namespace stomp_b200

@@ -6,4 +6,3 @@ python -m pytest tests/test_self_collision.py tests/test_gpu_parity.py -m gpu -x
 python tools/e2e_breakdown.py c3 60 20 8 > $O/e2e_breakdown_r4b.txt 2>&1; cat $O/e2e_breakdown_r4b.txt
 STOMP_B200_SOLVE_AHEAD=2 python tools/e2e_breakdown.py c3 60 20 8 > $O/e2e_breakdown_r4b_ahead2.txt 2>&1; head -7 $O/e2e_breakdown_r4b_ahead2.txt
 timeout 600 python tools/self_collision_cost.py > $O/self_collision_cost_r4b.json 2>&1; cat $O/self_collision_cost_r4b.json
-for B in 128 96 160 192 64; do echo "=== STATES_BLOCK=$B"; STOMP_B200_STATES_BLOCK=$B python tools/timeline.py c3 40 | grep -E "cost|period"; done > $O/state_block_variants_r4b.txt 2>&1; cat $O/state_block_variants_r4b.txt

@@ -20,10 +20,8 @@ def main():
     pairs = P.self_collision_pairs(pb.chain, pb.spheres, disabled_links=inside)
     out = {"workload": f"dual arm K={K} T={T} D=14 S=48 sdf={n}^3", "pairs": int(len(pairs))}
     none = np.zeros((0, 2), dtype=np.int32)
-    variants = [("world_only", none, {}), ("list_walk_generic_fk", pairs, {"STOMP_B200_SELF": "generic"})]
-    for lanes, bt, mb in (("rollout", 128, 3), ("time", 128, 3), ("rollout", 128, 2), ("rollout", 128, 4), ("rollout", 64, 6), ("rollout", 256, 1), ("rollout", 256, 2)):
-        variants.append((f"pair_rule_in_specialised_kernel_lanes_{lanes}_block{bt}_minblocks{mb}", pairs,
-                         {"STOMP_B200_SELF": "spec", "STOMP_B200_SELF_LANES": lanes, "STOMP_B200_SELF_BLOCK": str(bt), "STOMP_B200_SELF_MIN_BLOCKS": str(mb)}))
+    variants = [("world_only", none, {}), ("list_walk_generic_fk", pairs, {"STOMP_B200_SELF": "generic"}),
+                ("pair_rule_in_specialised_kernel", pairs, {"STOMP_B200_SELF": "spec"})]
     for label, pr, env in variants:
         os.environ.update(env)
         e = binding.engine_for_problem(pb)

@@ -41,12 +41,8 @@ int main(int argc, char** argv)
     if (getenv("LAG")) opt.compare_lag = atoi(getenv("LAG"));
     if (getenv("MINB")) opt.min_blocks = atoi(getenv("MINB"));
     if (getenv("BATCH")) opt.batch_sincos = atoi(getenv("BATCH"));
-    if (getenv("BLOCK")) opt.block_threads = atoi(getenv("BLOCK"));
-    if (getenv("FOLD")) opt.fold_identity = atoi(getenv("FOLD")) != 0;
     if (getenv("NOTAIL")) opt.no_tail = atoi(getenv("NOTAIL")) != 0;
     if (getenv("LANES")) opt.rollout_lanes = true;
-    if (getenv("SPT")) opt.states_per_thread = atoi(getenv("SPT"));
-    if (getenv("PREFETCH")) opt.prefetch_joints = atoi(getenv("PREFETCH"));
     if (getenv("STATIC")) opt.hoist_static = atoi(getenv("STATIC")) != 0;
     codegen::SelfPairStructure sp;
     if (dual && getenv("PAIRS")) {      // the sphere-pair rule inside the kernel: every sphere of the first arm (object included) against every one of the second

@@ -6,9 +6,10 @@
 //   doGenRollouts      -> [reuse_rollouts_kernel] sample_rollouts_banded_kernel (recurrence through the banded L^-1, control-cost
 //                         rows fused; draws before it waits for the previous update kernel) | sample_rollouts_dmma_kernel
 //                         (injected epsilon, factors without a band table) | sample_rollouts_kernel | shift_rollouts_kernel
-//   doExecuteRollouts  -> stomp_b200_states_specialised (generated, state_codegen.hpp; static spheres once per scene by
+//   doExecuteRollouts  -> a state pass (launch_state_pass, also for the noise-less rollout and stomp_b200_evaluate_states):
+//                         stomp_b200_states_specialised (generated, state_codegen.hpp; static spheres once per scene by
 //                         stomp_b200_static_spheres) | rollout_states_kernel; states_self_collision_kernel / the generated
-//                         pair-rule kernel with a sphere-pair list; state_cost_extras_kernel for the alternative costs
+//                         pair-rule kernel with a sphere-pair list; then state_cost_extras_kernel for the alternative costs
 //   setRolloutCosts    -> inside the sampler | control_rows_tile_kernel | control_rows_fast_kernel | control_rows_kernel
 //                         [reused_control_cost_kernel]
 //   improvePolicy + updateParameters
@@ -16,7 +17,7 @@
 //                         rollout shards | with the NCCL exchange, rollout reuse or per-kernel profiling: [allgather]
 //                         rollout_weights_kernel, weighted_update_kernel, reduce_partials_kernel, [allreduce], apply_update_kernel
 //   doNoiselessRollout -> control costs in the update kernel's last CTA per joint, the T states as a tail of the next state kernel
-//                         launch (alone at a join) | the state kernel on the T states + noiseless_rollout_kernel (side stream)
+//                         launch (alone at a join) | a state pass on the T states + noiseless_rollout_kernel (side stream)
 // The rollout bookkeeping (PolicyImprovement.cpp:170-186,304-308) is host integer arithmetic and stays here.
 #include <algorithm>
 #include <cmath>
@@ -356,14 +357,6 @@ int check_launch(stomp_b200_engine* e, const char* what)
     return 0;
 }
 
-// the state kernel with the sphere-pair rule (stomp_b200_set_self_collision), its centre storage sized to the robot
-template <int kCap>
-void launch_states_self_collision_t(stomp_b200_engine* e, const StateKernelArgs& a, dim3 grid, cudaStream_t stream)
-{
-    if (e->robot.simple_chain) states_self_collision_kernel<kCap, true><<<grid, 128, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
-    else states_self_collision_kernel<kCap, false><<<grid, 128, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
-}
-
 codegen::StateKernelOptions state_kernel_options(const stomp_b200_engine* e);
 
 // the specialised kernel with the pair rule for the pair list as it is now, or null (then states_self_collision_kernel runs)
@@ -389,22 +382,6 @@ void resolve_self_kernel(stomp_b200_engine* e)
     std::string err;
     e->spec_self = codegen::specialised_state_kernel(e->robot, opt, err);
     e->spec_self_note = e->spec_self ? std::string() : err;
-}
-
-void launch_states_self_collision(stomp_b200_engine* e, const StateKernelArgs& a, dim3 grid, cudaStream_t stream, bool sane = true)
-{
-    resolve_self_kernel(e);
-    if (e->spec_self && sane) {
-        constexpr int tw = codegen::kStateThreads / 32;      // time steps per CTA when the lanes of a warp are rollouts
-        const unsigned blocks = e->spec_self->rollout_lanes ? (unsigned)((a.num_gen + 31) / 32) * (unsigned)((a.T + tw - 1) / tw) : grid.x;
-        void* args[] = {(void*)&a, &e->robot, &e->sdf, &e->self_pairs, e->self_bands.data()};
-        (void)cudaLaunchKernel((const void*)e->spec_self->kernel, dim3(blocks, grid.y), dim3(codegen::kStateThreads), args, 0, stream);
-        return;
-    }
-    const int S = e->robot.num_spheres;
-    if (S <= 32) launch_states_self_collision_t<32>(e, a, grid, stream);
-    else if (S <= 64) launch_states_self_collision_t<64>(e, a, grid, stream);
-    else launch_states_self_collision_t<STOMP_B200_MAX_SPHERES>(e, a, grid, stream);
 }
 
 // tiles per slab: the slabs of a launch are equally wide (ceil(T / 8) n8 tiles over ceil(T / 104) slabs)
@@ -474,15 +451,17 @@ int launch_sample(stomp_b200_engine* e, const LoopParams& lp)
 
 enum NoiseMode { kNoisePhilox = 0, kNoiseUnit = 1, kNoiseEpsilon = 2 };
 
-// the control-cost operator has the shape the fused / register-window kernels are written for: one rule with taps
-// -2 .. +2, Toeplitz R of half bandwidth <= 4, even T
-bool rows_shape_is_shipped(const stomp_b200_engine* e, const LoopParams& rl)
+// which control-cost row kernels the operator's shape allows.  kRowsWindow: one rule with Toeplitz interior rows, Toeplitz R
+// (or no noise adaptation), even T and N >= 12 — the register-window kernel.  kRowsTile: besides, taps -2 .. +2 and R of half
+// bandwidth <= 4 — what the fused sampler and the tile kernel are written for.
+enum RowsShape { kRowsGeneric, kRowsWindow, kRowsTile };
+
+RowsShape rows_shape(const stomp_b200_engine* e, const LoopParams& lp)
 {
-    const bool fast = rl.st_n > 0 && rl.num_rules == 1 && (rl.r_toeplitz || !rl.use_noise_adaptation) && e->T % 2 == 0 && e->N >= 12;
-    if (!fast) return false;
-    for (int j = 0; j < rl.st_n; ++j)
-        if (!(rl.st_off[j] > -3 && rl.st_off[j] < 3)) return false;
-    return rl.rband_halfwidth <= 4;
+    if (!(lp.st_n > 0 && lp.num_rules == 1 && (lp.r_toeplitz || !lp.use_noise_adaptation) && e->T % 2 == 0 && e->N >= 12)) return kRowsGeneric;
+    for (int j = 0; j < lp.st_n; ++j)
+        if (!(lp.st_off[j] > -3 && lp.st_off[j] < 3)) return kRowsWindow;
+    return lp.rband_halfwidth <= 4 ? kRowsTile : kRowsWindow;
 }
 
 // recurrence sampler (L^-1 is banded); fuse: control-cost sums + n^T R n in the same pass
@@ -510,7 +489,7 @@ int launch_sample_banded(stomp_b200_engine* e, const LoopParams& lp, bool fuse)
 // one Stomp::runSingleIteration for all local queries, queued on the stream (no host synchronisation)
 // eight-rows-per-warp control-cost kernel (kernels.cuh): instantiated for the group counts of the usual T
 template <int kGroups>
-bool launch_rows_tile_g(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream, bool share_sm)
+bool launch_rows_tile_g(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream)
 {
     const size_t smem = sizeof(double) * (size_t)kTileWarps * 8 * tile_noise_stride(kGroups);
     const dim3 grid((rows + kTileWarps * 8 - 1) / (kTileWarps * 8), lp.Q);
@@ -527,22 +506,40 @@ bool launch_rows_tile_g(stomp_b200_engine* e, const LoopParams& lp, int rows, cu
     // (Capping this grid's residency so that it shares every SM with the state kernel was tried — 32 KB of shared memory
     // per one-warp CTA, 7 per SM — and lost: a tile's latency is ~10 us whatever runs beside it, so 3.5 waves of 7 warps
     // took 42 us.  The two kernels overlap only at their tails.)
-    (void)share_sm;
-    const size_t request = smem;
-    if (lp.control_costs) control_rows_tile_kernel<kGroups, true><<<grid, kTileWarps * 32, request, stream>>>(lp);
-    else control_rows_tile_kernel<kGroups, false><<<grid, kTileWarps * 32, request, stream>>>(lp);
+    if (lp.control_costs) control_rows_tile_kernel<kGroups, true><<<grid, kTileWarps * 32, smem, stream>>>(lp);
+    else control_rows_tile_kernel<kGroups, false><<<grid, kTileWarps * 32, smem, stream>>>(lp);
     return true;
 }
 
-bool launch_rows_tile(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream, bool share_sm)
+bool launch_rows_tile(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream)
 {
     const int g = tile_groups(lp.N);
-    if (g <= 2) return launch_rows_tile_g<2>(e, lp, rows, stream, share_sm);
-    if (g <= 4) return launch_rows_tile_g<4>(e, lp, rows, stream, share_sm);
-    if (g <= 7) return launch_rows_tile_g<7>(e, lp, rows, stream, share_sm);
-    if (g <= 11) return launch_rows_tile_g<11>(e, lp, rows, stream, share_sm);
-    if (g <= 14) return launch_rows_tile_g<14>(e, lp, rows, stream, share_sm);
+    if (g <= 2) return launch_rows_tile_g<2>(e, lp, rows, stream);
+    if (g <= 4) return launch_rows_tile_g<4>(e, lp, rows, stream);
+    if (g <= 7) return launch_rows_tile_g<7>(e, lp, rows, stream);
+    if (g <= 11) return launch_rows_tile_g<11>(e, lp, rows, stream);
+    if (g <= 14) return launch_rows_tile_g<14>(e, lp, rows, stream);
     return false;
+}
+
+// control costs + n^T R n of `rows` (rollout, joint) rows with the kernel the shape allows (the tile kernel where its shared
+// memory can be had, else the register-window kernel), then the per-time-step costs when they are kept
+int launch_rows(stomp_b200_engine* e, const LoopParams& rl, RowsShape shape, int rows, cudaStream_t stream)
+{
+    if (shape == kRowsGeneric) {
+        const size_t row_smem = sizeof(double) * (size_t)kRowWarps * (control_row_x_stride(e->N) + control_row_n_stride(e->T));
+        control_rows_kernel<<<dim3((rows + kRowWarps - 1) / kRowWarps, e->Q), kRowWarps * 32, row_smem, stream>>>(rl);
+    } else if (!(shape == kRowsTile && launch_rows_tile(e, rl, rows, stream))) {
+        const dim3 grid((rows + 7) / 8, e->Q);
+        if (shape == kRowsTile) control_rows_fast_kernel<true, true><<<grid, 256, 0, stream>>>(rl);
+        else control_rows_fast_kernel<false, false><<<grid, 256, 0, stream>>>(rl);
+    }
+    if (int rc = check_launch(e, "control_rows_kernel")) return rc;
+    if (rl.control_costs) {
+        fold_control_costs_kernel<<<dim3((rows + 127) / 128, e->Q), 128, 0, stream>>>(rl);
+        if (int rc = check_launch(e, "fold_control_costs_kernel")) return rc;
+    }
+    return 0;
 }
 
 codegen::StateKernelOptions state_kernel_options(const stomp_b200_engine* e)
@@ -610,9 +607,11 @@ void resolve_state_kernel(stomp_b200_engine* e)
 
 // the two arguments of the specialised kernel that come from the engine rather than from the loop: the verdict of the static
 // spheres, and the multiplier that replaces idx / T where the host can prove it exact (M = floor(2^32 / T) + 1 has
-// M T = 2^32 + r with 0 < r <= T, so umulhi(idx, M) = floor(idx / T + idx r / (T 2^32)) = idx / T whenever idx r < 2^32)
-void finish_state_args(const stomp_b200_engine* e, StateKernelArgs& a)
+// M T = 2^32 + r with 0 < r <= T, so umulhi(idx, M) = floor(idx / T + idx r / (T 2^32)) = idx / T whenever idx r < 2^32).
+// The static verdict exists once the state kernel is resolved, so that happens here.
+void finish_state_args(stomp_b200_engine* e, StateKernelArgs& a)
 {
+    resolve_state_kernel(e);
     a.static_hit = (e->spec && e->spec->static_kernel) ? e->d_static_hit : nullptr;
     const unsigned long long T = (unsigned long long)std::max(a.T, 0), n = (unsigned long long)std::max(a.num_gen, 0);
     a.t_magic = (T >= 2 && n * T * T < (1ull << 32)) ? (uint32_t)((1ull << 32) / T + 1) : 0u;
@@ -633,74 +632,122 @@ void fill_noiseless_tail(const stomp_b200_engine* e, const LoopParams& lp, doubl
     nl.iters = lp.iters_used; nl.stop = lp.stop; nl.counter = e->d_nl_counter; nl.note = lp.note; nl.min_cost_improvement = lp.min_cost_improvement;
 }
 
-// the state kernel on the T noise-less states + noiseless_rollout_kernel (K10 + the wrapper's stop rule) for the iteration
-// recorded in e->nl_lp, on the side stream, behind everything queued on the main stream so far
+// ---- the argument blocks of the state passes (StateKernelArgs is filled nowhere else) ----
+// the generated rollouts of an iteration; with `tail`, the noise-less rollout owed by the previous iteration rides along
+StateKernelArgs rollout_state_args(stomp_b200_engine* e, const LoopParams& lp, bool tail)
+{
+    StateKernelArgs a{};
+    a.rollouts = lp.rollouts; a.state_costs = lp.state_costs; a.verdicts = lp.verdicts; a.validity = lp.validity;
+    a.sums = lp.sums; a.s_compact = lp.s_compact; a.stop = lp.stop; a.tile_counter = lp.tile_counter;
+    a.timeline = lp.timeline ? lp.timeline + 2 * 1 : nullptr;
+    a.T = lp.T; a.D = lp.D; a.slots = lp.slots; a.gslots = lp.gslots; a.sumw = lp.sumw; a.num_gen = lp.num_gen;
+    a.gen_offset = lp.gen_offset; a.honour_stop = lp.honour_stop;
+    a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
+    if (tail) fill_noiseless_tail(e, lp, lp.nl_sums, a.nl);
+    finish_state_args(e, a);
+    return a;
+}
+
+// the T noise-less states of the iteration `lp`, read in place from the padded policy rows.  With `tail`: the tail alone (no
+// generated rollouts), which also finishes the record the next iteration reads; without: one rollout whose verdicts go to
+// nl_state / nl_verdict / nl_valid for noiseless_rollout_kernel
+StateKernelArgs noiseless_state_args(stomp_b200_engine* e, const LoopParams& lp, bool tail)
+{
+    StateKernelArgs a{};
+    a.stop = lp.stop; a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.honour_stop = lp.honour_stop;
+    if (tail) {
+        a.num_gen = 0; a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
+        fill_noiseless_tail(e, lp, e->nl_sums2[e->nl_parity], a.nl);
+    } else {
+        a.rollouts = lp.theta_all + kPad; a.state_costs = lp.nl_state; a.verdicts = lp.nl_verdict; a.validity = lp.nl_valid;
+        a.num_gen = 1; a.row_stride = lp.N; a.rollout_stride = (int64_t)lp.D * lp.N;
+    }
+    finish_state_args(e, a);
+    return a;
+}
+
+// the caller's trajectories theta [K][D][T] of stomp_b200_evaluate_states, as one query
+StateKernelArgs trajectory_state_args(stomp_b200_engine* e, const double* theta, int K, int T, double* costs, uint8_t* verdicts,
+                                      uint8_t* validity)
+{
+    StateKernelArgs a{};
+    a.rollouts = theta; a.state_costs = costs; a.verdicts = verdicts; a.validity = validity;
+    a.T = T; a.D = e->D; a.slots = K; a.gslots = 1; a.sumw = 1; a.num_gen = K;
+    a.row_stride = T; a.rollout_stride = (int64_t)e->D * T;
+    finish_state_args(e, a);
+    return a;
+}
+
+// One state pass over `queries` queries, with the kernel that serves it: while a pair list is set the generated kernel with
+// the pair rule when `sane`, else the list walk with centre storage for the robot's spheres; without one the generated
+// world-only kernel when `sane`, else the generic kernel.  `sane`: every joint value is finite with |q| <= 1e6 (the generated
+// kernels leave out clamps only such values make redundant).  The grids have codegen::kStateThreads threads per CTA; the
+// tail's CTAs come first (state_codegen.hpp).  The caller counts the launch (its profiling Scope, or the noise-less rollout's
+// category).
+int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream_t stream, int queries, int pdl_bit, bool sane)
+{
+    resolve_state_kernel(e);
+    constexpr int bt = codegen::kStateThreads;
+    const unsigned tail_blocks = a.nl.theta ? (unsigned)((a.T + bt - 1) / bt) : 0u;
+    const dim3 grid((unsigned)(((long long)a.num_gen * a.T + bt - 1) / bt) + tail_blocks, (unsigned)queries), block(bt);
+    if (e->self_pairs.n > 0) {
+        resolve_self_kernel(e);
+        if (e->spec_self && sane) {
+            constexpr int tw = bt / 32;      // time steps per CTA when the lanes of a warp are rollouts
+            const dim3 lanes_grid((unsigned)((a.num_gen + 31) / 32) * (unsigned)((a.T + tw - 1) / tw), grid.y);
+            void* args[] = {(void*)&a, &e->robot, &e->sdf, &e->self_pairs, e->self_bands.data()};
+            (void)cudaLaunchKernel((const void*)e->spec_self->kernel, e->spec_self->rollout_lanes ? lanes_grid : grid, block, args, 0, stream);
+            return check_launch(e, "stomp_b200_states_specialised (pair rule)");
+        }
+        const int S = e->robot.num_spheres;
+        auto walk = [&](auto simple_kernel, auto kernel) {
+            if (e->robot.simple_chain) simple_kernel<<<grid, block, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
+            else kernel<<<grid, block, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
+        };
+        if (S <= 32) walk(states_self_collision_kernel<32, true>, states_self_collision_kernel<32, false>);
+        else if (S <= 64) walk(states_self_collision_kernel<64, true>, states_self_collision_kernel<64, false>);
+        else walk(states_self_collision_kernel<STOMP_B200_MAX_SPHERES, true>, states_self_collision_kernel<STOMP_B200_MAX_SPHERES, false>);
+        return check_launch(e, "states_self_collision_kernel");
+    }
+    if (e->spec && sane) {
+        void* args[] = {(void*)&a, &e->robot, &e->sdf};
+        // Only this kernel may be a programmatic dependent: it is the only state kernel that executes griddepcontrol.wait.
+        // Any other, launched that way, could read the stop flag and its joint values before the kernel before it wrote them.
+        if (pdl_bit >= 0) (void)launch_dependent(e, pdl_bit, (const void*)e->spec->kernel, grid, block, 0, stream, args);
+        else (void)cudaLaunchKernel((const void*)e->spec->kernel, grid, block, args, 0, stream);
+        return check_launch(e, "stomp_b200_states_specialised");
+    }
+    if (e->robot.simple_chain) rollout_states_kernel<true><<<grid, block, 0, stream>>>(a, e->robot, e->sdf);
+    else rollout_states_kernel<false><<<grid, block, 0, stream>>>(a, e->robot, e->sdf);
+    return check_launch(e, "rollout_states_kernel");
+}
+
+// the noise-less rollout of the iteration recorded in e->nl_lp (K10 + the wrapper's stop rule): a state pass over its T states,
+// then noiseless_rollout_kernel unless the pass was the tail of the specialised kernel, which finishes the record itself.  On
+// the side stream behind everything queued on the main stream so far; on_main_stream: the caller is about to wait for the
+// result (a join), nothing is there to overlap with — queue behind the update kernel directly; the cross-stream hand-over
+// alone cost 13 us of every isolated iteration
 int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
 {
     const LoopParams& lp = e->nl_lp;
     e->nl_deferred = false;
-    if (noiseless_tail_available(e)) {
-        // the tail alone: no generated rollouts, T noise-less states; the record is the one the next iteration will read
-        cudaStream_t st = on_main_stream ? e->stream : e->side_stream;
-        if (!on_main_stream) {
-            CUDA_TRY(e, cudaEventRecord(e->ev_applied, e->stream));
-            CUDA_TRY(e, cudaStreamWaitEvent(e->side_stream, e->ev_applied, 0));
-        }
-        StateKernelArgs a{};
-        a.stop = lp.stop; a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.num_gen = 0;
-        a.honour_stop = lp.honour_stop; a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
-        fill_noiseless_tail(e, lp, e->nl_sums2[e->nl_parity], a.nl);
-        finish_state_args(e, a);
-        void* args[] = {&a, &e->robot, &e->sdf};
-        constexpr int bt = codegen::kStateThreads;
-        // at a join (the caller waits) the tail follows the update kernel on the main stream: as a programmatic dependent its
-        // CTAs are resident and waiting when the update kernel's last CTA retires (bit 3 of STOMP_B200_PDL)
-        if (on_main_stream) CUDA_TRY(e, launch_dependent(e, 3, (const void*)e->spec->kernel, dim3((lp.T + bt - 1) / bt, e->Q), dim3(bt), 0, st, args));
-        else CUDA_TRY(e, cudaLaunchKernel((const void*)e->spec->kernel, dim3((lp.T + bt - 1) / bt, e->Q), dim3(bt), args, 0, st));
-        e->launch_count++;
-        e->kernel_launches[STOMP_B200_KERNEL_APPLY]++;
-        if (!on_main_stream) {
-            CUDA_TRY(e, cudaEventRecord(e->ev_noiseless, e->side_stream));
-            e->noiseless_pending = true;
-        }
-        return 0;
-    }
-    // on_main_stream: the caller is about to wait for the result (a join), nothing is there to overlap with — queue the two
-    // kernels behind the update kernel directly; the cross-stream hand-over alone cost 13 us of every isolated iteration
-    cudaStream_t nl_stream = on_main_stream ? e->stream : e->side_stream;
+    const bool tail = noiseless_tail_available(e);     // first: resolving may queue the static-sphere kernel on the main stream
+    cudaStream_t st = on_main_stream ? e->stream : e->side_stream;
     if (!on_main_stream) {
         CUDA_TRY(e, cudaEventRecord(e->ev_applied, e->stream));
         CUDA_TRY(e, cudaStreamWaitEvent(e->side_stream, e->ev_applied, 0));
     }
-    const size_t smem = sizeof(double) * ((size_t)e->D * e->N + e->T + e->sumw);
+    // at a join the tail follows the update kernel on the main stream: as a programmatic dependent its CTAs are resident and
+    // waiting when the update kernel's last CTA retires (bit 3 of STOMP_B200_PDL)
+    if (int rc = launch_state_pass(e, noiseless_state_args(e, lp, tail), st, e->Q, tail && on_main_stream ? 3 : -1, true)) return rc;
     e->launch_count++;
     e->kernel_launches[STOMP_B200_KERNEL_APPLY]++;
-    int states_done = 0;
-    if (e->self_pairs.n > 0 || e->spec) {
-        // the verdicts of the T noise-less states from the specialised state kernel, reading the padded policy rows in
-        // place (2.5x faster than the generic FK inside noiseless_rollout_kernel, which sits at the end of every
-        // isolated iteration)
-        StateKernelArgs a{};
-        a.rollouts = lp.theta_all + kPad; a.state_costs = lp.nl_state; a.verdicts = lp.nl_verdict; a.validity = lp.nl_valid;
-        a.sums = nullptr; a.s_compact = nullptr; a.stop = lp.stop; a.tile_counter = nullptr; a.timeline = nullptr;
-        a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.num_gen = 1; a.gen_offset = 0;
-        a.honour_stop = lp.honour_stop;
-        a.row_stride = lp.N; a.rollout_stride = (int64_t)lp.D * lp.N;
-        finish_state_args(e, a);
-        if (e->self_pairs.n > 0) {
-            launch_states_self_collision(e, a, dim3((lp.T + 127) / 128, e->Q), nl_stream);
-            if (int rc = check_launch(e, "states_self_collision_kernel")) return rc;
-            e->launch_count++;
-        } else {
-            void* args[] = {&a, &e->robot, &e->sdf};
-            constexpr int bt = codegen::kStateThreads;
-            CUDA_TRY(e, cudaLaunchKernel((const void*)e->spec->kernel, dim3((lp.T + bt - 1) / bt, e->Q), dim3(bt), args, 0, nl_stream));
-            e->launch_count++;
-        }
-        states_done = 1;
+    if (!tail) {
+        const size_t smem = sizeof(double) * ((size_t)e->D * e->N + e->T + e->sumw);
+        noiseless_rollout_kernel<<<e->Q, 256, smem, st>>>(lp, e->robot, e->sdf, e->extras);
+        e->launch_count++;
+        if (int rc = check_launch(e, "noiseless_rollout_kernel")) return rc;
     }
-    noiseless_rollout_kernel<<<e->Q, 256, smem, nl_stream>>>(lp, e->robot, e->sdf, states_done, e->extras);
-    if (int rc = check_launch(e, "noiseless_rollout_kernel")) return rc;
     if (!on_main_stream) {
         CUDA_TRY(e, cudaEventRecord(e->ev_noiseless, e->side_stream));
         e->noiseless_pending = true;
@@ -794,16 +841,17 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     // epsilon goes through the contraction with the caller's L (parity mode) unless STOMP_B200_SAMPLER=banded
     const bool banded = lp.Lband != nullptr && mode != kNoiseUnit &&
                         ((mode == kNoisePhilox && (e->sampler_mode == 0 || e->sampler_mode == 3)) || (mode == kNoiseEpsilon && e->sampler_mode == 3));
-    const bool fused_rows = banded && !lp.Mproj && rows_shape_is_shipped(e, lp);
+    const RowsShape rows_kind = rows_shape(e, lp);
+    const bool fused_rows = banded && !lp.Mproj && rows_kind == kRowsTile;
     // the shipped large-K loop (fused sampler, fused weights / update kernel, nothing reads `noise` back): the noise
     // tensor is not materialised — weights_update_kernel subtracts theta from the rollout rows it streams
     // rollout sharding: both exchanges inside weights_update_peer_kernel over the peer-mapped mailboxes (every rank takes
     // the same decision: the flags involved are set alike on all ranks)
     const bool peer = world > 1 && e->peer_ready && !e->profiling && c.use_cumulative_costs == 1 && e->fuse_weights_allowed;
-    {
-        const bool fuse_weights_ahead = e->fuse_weights_allowed && (world == 1 || peer) && !e->profiling && !e->reuse_possible && reused == 0 && c.use_cumulative_costs == 1;
-        lp.noise_from_rollouts = (fused_rows && fuse_weights_ahead && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
-    }
+    // one launch for K7-K9 when nothing sits between them (no exchange, no reused rollouts, no per-kernel profiling)
+    const bool per_timestep = c.use_cumulative_costs != 1;      // 0: per-time-step costs; 2: forward cumulation (cost-to-go)
+    const bool fuse_weights = e->fuse_weights_allowed && (world == 1 || peer) && !e->profiling && !e->reuse_possible && reused == 0 && !per_timestep;
+    lp.noise_from_rollouts = (fused_rows && fuse_weights && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
     if (banded) {
         if (int rc = (mode == kNoisePhilox ? launch_sample_banded<true>(e, lp, fused_rows) : launch_sample_banded<false>(e, lp, fused_rows))) return rc;
     } else if (mode == kNoiseUnit) {
@@ -831,29 +879,6 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     {
         const int rows = gen_local * e->D;
         Scope sc(e, STOMP_B200_KERNEL_ROWS);
-        auto launch_rows = [&](const LoopParams& rl) -> int {
-            // one rule with Toeplitz interior rows, Toeplitz R, even T and 16-byte aligned rows: the register-window kernel
-            const bool fast = rl.st_n > 0 && rl.num_rules == 1 && (rl.r_toeplitz || !rl.use_noise_adaptation) && e->T % 2 == 0 && e->N >= 12;
-            if (fast) {
-                bool taps5 = true;
-                for (int j = 0; j < rl.st_n; ++j) taps5 = taps5 && rl.st_off[j] > -3 && rl.st_off[j] < 3;
-                const bool rb4 = rl.rband_halfwidth <= 4;
-                const dim3 grid((rows + 7) / 8, e->Q);
-                if (taps5 && rb4 && launch_rows_tile(e, rl, rows, rows_stream, overlap_rows)) {
-                    // launched
-                } else if (taps5 && rb4) control_rows_fast_kernel<true, true><<<grid, 256, 0, rows_stream>>>(rl);
-                else control_rows_fast_kernel<false, false><<<grid, 256, 0, rows_stream>>>(rl);
-            } else {
-                const size_t row_smem = sizeof(double) * (size_t)kRowWarps * (control_row_x_stride(e->N) + control_row_n_stride(e->T));
-                control_rows_kernel<<<dim3((rows + kRowWarps - 1) / kRowWarps, e->Q), kRowWarps * 32, row_smem, rows_stream>>>(rl);
-            }
-            if (int rc = check_launch(e, "control_rows_kernel")) return rc;
-            if (rl.control_costs) {
-                fold_control_costs_kernel<<<dim3((rows + 127) / 128, e->Q), 128, 0, rows_stream>>>(rl);
-                if (int rc = check_launch(e, "fold_control_costs_kernel")) return rc;
-            }
-            return 0;
-        };
         if (lp.Mproj) {
             // M-projection (PolicyImprovement.cpp:421-440): noise_projected_ = M * noise_ for the generated rollouts, then
             // the control costs from parameters_ + noise_projected_ (:812-817) and n^T R n from noise_ (:656-663)
@@ -861,48 +886,28 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
             e->launch_count++;
             if (int rc = check_launch(e, "project_noise_dmma_kernel")) return rc;
             LoopParams cpass = lp; cpass.rows_noise = lp.noise_proj; cpass.rows_mask = 1;
-            if (int rc = launch_rows(cpass)) return rc;
+            if (int rc = launch_rows(e, cpass, rows_kind, rows, rows_stream)) return rc;
             LoopParams qpass = lp; qpass.rows_noise = lp.noise; qpass.rows_mask = 2; qpass.control_costs = nullptr;
             e->launch_count++;
-            if (int rc = launch_rows(qpass)) return rc;
+            if (int rc = launch_rows(e, qpass, rows_kind, rows, rows_stream)) return rc;
         } else if (fused_rows) {
             // the sampler left C_d and n^T R n; only the per-time-step control costs (read-backs, per-time-step mode) are missing
             if (lp.control_costs) {
                 LoopParams store = lp; store.rows_mask = 0;
-                if (int rc = launch_rows(store)) return rc;
+                if (int rc = launch_rows(e, store, rows_kind, rows, rows_stream)) return rc;
             } else {
                 e->kernel_launches[STOMP_B200_KERNEL_ROWS]--;     // nothing launched in this scope
                 e->launch_count--;
             }
         } else {
-            if (int rc = launch_rows(lp)) return rc;
+            if (int rc = launch_rows(e, lp, rows_kind, rows, rows_stream)) return rc;
         }
     }
     if (overlap_rows) CUDA_TRY(e, cudaEventRecord(e->ev_rows, rows_stream));
     {
         const int states = gen_local * e->T;
-        dim3 grid((states + 255) / 256, e->Q);
         Scope sc(e, STOMP_B200_KERNEL_COST);
-        resolve_state_kernel(e);
-        StateKernelArgs a{};
-        a.rollouts = lp.rollouts; a.state_costs = lp.state_costs; a.verdicts = lp.verdicts; a.validity = lp.validity;
-        a.sums = lp.sums; a.s_compact = lp.s_compact; a.stop = lp.stop; a.tile_counter = lp.tile_counter;
-        a.timeline = lp.timeline ? lp.timeline + 2 * 1 : nullptr;
-        a.T = lp.T; a.D = lp.D; a.slots = lp.slots; a.gslots = lp.gslots; a.sumw = lp.sumw; a.num_gen = lp.num_gen;
-        a.gen_offset = lp.gen_offset; a.honour_stop = lp.honour_stop;
-        a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
-        if (tail_in_state_kernel) fill_noiseless_tail(e, lp, lp.nl_sums, a.nl);
-        finish_state_args(e, a);
-        if (e->self_pairs.n > 0) {
-            launch_states_self_collision(e, a, dim3((states + 127) / 128, e->Q), e->stream);
-        } else if (e->spec) {
-            void* args[] = {&a, &e->robot, &e->sdf};
-            constexpr int bt = codegen::kStateThreads;
-            const int blocks = (states + bt - 1) / bt + (tail_in_state_kernel ? (e->T + bt - 1) / bt : 0);    // main CTAs, then the tail's
-            CUDA_TRY(e, launch_dependent(e, 1, (const void*)e->spec->kernel, dim3(blocks, e->Q), dim3(bt), 0, e->stream, args));
-        } else if (e->robot.simple_chain) rollout_states_kernel<true><<<grid, 256, 0, e->stream>>>(lp, e->robot, e->sdf);
-        else rollout_states_kernel<false><<<grid, 256, 0, e->stream>>>(lp, e->robot, e->sdf);
-        if (int rc = check_launch(e, "rollout_states_kernel")) return rc;
+        if (int rc = launch_state_pass(e, rollout_state_args(e, lp, tail_in_state_kernel), e->stream, e->Q, 1, true)) return rc;
         if (e->extras_on) {     // alternative state costs: a pass of their own, then S_k in a fixed order
             state_cost_extras_kernel<<<dim3((states + 127) / 128, e->Q), 128, 0, e->stream>>>(lp, e->robot, e->sdf, e->extras);
             if (int rc = check_launch(e, "state_cost_extras_kernel")) return rc;
@@ -934,10 +939,6 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
         NCCL_TRY(e, g_nccl.AllGather(lp.sums + (size_t)c.rank * count, lp.sums, count, ncclFloat64, e->comm, e->stream));
     }
 
-    // one launch for K7-K9 when nothing sits between them (no exchange, no reused rollouts, no per-kernel profiling)
-    const bool per_timestep = c.use_cumulative_costs != 1;      // 0: per-time-step costs; 2: forward cumulation (cost-to-go)
-    const bool fuse_weights = e->fuse_weights_allowed && (world == 1 || peer) && !e->profiling && !e->reuse_possible && reused == 0 && !per_timestep;
-    if (lp.noise_from_rollouts && !fuse_weights) return fail(e, STOMP_B200_ERR_CUDA, "internal: noise not materialised but the fused update kernel is not in use");
     const int nchunks = std::max(1, (lp.num_local + lp.chunk - 1) / lp.chunk);
     lp.nchunks = nchunks;
     if (peer) {
@@ -2593,25 +2594,9 @@ int stomp_b200_evaluate_states(stomp_b200_engine* e, const double* theta, int32_
     CUDA_TRY(e, cudaMemcpyAsync(d_theta, theta, sizeof(double) * states * e->D, cudaMemcpyHostToDevice, e->stream));
     {
         Scope sc(e, STOMP_B200_KERNEL_COST);
-        resolve_state_kernel(e);
-        StateKernelArgs a{};
-        a.rollouts = d_theta; a.state_costs = d_cost; a.verdicts = d_verdict; a.validity = d_valid;
-        a.sums = nullptr; a.s_compact = nullptr; a.stop = nullptr; a.tile_counter = nullptr; a.timeline = nullptr;
-        a.T = num_steps; a.D = e->D; a.slots = num_trajectories; a.gslots = 1; a.sumw = 1; a.num_gen = num_trajectories;
-        a.gen_offset = 0; a.honour_stop = 0;
-        a.row_stride = num_steps; a.rollout_stride = (int64_t)e->D * num_steps;
-        finish_state_args(e, a);
-        if (e->self_pairs.n > 0) {
-            launch_states_self_collision(e, a, dim3((unsigned)((states + 127) / 128), 1), e->stream, sane);
-        } else if (e->spec && sane) {
-            void* args[] = {&a, &e->robot, &e->sdf};
-            constexpr int bt = codegen::kStateThreads;
-            CUDA_TRY(e, cudaLaunchKernel((const void*)e->spec->kernel, dim3((unsigned)((states + bt - 1) / bt), 1), dim3(bt), args, 0, e->stream));
-        } else {
-            evaluate_states_kernel<<<(unsigned)((states + 127) / 128), 128, 0, e->stream>>>(e->robot, e->sdf, d_theta, num_trajectories, num_steps, d_cost, d_verdict, d_valid);
-        }
+        const StateKernelArgs a = trajectory_state_args(e, d_theta, num_trajectories, num_steps, d_cost, d_verdict, d_valid);
+        if (int rc = launch_state_pass(e, a, e->stream, 1, -1, sane)) return rc;
     }
-    if (int rc = check_launch(e, "evaluate_states")) return rc;
     if (e->extras_on) {
         evaluate_extras_kernel<<<(unsigned)((states + 127) / 128), 128, 0, e->stream>>>(e->robot, e->sdf, e->extras, d_theta, num_trajectories, num_steps, d_cost);
         e->launch_count++;

@@ -165,7 +165,8 @@ __device__ __forceinline__ void pdl_trigger_and_wait()
 
 struct TimelineScope {
     unsigned long long* slot;
-    __device__ __forceinline__ TimelineScope(const LoopParams& p, int kernel) : slot(p.timeline ? p.timeline + 2 * kernel : nullptr)
+    __device__ __forceinline__ TimelineScope(const LoopParams& p, int kernel) : TimelineScope(p.timeline ? p.timeline + 2 * kernel : nullptr) {}
+    __device__ __forceinline__ explicit TimelineScope(unsigned long long* s) : slot(s)
     {
         if (slot && threadIdx.x == 0 && threadIdx.y == 0) atomicMin(slot, global_timer_ns());
     }
@@ -1634,27 +1635,30 @@ fold_control_costs_kernel(const __grid_constant__ LoopParams p)
 // gathers through the read-only path, cost / verdict written back; S_k = sum_t cost accumulated with
 // atomicAdd (the terms are 0 / 1, so the double sum is exact in any order).  This is the roofline kernel:
 // 8D + 4S + 9 algorithmic bytes per state.
+// It serves every world-only state pass the generated kernel cannot (no NVRTC, STOMP_B200_STATES=generic, joint values
+// that kernel cannot vouch for); null pointers in StateKernelArgs as in states_self_collision_kernel, no NoiselessTail.
 template <bool kSimple>
-__global__ void __launch_bounds__(256)
-rollout_states_kernel(const __grid_constant__ LoopParams p, const __grid_constant__ RobotParams robot,
+__global__ void __launch_bounds__(128)
+rollout_states_kernel(const __grid_constant__ StateKernelArgs a, const __grid_constant__ RobotParams robot,
                       const __grid_constant__ SdfParams sdf)
 {
     const int q = blockIdx.y;
-    if (blockIdx.x == 0 && q == 0 && threadIdx.x < 4) p.tile_counter[threadIdx.x] = 0u;   // for the next sampling launch
-    if (query_frozen(p, q)) return;
-    TimelineScope tls(p, 1);
-    const int T = p.T, D = p.D;
+    if (a.tile_counter && blockIdx.x == 0 && q == 0 && threadIdx.x < 4) a.tile_counter[threadIdx.x] = 0u;   // for the next sampling launch
+    if (a.honour_stop && a.stop[q] != 0) return;
+    TimelineScope tls(a.timeline);
+    const int T = a.T;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx < p.num_gen * T) {
+    if (idx < a.num_gen * T) {
         const int k = idx / T, t = idx - k * T;
-        const double* xq = p.rollouts + ((size_t)q * p.slots + k) * D * T + t;
-        const bool hit = state_collides<kSimple>(robot, sdf, [&](int d) { return xq[(size_t)d * T]; });
-        const size_t o = ((size_t)q * p.slots + k) * T + t;
-        p.state_costs[o] = hit ? 1.0 : 0.0;
-        p.verdicts[o] = hit ? 1 : 0;
-        if (t == T - 1) p.validity[(size_t)q * p.slots + k] = hit ? 0 : 1;   // last timestep only (OptimizationTask.cpp:192-202)
-        if (hit) atomicAdd(p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw, 1.0);
-        if (hit && p.s_compact) atomicAdd(p.s_compact + (size_t)q * p.gslots + (p.gen_offset + k), 1.0);
+        const double* xq = a.rollouts + ((size_t)q * a.slots + k) * a.rollout_stride + t;
+        const size_t rs = (size_t)a.row_stride;
+        const bool hit = state_collides<kSimple>(robot, sdf, [&](int d) { return xq[(size_t)d * rs]; });
+        const size_t o = ((size_t)q * a.slots + k) * T + t;
+        if (a.state_costs) a.state_costs[o] = hit ? 1.0 : 0.0;
+        if (a.verdicts) a.verdicts[o] = hit ? 1 : 0;
+        if (a.validity && t == T - 1) a.validity[(size_t)q * a.slots + k] = hit ? 0 : 1;   // last timestep only (OptimizationTask.cpp:192-202)
+        if (hit && a.sums) atomicAdd(a.sums + ((size_t)q * a.gslots + (a.gen_offset + k)) * a.sumw, 1.0);
+        if (hit && a.s_compact) atomicAdd(a.s_compact + (size_t)q * a.gslots + (a.gen_offset + k), 1.0);
     }
     tls.end();
 }
@@ -1780,31 +1784,14 @@ __device__ __forceinline__ void materialise_noiseless(const LoopParams& p, int q
         p.sums[((size_t)q * p.gslots + p.noiseless_gslot) * p.sumw + e] = p.nl_sums[(size_t)q * p.sumw + e];
 }
 
-// stand-alone verdicts for arbitrary trajectories theta [K][D][Tq] (stomp_b200_evaluate_states)
-__global__ void __launch_bounds__(128)
-evaluate_states_kernel(const __grid_constant__ RobotParams robot, const __grid_constant__ SdfParams sdf,
-                       const double* __restrict__ theta, int K, int Tq, double* __restrict__ costs,
-                       uint8_t* __restrict__ verdicts, uint8_t* __restrict__ validity)
-{
-    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= (size_t)K * Tq) return;
-    const int k = (int)(idx / Tq), t = (int)(idx - (size_t)k * Tq);
-    const int D = robot.num_joints;
-    const double* base = theta + (size_t)k * D * Tq + t;
-    const bool hit = state_collides<false>(robot, sdf, [&](int d) { return base[(size_t)d * Tq]; });
-    if (costs) costs[idx] = hit ? 1.0 : 0.0;
-    if (verdicts) verdicts[idx] = hit ? 1 : 0;
-    if (validity && t == Tq - 1) validity[k] = hit ? 0 : 1;
-}
-
 // =====================================================================================================
 // Self collision (SURVEY.md §8f rank 3: the "self" half of robot_model's isStateValid, with the SRDF's disabled
 // link pairs removed on the host — reference test/data/kuka_iiwa.srdf:46-70).  A state is in collision when a
 // link sphere is inside an obstacle (as above) OR two spheres of a listed pair overlap:
 //   |c_i - c_j|^2 < (r_i + r_j)^2,   |.|^2 = fma(dz, dz, fma(dy, dy, dx * dx)),   the limit squared on the host.
-// Replaces the state kernel (generated or generic) at all of its call sites while a pair list is set; the
-// argument block is the generated kernel's, so the noisy rollouts, the padded policy rows of the noise-less
-// rollout and stomp_b200_evaluate_states all go through this one kernel.
+// While a pair list is set, this kernel or the generated one with the pair rule serves every state pass in place of
+// the world-only kernels (engine.cu: launch_state_pass).  It takes the same StateKernelArgs, so the noisy rollouts,
+// the padded policy rows of the noise-less rollout and stomp_b200_evaluate_states all go through it.
 // Sphere centres and one bounding sphere per link live in thread-local memory (L1).  The host sorts the pairs into
 // blocks by link pair; a block is only walked when the two links' bounding spheres overlap.  The bounding radii are
 // inflated by far more than the rounding of the centres, so the cull never removes a pair that the exact rule
@@ -2808,11 +2795,12 @@ weights_update_peer_kernel(const __grid_constant__ LoopParams p, const __grid_co
 // K10: Stomp::doNoiselessRollout (stomp/src/Stomp.cpp:253-272) + setNoiselessRolloutCosts
 // (PolicyImprovement.cpp:401-419) and the wrapper's stop rule (src/wrappers/stomp/StompPlanner.cpp:107-118).
 // One CTA per query; runs on the engine's side stream, overlapped with the next iteration's sampling and
-// rollout costs (its result is first needed by the next rollout_weights_kernel).
+// rollout costs (its result is first needed by the next rollout_weights_kernel).  The verdicts of the T states are
+// the ones a state pass over the padded policy rows wrote to nl_state just before, on the same stream.
 // =====================================================================================================
 __global__ void __launch_bounds__(256)
 noiseless_rollout_kernel(const __grid_constant__ LoopParams p, const __grid_constant__ RobotParams robot,
-                         const __grid_constant__ SdfParams sdf, int states_done, const __grid_constant__ CostExtras extras)
+                         const __grid_constant__ SdfParams sdf, const __grid_constant__ CostExtras extras)
 {
     extern __shared__ double smem[];
     const int q = blockIdx.x;
@@ -2825,19 +2813,7 @@ noiseless_rollout_kernel(const __grid_constant__ LoopParams p, const __grid_cons
     double* ssum = sstate + T;              // [1 + 2D]
 #pragma unroll 4
     for (int e = tid; e < D * N; e += blockDim.x) sx[e] = p.theta_all[(size_t)q * D * N + e];
-    __syncthreads();
-    if (states_done) {      // the specialised state kernel ran on the padded policy rows just before this launch
-        for (int t = tid; t < T; t += blockDim.x) sstate[t] = p.nl_state[(size_t)q * T + t];
-    } else {
-        for (int t = tid; t < T; t += blockDim.x) {
-            const double* xq = sx + kPad + t;
-            const bool hit = state_collides<false>(robot, sdf, [&](int d) { return xq[(size_t)d * N]; });
-            sstate[t] = hit ? 1.0 : 0.0;
-            p.nl_state[(size_t)q * T + t] = sstate[t];
-            p.nl_verdict[(size_t)q * T + t] = hit ? 1 : 0;
-            if (t == T - 1) p.nl_valid[q] = hit ? 0 : 1;
-        }
-    }
+    for (int t = tid; t < T; t += blockDim.x) sstate[t] = p.nl_state[(size_t)q * T + t];
     __syncthreads();
     if (extras.smooth || extras.joint_constraint) {     // alternative state costs of the noise-less states (see CostExtras)
         for (int t = tid; t < T; t += blockDim.x) {

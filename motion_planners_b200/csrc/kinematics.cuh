@@ -384,7 +384,7 @@ struct SelfPairs {
     int32_t n, nblocks;
 };
 
-// arguments of the specialised state kernel (the subset of LoopParams that rollout_states_kernel reads)
+// arguments of every state kernel (generated, generic, pair rule); filled only by the builders in engine.cu
 struct StateKernelArgs {
     const double* rollouts;        // [Q][slots][D][T]
     double* state_costs;           // [Q][slots][T]

@@ -374,10 +374,41 @@ def test_specialised_state_kernel_equals_generic_kernel_and_oracle(shape, medium
         np.testing.assert_array_equal(spec.tensor("state_costs")[0], gen.tensor("state_costs")[0])
         np.testing.assert_array_equal(spec.tensor("rollout_validity")[0], gen.tensor("rollout_validity")[0])
         np.testing.assert_array_equal(spec.tensor("parameters")[0], gen.tensor("parameters")[0])
+        # the noise-less states: the tail of the specialised kernel against a generic state pass over the policy rows
+        np.testing.assert_array_equal(spec.tensor("noiseless_state_costs")[0], gen.tensor("noiseless_state_costs")[0])
         _, rv, _ = o.state_costs(spec.tensor("rollouts")[0][:K], threads=4)
         np.testing.assert_array_equal(vs[:K], rv)
         hits += int(vs.sum())
     assert hits > 0
+
+
+def test_evaluate_states_beyond_the_specialised_kernels_range(medium_problem):
+    """Joint values the specialised kernel cannot vouch for (|q| > 1e6) send stomp_b200_evaluate_states to the generic
+    kernel even where the specialised one is in use: its verdicts must still be the oracle's, bit for bit.  A NaN in one
+    state must not fail the call nor change any other state's verdict."""
+    pb = medium_problem
+    o, e, _ = _pair(pb)
+    assert e.state_kernel_kind()[0] == "specialised"
+    D, T = pb.chain.num_dimensions, pb.num_time_steps
+    rng = np.random.default_rng(17)
+    theta = rng.uniform(pb.chain.lower[None, :, None], pb.chain.upper[None, :, None], (32, D, T))
+    far = rng.random(theta.shape) < 0.3
+    theta[far] += rng.choice([-1.0, 1.0], far.sum()) * rng.uniform(2e6, 1e7, far.sum())
+    assert np.abs(theta).max() > 1e6
+    costs, verdicts, validity = e.evaluate_states(theta)
+    rc, rv, rval = o.state_costs(theta, threads=4)
+    np.testing.assert_array_equal(verdicts, rv)
+    np.testing.assert_array_equal(costs, rc)
+    np.testing.assert_array_equal(validity, rval)
+    assert 0.0 < costs.mean() < 1.0
+    bad = theta.copy()
+    bad[5, 3, 40] = np.nan
+    c2, v2, val2 = e.evaluate_states(bad)
+    keep = np.ones((32, T), dtype=bool)
+    keep[5, 40] = False
+    np.testing.assert_array_equal(v2[keep], verdicts[keep])
+    np.testing.assert_array_equal(c2[keep], costs[keep])
+    np.testing.assert_array_equal(val2, validity)
 
 
 def test_static_spheres_are_walked_once_per_scene_and_follow_scene_changes(monkeypatch):

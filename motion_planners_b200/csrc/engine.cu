@@ -13,9 +13,11 @@
 //   setRolloutCosts    -> inside the sampler | control_rows_tile_kernel | control_rows_fast_kernel | control_rows_kernel
 //                         [reused_control_cost_kernel]
 //   improvePolicy + updateParameters
-//                      -> weights_update_kernel on one GPU, weights_update_peer_kernel (both exchanges over NVLink mailboxes) on
-//                         rollout shards | with the NCCL exchange, rollout reuse or per-kernel profiling: [allgather]
-//                         rollout_weights_kernel, weighted_update_kernel, reduce_partials_kernel, [allreduce], apply_update_kernel
+//                      -> launch_update_stage, in the shape update_shape classifies the iteration into: weights_update_kernel on
+//                         one GPU, weights_update_peer_kernel (both exchanges over NVLink mailboxes) on rollout shards | with the
+//                         NCCL exchange, rollout reuse or per-kernel profiling: [allgather] rollout_weights_kernel,
+//                         weighted_update_kernel, [reduce_partials_kernel, allreduce], apply_update_kernel | per-time-step costs:
+//                         rollout_weights_kernel, the pertimestep kernels, apply_update_kernel
 //   doNoiselessRollout -> control costs in the update kernel's last CTA per joint, the T states as a tail of the next state kernel
 //                         launch (alone at a join) | a state pass on the T states + noiseless_rollout_kernel (side stream)
 // The rollout bookkeeping (PolicyImprovement.cpp:170-186,304-308) is host integer arithmetic and stays here.
@@ -756,6 +758,109 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
 }
 
 
+// The update stage (K7-K9: computeRolloutProbabilities, computeParameterUpdates, updateParameters) takes one of four shapes.
+// Every rank of a sharded engine classifies alike: the fields involved are set alike on all ranks.
+enum class UpdateShape {
+    kPeer,          // rollout sharding over the peer-mapped mailboxes: weights_update_peer_kernel, both exchanges inside
+    kFused,         // one GPU, no rollout reuse: weights_update_kernel, one launch
+    kPerTimestep,   // per-time-step costs (or forward cumulation): rollout_weights_kernel, the pertimestep kernels, apply_update_kernel
+    kSeparate,      // rollout_weights_kernel -> weighted_update_kernel -> apply_update_kernel: the NCCL exchange (which sits
+                    // between them), rollout reuse, per-kernel profiling, STOMP_B200_FUSE_WEIGHTS=0
+};
+
+// world > 1 implies no rollout reuse (stomp_b200_create), and without reuse buffers no rollout is reused (iterate_body)
+UpdateShape update_shape(const stomp_b200_engine* e, int world)
+{
+    if (e->cfg.use_cumulative_costs != 1) return UpdateShape::kPerTimestep;
+    if (!e->fuse_weights_allowed || e->profiling) return UpdateShape::kSeparate;
+    if (world > 1) return e->peer_ready ? UpdateShape::kPeer : UpdateShape::kSeparate;
+    return e->reuse_possible ? UpdateShape::kSeparate : UpdateShape::kFused;
+}
+
+// K7-K9 of an iteration on the main stream, with the exchanges of a sharded engine; sets lp.nchunks, lp.wblocks and
+// lp.forward_cumulation, which the noise-less rollout and the read-backs take from lp
+int launch_update_stage(stomp_b200_engine* e, LoopParams& lp, UpdateShape shape, int world, bool on_graph)
+{
+    const stomp_b200_config& c = e->cfg;
+    if (world > 1 && !e->comm) return fail(e, STOMP_B200_ERR_NOT_READY, "world_size > 1 needs stomp_b200_comm_init");
+    lp.nchunks = std::max(1, (lp.num_local + lp.chunk - 1) / lp.chunk);
+    // the chunk's weights and weights * quad, later the column sums and the updated row (apply_update_body)
+    const size_t update_smem = sizeof(double) * std::max<size_t>(2 * (size_t)lp.chunk, (size_t)e->T + 2 + (size_t)e->N);
+    auto launch_weights = [&]() -> int {
+        lp.wblocks = std::max(1, std::min(kWeightBlocksMax, (lp.num_rollouts + kWeightThreads - 1) / kWeightThreads));
+        Scope sc(e, STOMP_B200_KERNEL_WEIGHTS);
+        rollout_weights_kernel<<<dim3(lp.wblocks, e->D, e->Q), kWeightThreads, 0, e->stream>>>(lp);
+        return check_launch(e, "rollout_weights_kernel");
+    };
+    auto launch_apply = [&](UpdateSums sums) -> int {
+        Scope sc(e, STOMP_B200_KERNEL_APPLY);
+        apply_update_kernel<<<dim3(e->D, e->Q), 256, sizeof(double) * ((size_t)e->T + 2 + (size_t)e->N), e->stream>>>(lp, sums, lp.nchunks);
+        return check_launch(e, "apply_update_kernel");
+    };
+    switch (shape) {
+    case UpdateShape::kPeer: {
+        lp.wblocks = 1;
+        e->px.epoch = ++e->peer_epoch;
+        e->px.epoch_ptr = on_graph ? e->d_counters + 1 : nullptr;
+        e->tables_gathered = false;
+        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
+        void* args[] = {&lp, &e->px};
+        CUDA_TRY(e, launch_dependent(e, 2, (const void*)weights_update_peer_kernel, dim3(lp.nchunks * e->D), dim3(kUpdateThreads), update_smem, e->stream, args));
+        return check_launch(e, "weights_update_peer_kernel");
+    }
+    case UpdateShape::kFused: {
+        lp.wblocks = 1;
+        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
+        void* args[] = {&lp};
+        CUDA_TRY(e, launch_dependent(e, 2, (const void*)weights_update_kernel, dim3(lp.nchunks, e->D, e->Q), dim3(kUpdateThreads), update_smem, e->stream, args));
+        return check_launch(e, "weights_update_kernel");
+    }
+    case UpdateShape::kPerTimestep: {     // Stomp::setCostCumulation(false): probabilities per time step
+        if (int rc = launch_weights()) return rc;
+        {
+            Scope sc(e, STOMP_B200_KERNEL_UPDATE);
+            lp.forward_cumulation = c.use_cumulative_costs == 2 ? 1 : 0;
+            if (lp.forward_cumulation) {
+                pertimestep_suffix_kernel<<<dim3((lp.num_local * e->D + 127) / 128, e->Q), 128, 0, e->stream>>>(lp);
+                if (int rc = check_launch(e, "pertimestep_suffix_kernel")) return rc;
+            }
+            pertimestep_minmax_kernel<<<dim3(e->D, e->Q), 1024, 0, e->stream>>>(lp);
+            if (int rc = check_launch(e, "pertimestep_minmax_kernel")) return rc;
+            pertimestep_update_kernel<<<dim3((e->T + 127) / 128, e->D, e->Q), 128, 0, e->stream>>>(lp);
+            if (int rc = check_launch(e, "pertimestep_update_kernel")) return rc;
+        }
+        return launch_apply(kSumsReduced);
+    }
+    case UpdateShape::kSeparate: {
+        const bool nccl = world > 1;
+        if (nccl) {     // ---- exchange 1: per-rollout cost scalars (SURVEY.md §8e) ----
+            e->tables_gathered = true;
+            const size_t count = (size_t)lp.num_gen * e->sumw;
+            NCCL_TRY(e, g_nccl.AllGather(lp.sums + (size_t)c.rank * count, lp.sums, count, ncclFloat64, e->comm, e->stream));
+        }
+        if (int rc = launch_weights()) return rc;
+        // the apply step rides on the update kernel's last chunk CTA unless the exchange or per-kernel profiling sits between
+        const bool fuse_apply = !nccl && !e->profiling;
+        {
+            Scope sc(e, STOMP_B200_KERNEL_UPDATE);
+            weighted_update_kernel<<<dim3(lp.nchunks, e->D, e->Q), kUpdateThreads, update_smem, e->stream>>>(lp, fuse_apply ? 1 : 0);
+            if (int rc = check_launch(e, "weighted_update_kernel")) return rc;
+        }
+        if (nccl) {     // ---- exchange 2: update rows + adaptation numerators ----
+            {
+                Scope sc(e, STOMP_B200_KERNEL_UPDATE);
+                reduce_partials_kernel<<<dim3(e->D, e->Q), 256, 0, e->stream>>>(lp, lp.nchunks);
+                if (int rc = check_launch(e, "reduce_partials_kernel")) return rc;
+            }
+            const size_t count = (size_t)e->Q * e->D * (e->T + 2);
+            NCCL_TRY(e, g_nccl.AllReduce(lp.updbuf, lp.updbuf, count, ncclFloat64, ncclSum, e->comm, e->stream));
+        }
+        return fuse_apply ? 0 : launch_apply(nccl ? kSumsReduced : kSumsPartials);
+    }
+    }
+    return 0;
+}
+
 int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop, bool on_graph)
 {
     const stomp_b200_config& c = e->cfg;
@@ -844,14 +949,10 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     const RowsShape rows_kind = rows_shape(e, lp);
     const bool fused_rows = banded && !lp.Mproj && rows_kind == kRowsTile;
     // the shipped large-K loop (fused sampler, fused weights / update kernel, nothing reads `noise` back): the noise
-    // tensor is not materialised — weights_update_kernel subtracts theta from the rollout rows it streams
-    // rollout sharding: both exchanges inside weights_update_peer_kernel over the peer-mapped mailboxes (every rank takes
-    // the same decision: the flags involved are set alike on all ranks)
-    const bool peer = world > 1 && e->peer_ready && !e->profiling && c.use_cumulative_costs == 1 && e->fuse_weights_allowed;
-    // one launch for K7-K9 when nothing sits between them (no exchange, no reused rollouts, no per-kernel profiling)
-    const bool per_timestep = c.use_cumulative_costs != 1;      // 0: per-time-step costs; 2: forward cumulation (cost-to-go)
-    const bool fuse_weights = e->fuse_weights_allowed && (world == 1 || peer) && !e->profiling && !e->reuse_possible && reused == 0 && !per_timestep;
-    lp.noise_from_rollouts = (fused_rows && fuse_weights && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
+    // tensor is not materialised — the update kernel subtracts theta from the rollout rows it streams
+    const UpdateShape shape = update_shape(e, world);
+    const bool one_update_launch = shape == UpdateShape::kFused || shape == UpdateShape::kPeer;
+    lp.noise_from_rollouts = (fused_rows && one_update_launch && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
     if (banded) {
         if (int rc = (mode == kNoisePhilox ? launch_sample_banded<true>(e, lp, fused_rows) : launch_sample_banded<false>(e, lp, fused_rows))) return rc;
     } else if (mode == kNoiseUnit) {
@@ -931,83 +1032,14 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
         if (int rc = check_launch(e, "reused_control_cost_kernel")) return rc;
     }
 
-    // ---- exchange 1: per-rollout cost scalars (SURVEY.md §8e) ----
-    if (world > 1 && !e->comm) return fail(e, STOMP_B200_ERR_NOT_READY, "world_size > 1 needs stomp_b200_comm_init");
-    if (world > 1 && !peer) {
-        e->tables_gathered = true;
-        const size_t count = (size_t)gen_local * e->sumw;
-        NCCL_TRY(e, g_nccl.AllGather(lp.sums + (size_t)c.rank * count, lp.sums, count, ncclFloat64, e->comm, e->stream));
-    }
-
-    const int nchunks = std::max(1, (lp.num_local + lp.chunk - 1) / lp.chunk);
-    lp.nchunks = nchunks;
-    if (peer) {
-        lp.wblocks = 1;
-        e->px.epoch = ++e->peer_epoch;
-        e->px.epoch_ptr = on_graph ? e->d_counters + 1 : nullptr;
-        e->tables_gathered = false;
-        const size_t smem = sizeof(double) * std::max<size_t>(2 * (size_t)lp.chunk, (size_t)e->T + 2 + (size_t)e->N);
-        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
-        void* args[] = {&lp, &e->px};
-        CUDA_TRY(e, launch_dependent(e, 2, (const void*)weights_update_peer_kernel, dim3(lp.nchunks * e->D), dim3(kUpdateThreads), smem, e->stream, args));
-        if (int rc = check_launch(e, "weights_update_peer_kernel")) return rc;
-    } else if (fuse_weights) {
-        lp.wblocks = 1;
-        const size_t smem = sizeof(double) * std::max<size_t>(2 * (size_t)lp.chunk, (size_t)e->T + 2 + (size_t)e->N);
-        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
-        void* args[] = {&lp};
-        CUDA_TRY(e, launch_dependent(e, 2, (const void*)weights_update_kernel, dim3(lp.nchunks, e->D, e->Q), dim3(kUpdateThreads), smem, e->stream, args));
-        if (int rc = check_launch(e, "weights_update_kernel")) return rc;
-    }
-    // ---- probabilities (K7) ----
-    if (!fuse_weights) {
-        lp.wblocks = std::max(1, std::min(kWeightBlocksMax, (n + kWeightThreads - 1) / kWeightThreads));
-        Scope sc(e, STOMP_B200_KERNEL_WEIGHTS);
-        rollout_weights_kernel<<<dim3(lp.wblocks, e->D, e->Q), kWeightThreads, 0, e->stream>>>(lp);
-        if (int rc = check_launch(e, "rollout_weights_kernel")) return rc;
-    }
-    // ---- weighted sums (K8) ----
-    const bool fuse_apply = world == 1 && !e->profiling && !per_timestep;     // the apply step rides on the update kernel's last chunk CTA
-    if (per_timestep) {      // Stomp::setCostCumulation(false): probabilities per time step
-        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
-        lp.forward_cumulation = c.use_cumulative_costs == 2 ? 1 : 0;
-        if (lp.forward_cumulation) {
-            pertimestep_suffix_kernel<<<dim3((lp.num_local * e->D + 127) / 128, e->Q), 128, 0, e->stream>>>(lp);
-            if (int rc = check_launch(e, "pertimestep_suffix_kernel")) return rc;
-        }
-        pertimestep_minmax_kernel<<<dim3(e->D, e->Q), 1024, 0, e->stream>>>(lp);
-        if (int rc = check_launch(e, "pertimestep_minmax_kernel")) return rc;
-        pertimestep_update_kernel<<<dim3((e->T + 127) / 128, e->D, e->Q), 128, 0, e->stream>>>(lp);
-        if (int rc = check_launch(e, "pertimestep_update_kernel")) return rc;
-    } else if (!fuse_weights) {
-        const size_t smem = sizeof(double) * std::max<size_t>(2 * (size_t)lp.chunk, (size_t)e->T + 2 + (size_t)e->N);
-        Scope sc(e, STOMP_B200_KERNEL_UPDATE);
-        weighted_update_kernel<<<dim3(nchunks, e->D, e->Q), kUpdateThreads, smem, e->stream>>>(lp, fuse_apply ? 1 : 0);
-        if (int rc = check_launch(e, "weighted_update_kernel")) return rc;
-    }
-    // ---- exchange 2: update rows + adaptation numerators ----
-    if (world > 1 && !fuse_weights) {
-        {
-            Scope sc(e, STOMP_B200_KERNEL_UPDATE);
-            reduce_partials_kernel<<<dim3(e->D, e->Q), 256, 0, e->stream>>>(lp, nchunks);
-            if (int rc = check_launch(e, "reduce_partials_kernel")) return rc;
-        }
-        const size_t count = (size_t)e->Q * e->D * (e->T + 2);
-        NCCL_TRY(e, g_nccl.AllReduce(lp.updbuf, lp.updbuf, count, ncclFloat64, ncclSum, e->comm, e->stream));
-    }
-    // ---- apply (K9) ----
-    if (!fuse_apply && !fuse_weights) {
-        Scope sc(e, STOMP_B200_KERNEL_APPLY);
-        apply_update_kernel<<<dim3(e->D, e->Q), 256, sizeof(double) * ((size_t)e->T + 2 + (size_t)e->N), e->stream>>>(lp, (world > 1 || per_timestep) ? 0 : 1, nchunks);
-        if (int rc = check_launch(e, "apply_update_kernel")) return rc;
-    }
+    if (int rc = launch_update_stage(e, lp, shape, world, on_graph)) return rc;
     e->last_wblocks = lp.wblocks;
     e->last_noise_from_rollouts = lp.noise_from_rollouts != 0;
     // ---- noise-less rollout (K10): owed; launched on the side stream by the next iteration or the next join ----
     e->nl_lp = lp;
     e->nl_deferred = true;
     e->nl_parity ^= 1;                            // the record this iteration's update wrote is what the next one reads
-    if (on_graph && !peer) ++e->peer_epoch;       // the sampler advances counters[1] on every replayed iteration: keep the host's mirror in step
+    if (on_graph && shape != UpdateShape::kPeer) ++e->peer_epoch;       // the sampler advances counters[1] on every replayed iteration: keep the host's mirror in step
 
     e->num_rollouts = n;
     e->last_gen = gen_local;
@@ -1064,10 +1096,11 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
     e->note_writers_in_flight = true;
     const stomp_b200_config& c = e->cfg;
     const int world = c.shard_mode == 0 ? c.world_size : 1;
-    bool eligible = allow_graph && e->graphs_allowed && e->d_counters && mode == kNoisePhilox && !e->profiling && !e->timeline_on && !e->reuse_possible &&
-                    e->noiseless_valid && c.use_cumulative_costs == 1 && !c.keep_debug_tensors && !e->edge_dirty && !c.use_projection && !e->extras_on &&
-                    e->base.Lband != nullptr && (e->sampler_mode == 0 || e->sampler_mode == 3) && e->fuse_weights_allowed &&
-                    (world == 1 || e->peer_ready) && c.num_rollouts_per_iteration % world == 0 &&
+    const UpdateShape shape = update_shape(e, world);
+    bool eligible = allow_graph && e->graphs_allowed && e->d_counters && mode == kNoisePhilox && !e->timeline_on &&
+                    (shape == UpdateShape::kFused || shape == UpdateShape::kPeer) &&
+                    e->noiseless_valid && !c.keep_debug_tensors && !e->edge_dirty && !c.use_projection && !e->extras_on &&
+                    e->base.Lband != nullptr && (e->sampler_mode == 0 || e->sampler_mode == 3) &&
                     !e->noiseless_pending && (!e->nl_deferred || e->nl_lp.honour_stop == honour_stop);
     eligible = eligible && noiseless_tail_available(e);      // the side-stream rollout bakes per-iteration state into its parameters
     // A sampler that is launched as a programmatic dependent of the previous iteration's update kernel draws its noise beside
@@ -1351,12 +1384,14 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
     if (cfg->num_queries < 1 || cfg->world_size < 1 || cfg->rank < 0 || cfg->rank >= cfg->world_size)
         return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (cfg->shard_mode != 0 && cfg->shard_mode != 1) return STOMP_B200_ERR_INVALID_ARGUMENT;
+    const bool reuse_possible = cfg->num_rollouts_per_iteration < cfg->max_rollouts || cfg->min_rollouts > cfg->num_rollouts_per_iteration;
     // Stomp::setCostCumulation(false): built for the plain case (one GPU, no rollout reuse)
     if (cfg->use_cumulative_costs < 0 || cfg->use_cumulative_costs > 2) return STOMP_B200_ERR_INVALID_ARGUMENT;
-    if (cfg->use_cumulative_costs != 1 && (cfg->world_size > 1 || cfg->num_rollouts_per_iteration < cfg->max_rollouts ||
-                                       cfg->min_rollouts > cfg->num_rollouts_per_iteration))
-        return STOMP_B200_ERR_UNSUPPORTED;
+    if (cfg->use_cumulative_costs != 1 && (cfg->world_size > 1 || reuse_possible)) return STOMP_B200_ERR_UNSUPPORTED;
     if (cfg->shard_mode == 0 && cfg->world_size > 1 && cfg->num_queries != 1) return STOMP_B200_ERR_UNSUPPORTED;
+    // rollout sharding: every rank draws the same number of rollouts every iteration, and none is reused
+    if (cfg->shard_mode == 0 && cfg->world_size > 1 && (reuse_possible || cfg->num_rollouts_per_iteration % cfg->world_size != 0))
+        return STOMP_B200_ERR_UNSUPPORTED;
 
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return STOMP_B200_ERR_NO_DEVICE;
@@ -1377,8 +1412,7 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
         e->Q = cfg->num_queries;
     }
     const int world = cfg->shard_mode == 0 ? cfg->world_size : 1;
-    e->reuse_possible = cfg->num_rollouts_per_iteration < cfg->max_rollouts || cfg->min_rollouts > cfg->num_rollouts_per_iteration;
-    if (world > 1 && e->reuse_possible) { delete e; return STOMP_B200_ERR_UNSUPPORTED; }
+    e->reuse_possible = reuse_possible;
     e->gslots = cfg->max_rollouts + 1;
     e->slots = (world > 1 ? cfg->max_rollouts / world : cfg->max_rollouts) + 1;
     e->have_policy.assign(e->Q, 0);

@@ -2018,6 +2018,16 @@ __device__ __forceinline__ const double* cost_row(const LoopParams& p, int q, in
     return (k == p.noiseless_gslot) ? p.nl_sums + (size_t)q * p.sumw : p.sums + ((size_t)q * p.gslots + k) * p.sumw;
 }
 
+// total_cost_ (PolicyImprovement.cpp:451-462) of global slot g from its cost row s = cost_row(p, q, g): the state costs
+// plus the control costs of the D joints.  s and D are the caller's: read again after the caller's stores, they would
+// be loads of their own.
+__device__ __forceinline__ void store_total_cost(const LoopParams& p, int q, int g, const double* s, int D)
+{
+    double cost = s[0];
+    for (int dd = 0; dd < D; ++dd) cost += s[1 + dd];
+    p.total_cost[(size_t)q * p.gslots + g] = cost;
+}
+
 // grid (wblocks, D, Q), 512 threads.  Every CTA scans all K' rows for the min / max of its joint (two 8-byte loads per
 // row, unrolled so that they are all in flight at once: this kernel is pure L2 latency), then weighs its own slice of
 // the rollouts and leaves the sum of its unnormalised weights in wpart[block]; the consumers (weighted_update_kernel,
@@ -2060,24 +2070,11 @@ rollout_weights_kernel(const __grid_constant__ LoopParams p)
         prob[(size_t)k * D + d] = pr;
         fprob[(size_t)k * D + d] = pr;
         psum += pr;
-        if (d == 0) {   // total_cost_ (:451-462)
-            double cost = s[0];
-            for (int dd = 0; dd < D; ++dd) cost += s[1 + dd];
-            p.total_cost[(size_t)q * p.gslots + k] = cost;
-        }
+        if (d == 0) store_total_cost(p, q, k, s, D);
     }
     psum = block_reduce<0>(psum, scratch);
     if (tid == 0) p.wpart[((size_t)q * D + d) * p.wblocks_cap + blockIdx.x] = psum;
     tls.end();
-}
-
-// sum of the weights of joint d in block order (what every consumer divides by)
-__device__ __forceinline__ double weight_sum(const LoopParams& p, int q, int d)
-{
-    const double* part = p.wpart + ((size_t)q * p.D + d) * p.wblocks_cap;
-    double s = 0.0;
-    for (int b = 0; b < p.wblocks; ++b) s += part[b];
-    return s;
 }
 
 // =====================================================================================================
@@ -2089,14 +2086,108 @@ __device__ __forceinline__ double weight_sum(const LoopParams& p, int q, int d)
 // partial [Q][chunks][D][T+2]: update row, numerator, denominator.
 // =====================================================================================================
 constexpr int kUpdateThreads = 256;
-__device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, int d, int from_partials, int nchunks, double* s_cols);
 
-// 256 threads = two halves of 128: thread (half, lt) streams time step lt of every second rollout row of the chunk with
-// 16 loads in flight, the halves are added in a fixed order.
-// fuse_apply (single GPU): the LAST chunk CTA of a (joint, query) to finish — found with a ticket counter after a
-// __threadfence — also does the work of apply_update_kernel: it sums the partials in chunk order (so the result does
-// not depend on which CTA came last) and updates the parameters and the noise magnitude.  One launch and one
-// drain / fill gap less per iteration.
+// where apply_update_body finds the column sums [T + 2] (update row, adaptation numerator, sum of the weights)
+enum UpdateSums : int {
+    kSumsReduced = 0,            // updbuf: already summed (all-reduced over ranks, or per time step), normalised weights
+    kSumsPartials = 1,           // the chunk partials of normalised weights (weighted_update_kernel)
+    kSumsPartialsUnnormalised,   // the chunk partials of unnormalised weights (weights_update_kernel)
+    kSumsRanksUnnormalised,      // s_cols already holds the unnormalised sums over all ranks (weights_update_peer_kernel)
+};
+__device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, int d, UpdateSums sums, int nchunks, double* s_cols);
+
+// column t of the chunk partials of (joint d, query q), added in chunk order: the result does not depend on which CTA
+// finished last.  __ldcg: the partials may have been written by other CTAs of the running launch.  kUnroll: loads in flight
+// per thread (16 where a single CTA sums all T + 2 columns, on the critical path of the update kernels).
+template <int kUnroll>
+__device__ __forceinline__ double chunk_column_sum(const LoopParams& p, int q, int d, int T, int D, int t, int nchunks)
+{
+    const double* col = p.partial + ((size_t)q * p.nchunks * D + d) * (T + 2) + t;
+    const size_t stride = (size_t)D * (T + 2);
+    double u = 0.0;
+#pragma unroll kUnroll
+    for (int c = 0; c < nchunks; ++c) u += __ldcg(col + (size_t)c * stride);
+    return u;
+}
+
+// The chunk stream: 256 threads = two halves of 128, thread (half, lt) streams time step lt of every second row of the
+// chunk (rows k_begin .. k_begin + nk) with 16 loads in flight, four accumulators; the halves are added in a fixed order.
+// sp / sq: the chunk's row weights and weight * quad in shared memory.  Leaves out[0..T+1] = update row, adaptation
+// numerator, sum of the weights (wsum_part: this thread's share).  T, D, sp and sq are the caller's: read again from p
+// after the caller's stores, they would be loads of their own and change the update kernels' code.
+// rollout_rows (the one-launch update kernels): when LoopParams::noise_from_rollouts is set, the rows are rollouts and
+// noise_ = parameters_noise_ - parameters_ (PolicyImprovement.cpp:803-810) is formed here from the rollout row and theta —
+// the same subtraction of the same two doubles the sampler would do.  theta is only written by the last chunk CTA of the
+// launch, after every chunk CTA has finished streaming.  Otherwise the subtraction is of +0.0, the identity, which the
+// compiler drops.
+__device__ __forceinline__ void stream_chunk(const LoopParams& p, int q, int d, int T, int D, int k_begin, int nk, bool rollout_rows,
+                                             const double* sp, const double* sq, double wsum_part, double* out, double* scratch,
+                                             double* s_half)
+{
+    const int tid = threadIdx.x;
+    const int half = tid >> 7, lt = tid & 127;
+    for (int t0 = 0; t0 < T; t0 += 128) {
+        const int t = t0 + lt;
+        double acc = 0.0;
+        if (t < T) {
+            const bool from_rollouts = rollout_rows && p.noise_from_rollouts != 0;
+            const double* nz = (from_rollouts ? p.rollouts : p.noise) + (((size_t)q * p.slots + k_begin) * D + d) * T + t;
+            const double th_t = from_rollouts ? p.theta_all[((size_t)q * D + d) * p.N + kPad + t] : 0.0;
+            const size_t stride = (size_t)D * T;
+            double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
+            int k = half;
+            for (; k + 30 < nk; k += 32) {       // rows k, k+2, ..., k+30
+                double v[16];
+#pragma unroll
+                for (int u = 0; u < 16; ++u) v[u] = nz[(size_t)(k + 2 * u) * stride] - th_t;
+#pragma unroll
+                for (int u = 0; u < 16; u += 4) {
+                    a0 += v[u] * sp[k + 2 * u]; a1 += v[u + 1] * sp[k + 2 * u + 2];
+                    a2 += v[u + 2] * sp[k + 2 * u + 4]; a3 += v[u + 3] * sp[k + 2 * u + 6];
+                }
+            }
+            for (; k < nk; k += 2) a0 += (nz[(size_t)k * stride] - th_t) * sp[k];
+            acc = (a0 + a1) + (a2 + a3);
+        }
+        if (half != 0) s_half[lt] = acc;       // the second half (half is 0 or 1 with 256 threads)
+        __syncthreads();
+        if (half == 0 && t < T) out[t] = acc + s_half[lt];
+        __syncthreads();
+    }
+    double numer = 0.0;
+    for (int k = tid; k < nk; k += blockDim.x) numer += sq[k];
+    numer = block_reduce<0>(numer, scratch);
+    wsum_part = block_reduce<0>(wsum_part, scratch);
+    if (tid == 0) { out[T] = numer; out[T + 1] = wsum_part; }
+}
+
+// chunk CTAs per (joint, query): gridDim.x of a (chunks, D, Q) grid, p.nchunks for weights_update_peer_kernel's
+// one-dimensional grid.  Read where it is used: held from before the __threadfence below, it costs a register.
+template <bool kPeer>
+__device__ __forceinline__ unsigned int chunk_ctas(const LoopParams& p)
+{
+    return kPeer ? (unsigned int)p.nchunks : gridDim.x;
+}
+
+// The LAST chunk CTA of a (joint, query) to finish — found with a ticket counter after a __threadfence — runs apply(),
+// when every chunk's partials are visible, and resets the ticket for the next launch.  D is the caller's copy of p.D and
+// s_last the caller's __shared__ int: declared here, it would reorder the caller's shared memory and change its code.
+template <bool kPeer, class Apply>
+__device__ __forceinline__ void last_chunk_cta(const LoopParams& p, int q, int d, int D, int& s_last, Apply apply)
+{
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = (atomicAdd(p.done_counter + (size_t)q * D + d, 1u) == chunk_ctas<kPeer>(p) - 1u) ? 1 : 0;
+    __syncthreads();
+    if (s_last) {
+        __threadfence();
+        apply();
+        if (threadIdx.x == 0) p.done_counter[(size_t)q * D + d] = 0u;
+    }
+}
+
+// fuse_apply (single GPU): the last chunk CTA also does the work of apply_update_kernel.  One launch and one drain / fill
+// gap less per iteration.
 // dynamic shared memory: max(2 * chunk, T + 2 + N) doubles (the last CTA of a joint also stages the updated row: apply_update_body).
 __global__ void __launch_bounds__(kUpdateThreads)
 weighted_update_kernel(const __grid_constant__ LoopParams p, int fuse_apply)
@@ -2104,11 +2195,11 @@ weighted_update_kernel(const __grid_constant__ LoopParams p, int fuse_apply)
     extern __shared__ double smem[];   // [chunk] probabilities, [chunk] fprob * quad ; later [T + 2] column sums
     __shared__ double scratch[32];
     __shared__ double s_half[128];
+    __shared__ int s_last;
     const int d = blockIdx.y, q = blockIdx.z, c = blockIdx.x;
     if (query_frozen(p, q)) return;
     TimelineScope tls(p, 3);
     const int T = p.T, D = p.D, tid = threadIdx.x;
-    const int half = tid >> 7, lt = tid & 127;
     const int k_begin = c * p.chunk, k_end = min(p.num_local, (c + 1) * p.chunk);
     const int nk = k_end - k_begin;
     double* sp = smem;
@@ -2138,77 +2229,135 @@ weighted_update_kernel(const __grid_constant__ LoopParams p, int fuse_apply)
     }
     __syncthreads();
     double* out = p.partial + (((size_t)q * p.nchunks + c) * D + d) * (T + 2);
-    for (int t0 = 0; t0 < T; t0 += 128) {
-        const int t = t0 + lt;
-        double acc = 0.0;
-        if (t < T) {
-            const double* nz = p.noise + (((size_t)q * p.slots + k_begin) * D + d) * T + t;
-            const size_t stride = (size_t)D * T;
-            double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-            int k = half;
-            for (; k + 30 < nk; k += 32) {       // rows k, k+2, ..., k+30
-                double v[16];
-#pragma unroll
-                for (int u = 0; u < 16; ++u) v[u] = nz[(size_t)(k + 2 * u) * stride];
-#pragma unroll
-                for (int u = 0; u < 16; u += 4) {
-                    a0 += v[u] * sp[k + 2 * u]; a1 += v[u + 1] * sp[k + 2 * u + 2];
-                    a2 += v[u + 2] * sp[k + 2 * u + 4]; a3 += v[u + 3] * sp[k + 2 * u + 6];
-                }
-            }
-            for (; k < nk; k += 2) a0 += nz[(size_t)k * stride] * sp[k];
-            acc = (a0 + a1) + (a2 + a3);
-        }
-        if (half == 1) s_half[lt] = acc;
-        __syncthreads();
-        if (half == 0 && t < T) out[t] = acc + s_half[lt];
-        __syncthreads();
-    }
-    double numer = 0.0;
-    for (int k = tid; k < nk; k += blockDim.x) numer += sq[k];
-    numer = block_reduce<0>(numer, scratch);
-    fsum_part = block_reduce<0>(fsum_part, scratch);
-    if (tid == 0) { out[T] = numer; out[T + 1] = fsum_part; }
-    if (fuse_apply) {
-        __shared__ int s_last;
-        __threadfence();
-        __syncthreads();
-        if (tid == 0) s_last = (atomicAdd(p.done_counter + (size_t)q * D + d, 1u) == gridDim.x - 1) ? 1 : 0;
-        __syncthreads();
-        if (s_last) {
-            __threadfence();
-            apply_update_body(p, q, d, 1, (int)gridDim.x, smem);
-            if (tid == 0) p.done_counter[(size_t)q * D + d] = 0u;
-        }
-    }
+    stream_chunk(p, q, d, T, D, k_begin, nk, false, sp, sq, fsum_part, out, scratch, s_half);
+    if (fuse_apply)
+        last_chunk_cta<false>(p, q, d, D, s_last, [&] { apply_update_body(p, q, d, kSumsPartials, (int)gridDim.x, smem); });
     tls.end();
 }
 
-// K7 + K8 + K9 in one launch (single GPU, no rollout reuse): computeRolloutProbabilities, computeParameterUpdates and
-// updateParameters.  grid (chunks, D, Q), 256 threads.  Every CTA finds the min / max of its joint's costs itself — a
-// coalesced scan of the compact mirrors s_compact / c_compact (2 x 8 K' bytes, L2 hits after the first CTA) — weighs
-// the rollouts of its chunk (exp), streams their noise rows, and leaves the UNNORMALISED partial sums
+// =====================================================================================================
+// Rollout sharding without a collective library on the data path (SURVEY.md 8e, DESIGN.md 8).  Every rank maps the
+// other ranks' MAILBOX (cudaIpc, engine.cu: setup_peer_exchange) and the two exchanges of an iteration happen inside ONE
+// kernel, weights_update_peer_kernel, as plain stores over NVLink and spins on the rank's own memory:
+//   A. the min / max of cumulative_costs_[d] over the rank's own rollouts (2 doubles per joint) -> every rank takes the
+//      min / max over the ranks: the same two numbers the single-GPU scan finds, so the weights are bit-identical;
+//   B. the rank's unnormalised partial sums [T + 2] per joint (update row, adaptation numerator, sum of the weights) ->
+//      every rank adds the rows in RANK ORDER (deterministic, identical on all ranks) and applies the update.
+// Transport: every double travels as two self-validating 8-byte words {epoch : 32 | half of the bits : 32} (the "LL"
+// scheme: an aligned 8-byte store is atomic, so a word whose tag equals the exchange's epoch IS the data).  No fence, no
+// separate flag, no release / acquire pair: one NVLink crossing per exchange.  (The first version — data, then
+// __threadfence_system, then a release flag — cost 13 us per iteration on two B200s: MEMBAR.SYS is slow.)  The epoch is
+// one per iteration, the same on every rank; slots are double buffered by its parity (a rank reaches exchange A of epoch
+// e + 2 only after every rank has published B of e + 1, i.e. after it finished reading epoch e).  A spin that lasts 4 s
+// sets the error flag, which every later wait honours: a missing rank costs seconds, never a hung GPU.
+// Mailbox layout (bytes from the base; W ranks, D joints, T time steps):
+//   A [2][W][D][2 doubles as 4 words] | B [2][W][D][T + 2 doubles as 2 (T + 2) words] | barrier [W] u32
+// =====================================================================================================
+constexpr int kMaxPeers = 8;
+struct PeerExchange {
+    unsigned char* box[kMaxPeers];   // mailbox of every rank, own included (own: plain device memory)
+    int32_t world, rank;
+    uint32_t epoch;                  // this iteration's exchange number (>= 1) unless epoch_ptr is set
+    const uint32_t* epoch_ptr;       // device-side epoch (iterations replayed from a CUDA graph), or null
+    int32_t* error;                  // device flag: a wait timed out
+    int32_t D, T;
+};
+__host__ __device__ inline size_t peer_off_b(int W, int D) { return (size_t)2 * W * D * 32; }
+__host__ __device__ inline size_t peer_off_barrier(int W, int D, int T) { return peer_off_b(W, D) + (size_t)2 * W * D * (T + 2) * 16; }
+__host__ __device__ inline size_t peer_box_bytes(int W, int D, int T) { return peer_off_barrier(W, D, T) + 64; }
+
+__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p)
+{
+    uint32_t v;
+    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v)
+{
+    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+// waits until *flag has reached `epoch`; false (and the error flag) after 4 s, or at once when the flag is already set
+__device__ __forceinline__ bool peer_wait(const uint32_t* flag, uint32_t epoch, int32_t* error)
+{
+    unsigned long long t0 = 0;
+    int polls = 0;
+    while ((int32_t)(ld_acquire_sys(flag) - epoch) < 0) {
+        if (++polls == 256) {
+            polls = 0;
+            if (*(volatile int32_t*)error) return false;
+            const unsigned long long now = global_timer_ns();
+            if (t0 == 0) t0 = now;
+            else if (now - t0 > 4000000000ull) { atomicExch(error, 1); return false; }
+        }
+    }
+    return true;
+}
+// one double as two tagged words, 16 bytes at dst (16-byte aligned)
+__device__ __forceinline__ void ll_store(unsigned char* dst, double v, uint32_t epoch)
+{
+    const unsigned long long bits = (unsigned long long)__double_as_longlong(v), tag = (unsigned long long)epoch << 32;
+    const unsigned long long w0 = tag | (bits & 0xffffffffull), w1 = tag | (bits >> 32);
+    asm volatile("st.volatile.global.v2.u64 [%0], {%1, %2};" ::"l"(dst), "l"(w0), "l"(w1) : "memory");
+}
+// spins until both words at src carry `epoch`; 0.0 (and the error flag) after 4 s
+__device__ __forceinline__ double ll_load(const unsigned char* src, uint32_t epoch, int32_t* error)
+{
+    unsigned long long w0, w1, t0 = 0;
+    int polls = 0;
+    for (;;) {
+        asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(w0), "=l"(w1) : "l"(src) : "memory");
+        if ((uint32_t)(w0 >> 32) == epoch && (uint32_t)(w1 >> 32) == epoch) break;
+        if (++polls == 256) {
+            polls = 0;
+            if (*(volatile int32_t*)error) return 0.0;
+            const unsigned long long now = global_timer_ns();
+            if (t0 == 0) t0 = now;
+            else if (now - t0 > 4000000000ull) { atomicExch(error, 1); return 0.0; }
+        }
+    }
+    return __longlong_as_double((long long)((w1 << 32) | (w0 & 0xffffffffull)));
+}
+
+// all ranks meet on the device (timer brackets of a sharded run start together); one warp
+__global__ void peer_barrier_kernel(const __grid_constant__ PeerExchange px, uint32_t ticket)
+{
+    const int r = threadIdx.x;
+    if (r >= px.world) return;
+    const size_t off = peer_off_barrier(px.world, px.D, px.T);
+    st_release_sys(reinterpret_cast<uint32_t*>(px.box[r] + off) + px.rank, ticket);
+    peer_wait(reinterpret_cast<const uint32_t*>(px.box[px.rank] + off) + r, ticket, px.error);
+}
+
+// K7 + K8 + K9 in one launch: computeRolloutProbabilities, computeParameterUpdates and updateParameters.  256 threads
+// per CTA, one CTA per (chunk, joint, query).  Every CTA finds the min / max of its joint's costs itself — a coalesced
+// scan of the compact mirrors s_compact / c_compact (2 x 8 K' bytes, L2 hits after the first CTA) — weighs the rollouts
+// of its chunk (exp), streams their noise rows, and leaves the UNNORMALISED partial sums
 //   out[t] = sum_k p_k noise_k[t],  out[T] = sum_k p_k (n^T R n)_k,  out[T+1] = sum_k p_k
 // in `partial`; the last CTA of the (joint, query) adds the chunks in chunk order and divides by sum_k p_k
 // (probabilities_ = p / p_sum, PolicyImprovement.cpp:546-549; the division commutes with the sum over k up to
 // rounding).  Replaces rollout_weights_kernel -> gap -> weighted_update_kernel: one launch, one exposed L2 scan less.
-__global__ void __launch_bounds__(kUpdateThreads)
-weights_update_kernel(const __grid_constant__ LoopParams p)
+// kPeer (rollout sharding, px): the scan covers this rank's rollouts and the noise-less one, exchange A makes the min /
+// max global; exchange B adds the ranks' sums in rank order in front of the apply.
+// dynamic shared memory: max(2 * chunk, T + 2 + N) doubles.
+template <bool kPeer>
+__device__ __forceinline__ void weights_update_body(const LoopParams& p, const PeerExchange* px, int c, int d, int q)
 {
     extern __shared__ double smem[];   // [chunk] weights, [chunk] weight * quad ; later [T + 2] column sums
     __shared__ double scratch[32];
     __shared__ double s_half[128];
-    const int d = blockIdx.y, q = blockIdx.z, c = blockIdx.x;
+    __shared__ int s_last;
     pdl_trigger_and_wait();
     if (p.counters && c == 0 && d == 0 && q == 0 && threadIdx.x == 0) p.counters[0] += 1u;   // next iteration number (graph replay)
     if (query_frozen(p, q)) return;
     TimelineScope tls(p, 3);
     const int T = p.T, D = p.D, tid = threadIdx.x, n = p.num_rollouts;
-    const int half = tid >> 7, lt = tid & 127;
     const int k_begin = c * p.chunk, k_end = min(p.num_local, (c + 1) * p.chunk);
     const int nk = k_end - k_begin;
     double* sp = smem;
     double* sq = smem + p.chunk;
+    uint32_t epoch = 0;
+    if constexpr (kPeer) epoch = px->epoch_ptr ? __ldcg(px->epoch_ptr) : px->epoch;
+    const int parity = (int)(epoch & 1u);
     if (c == 0 && d == 0 && p.noiseless_slot >= 0) materialise_noiseless(p, q, tid, blockDim.x);
 
     // ---- min / max of cumulative_costs_[d] = S + C_d over all rollouts (PolicyImprovement.cpp:501-513) ----
@@ -2217,12 +2366,41 @@ weights_update_kernel(const __grid_constant__ LoopParams p)
     const double* nl = p.nl_sums + (size_t)q * p.sumw;
     auto cum_of = [&](int g) { return (g == p.noiseless_gslot) ? 1.0 * (nl[0] + nl[1 + d]) : 1.0 * (S[g] + C[g]); };
     double mn = 1e300, mx = -1e300;
+    if constexpr (kPeer) {     // this rank's rollouts and the noise-less one
 #pragma unroll 8
-    for (int k = tid; k < n; k += kUpdateThreads) {
-        const double cum = cum_of(k);
-        mn = fmin(mn, cum); mx = fmax(mx, cum);
+        for (int k = tid; k < p.num_gen; k += kUpdateThreads) {
+            const double cum = cum_of(p.gen_offset + k);
+            mn = fmin(mn, cum); mx = fmax(mx, cum);
+        }
+        if (tid == 0 && p.noiseless_gslot >= 0) { const double cum = cum_of(p.noiseless_gslot); mn = fmin(mn, cum); mx = fmax(mx, cum); }
+    } else {
+#pragma unroll 8
+        for (int k = tid; k < n; k += kUpdateThreads) {
+            const double cum = cum_of(k);
+            mn = fmin(mn, cum); mx = fmax(mx, cum);
+        }
     }
     mn = block_reduce<1>(mn, scratch); mx = block_reduce<2>(mx, scratch);
+    if constexpr (kPeer) {     // ---- exchange A: every rank takes the min / max over the ranks ----
+        __shared__ double s_mm[2 * kMaxPeers];
+        const int W = px->world, rank = px->rank;
+        if (c == 0 && tid < W && tid != rank) {
+            unsigned char* dst = px->box[tid] + (((size_t)parity * W + rank) * D + d) * 32;
+            ll_store(dst, mn, epoch);
+            ll_store(dst + 16, mx, epoch);
+        }
+        if (tid < W) {
+            double vmn = mn, vmx = mx;
+            if (tid != rank) {
+                const unsigned char* src = px->box[rank] + (((size_t)parity * W + tid) * D + d) * 32;
+                vmn = ll_load(src, epoch, px->error);
+                vmx = ll_load(src + 16, epoch, px->error);
+            }
+            s_mm[2 * tid] = vmn; s_mm[2 * tid + 1] = vmx;
+        }
+        __syncthreads();
+        for (int r = 0; r < W; ++r) { mn = fmin(mn, s_mm[2 * r]); mx = fmax(mx, s_mm[2 * r + 1]); }
+    }
     double den = mx - mn;
     if (den < 1e-8) den = 1e-8;
     const double h = p.cost_scaling_h;
@@ -2230,75 +2408,66 @@ weights_update_kernel(const __grid_constant__ LoopParams p)
     // ---- unnormalised weights of this chunk ----
     double psum_part = 0.0;
     for (int k = k_begin + tid; k < k_end; k += blockDim.x) {
-        const int g = (k == p.noiseless_slot) ? p.noiseless_gslot : ((k < p.num_gen) ? p.gen_offset + k : k);
+        // a rank of a sharded engine reuses no rollouts: every slot but the noise-less one is a generated rollout
+        const int g = (k == p.noiseless_slot) ? p.noiseless_gslot : ((kPeer || k < p.num_gen) ? p.gen_offset + k : k);
         const double pr = 1.0 * exp(((-h) * (cum_of(g) - mn)) / den);      // importance_weight_ = 1
         const size_t o = ((size_t)q * p.gslots + g) * D + d;
         p.prob[o] = pr;
         p.fprob[o] = pr;
-        psum_part += pr;
+        // the noise-less rollout is replicated on every rank: only the first rank counts it in the sum of the weights
+        if (!(kPeer && k == p.noiseless_slot && px->rank != 0)) psum_part += pr;
         double w = pr, fq = 0.0;
         if (k == p.noiseless_slot) w = 0.0;       // zero noise: contributes nothing (PolicyImprovement.cpp:407-410)
         else if (p.use_noise_adaptation) fq = pr * p.sums[((size_t)q * p.gslots + g) * p.sumw + 1 + 2 * D + d];
         sp[k - k_begin] = w;
         sq[k - k_begin] = fq;
-        if (d == 0) {   // total_cost_ (:451-462)
-            const double* s = cost_row(p, q, g);
-            double cost = s[0];
-            for (int dd = 0; dd < D; ++dd) cost += s[1 + dd];
-            p.total_cost[(size_t)q * p.gslots + g] = cost;
-        }
+        if (d == 0) store_total_cost(p, q, g, cost_row(p, q, g), D);
     }
     __syncthreads();
     double* out = p.partial + (((size_t)q * p.nchunks + c) * D + d) * (T + 2);
-    for (int t0 = 0; t0 < T; t0 += 128) {
-        const int t = t0 + lt;
-        double acc = 0.0;
-        if (t < T) {
-            // noise_ = parameters_noise_ - parameters_ (PolicyImprovement.cpp:803-810).  When the sampler did not materialise it
-            // (LoopParams::noise_from_rollouts) it is formed here from the rollout row and theta — the same subtraction of the
-            // same two doubles — which halves the sampler's write burst; theta is only updated by the last CTA of this launch,
-            // after every chunk CTA has finished streaming.
-            const bool from_rollouts = p.noise_from_rollouts != 0;
-            const double* nz = (from_rollouts ? p.rollouts : p.noise) + (((size_t)q * p.slots + k_begin) * D + d) * T + t;
-            const double th_t = from_rollouts ? p.theta_all[((size_t)q * D + d) * p.N + kPad + t] : 0.0;
-            const size_t stride = (size_t)D * T;
-            double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-            int k = half;
-            for (; k + 30 < nk; k += 32) {       // rows k, k+2, ..., k+30
-                double v[16];
-#pragma unroll
-                for (int u = 0; u < 16; ++u) v[u] = nz[(size_t)(k + 2 * u) * stride] - th_t;
-#pragma unroll
-                for (int u = 0; u < 16; u += 4) {
-                    a0 += v[u] * sp[k + 2 * u]; a1 += v[u + 1] * sp[k + 2 * u + 2];
-                    a2 += v[u + 2] * sp[k + 2 * u + 4]; a3 += v[u + 3] * sp[k + 2 * u + 6];
-                }
-            }
-            for (; k < nk; k += 2) a0 += (nz[(size_t)k * stride] - th_t) * sp[k];
-            acc = (a0 + a1) + (a2 + a3);
-        }
-        if (half == 1) s_half[lt] = acc;
-        __syncthreads();
-        if (half == 0 && t < T) out[t] = acc + s_half[lt];
-        __syncthreads();
-    }
-    double numer = 0.0;
-    for (int k = tid; k < nk; k += blockDim.x) numer += sq[k];
-    numer = block_reduce<0>(numer, scratch);
-    psum_part = block_reduce<0>(psum_part, scratch);
-    if (tid == 0) { out[T] = numer; out[T + 1] = psum_part; }
+    stream_chunk(p, q, d, T, D, k_begin, nk, true, sp, sq, psum_part, out, scratch, s_half);
 
-    __shared__ int s_last;
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) s_last = (atomicAdd(p.done_counter + (size_t)q * D + d, 1u) == gridDim.x - 1) ? 1 : 0;
-    __syncthreads();
-    if (s_last) {
-        __threadfence();
-        apply_update_body(p, q, d, 2, (int)gridDim.x, smem);
-        if (tid == 0) p.done_counter[(size_t)q * D + d] = 0u;
-    }
+    last_chunk_cta<kPeer>(p, q, d, D, s_last, [&] {
+        if constexpr (kPeer) {
+            // ---- exchange B: this rank's sums in chunk order -> every mailbox; then all ranks' rows in rank order ----
+            const int W = px->world, rank = px->rank;
+            const size_t offb = peer_off_b(W, D);
+            for (int t = tid; t < T + 2; t += blockDim.x) {
+                const double mine = chunk_column_sum<8>(p, q, d, T, D, t, (int)chunk_ctas<kPeer>(p));
+                for (int r = 0; r < W; ++r)
+                    if (r != rank) ll_store(px->box[r] + offb + ((((size_t)parity * W + rank) * D + d) * (T + 2) + t) * 16, mine, epoch);
+                double u = 0.0;
+                for (int r = 0; r < W; ++r)
+                    u += (r == rank) ? mine : ll_load(px->box[rank] + offb + ((((size_t)parity * W + r) * D + d) * (T + 2) + t) * 16, epoch, px->error);
+                smem[t] = u;
+            }
+            apply_update_body(p, q, d, kSumsRanksUnnormalised, (int)chunk_ctas<kPeer>(p), smem);
+        } else {
+            apply_update_body(p, q, d, kSumsPartialsUnnormalised, (int)chunk_ctas<kPeer>(p), smem);
+        }
+    });
     tls.end();
+}
+
+// single GPU, no rollout reuse: grid (chunks, D, Q)
+__global__ void __launch_bounds__(kUpdateThreads)
+weights_update_kernel(const __grid_constant__ LoopParams p)
+{
+    const int d = blockIdx.y, q = blockIdx.z, c = blockIdx.x;
+    weights_update_body<false>(p, nullptr, c, d, q);
+}
+
+// a rollout-sharded engine (one query): grid nchunks * D CTAs in one dimension.  The D CTAs that publish exchange A come
+// first in dispatch order and no CTA ever waits for another CTA of its own grid before publishing, so the spins cannot
+// starve a publisher of an SM.
+__global__ void __launch_bounds__(kUpdateThreads)
+weights_update_peer_kernel(const __grid_constant__ LoopParams p, const __grid_constant__ PeerExchange px)
+{
+    const int D = p.D, nchunks = p.nchunks;
+    int c, d;
+    if ((int)blockIdx.x < D) { c = 0; d = blockIdx.x; }
+    else { const int r = blockIdx.x - D; d = r / (nchunks - 1); c = 1 + (r - d * (nchunks - 1)); }
+    weights_update_body<true>(p, &px, c, d, 0);
 }
 
 // -----------------------------------------------------------------------------------------------------
@@ -2414,21 +2583,16 @@ reduce_partials_kernel(const __grid_constant__ LoopParams p, int nchunks)
     const int d = blockIdx.x, q = blockIdx.y;
     if (query_frozen(p, q)) return;
     const int T = p.T, D = p.D;
-    for (int t = threadIdx.x; t < T + 2; t += blockDim.x) {
-        double s = 0.0;
-#pragma unroll 8
-        for (int c = 0; c < nchunks; ++c) s += p.partial[(((size_t)q * p.nchunks + c) * D + d) * (T + 2) + t];
-        p.updbuf[((size_t)q * D + d) * (T + 2) + t] = s;
-    }
+    for (int t = threadIdx.x; t < T + 2; t += blockDim.x) p.updbuf[((size_t)q * D + d) * (T + 2) + t] = chunk_column_sum<8>(p, q, d, T, D, t, nchunks);
 }
 
 // =====================================================================================================
 // K8 tail + K9: noise adaptation (PolicyImprovement.cpp:656-679) and CovariantMovementPrimitive::
-// updateParameters (stomp/src/CovariantMovementPrimitive.cpp:476-479).  grid (D, Q).  from_partials:
-// sum the chunk partials here (single GPU); otherwise read the all-reduced updbuf.
+// updateParameters (stomp/src/CovariantMovementPrimitive.cpp:476-479).  grid (D, Q).  sums: where the column sums
+// come from (UpdateSums).
 // =====================================================================================================
 // s_cols: T + 2 doubles of shared memory.  Column sums first (all threads, 16 loads in flight each), then the update.
-__device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, int d, int from_partials, int nchunks, double* s_cols)
+__device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, int d, UpdateSums sums, int nchunks, double* s_cols)
 {
     const int T = p.T, D = p.D, N = p.N;
     __syncthreads();
@@ -2437,33 +2601,22 @@ __device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, in
             const int j = i < kPad ? i : T + i;
             s_cols[(T + 2) + j] = p.theta_all[((size_t)q * D + d) * N + j];
         }
-    if (from_partials == 3) from_partials = 2;      // weights_update_peer_kernel: s_cols already holds the unnormalised sums over all ranks
-    else
-    for (int t = threadIdx.x; t < T + 2; t += blockDim.x) {
-        double u;
-        if (from_partials) {
-            u = 0.0;
-            const double* col = p.partial + ((size_t)q * p.nchunks * D + d) * (T + 2) + t;
-            const size_t stride = (size_t)D * (T + 2);
-#pragma unroll 16
-            for (int c = 0; c < nchunks; ++c) u += __ldcg(col + (size_t)c * stride);     // chunk order
-        } else {
-            u = p.updbuf[((size_t)q * D + d) * (T + 2) + t];
-        }
-        s_cols[t] = u;
-    }
+    if (sums != kSumsRanksUnnormalised)
+        for (int t = threadIdx.x; t < T + 2; t += blockDim.x)
+            s_cols[t] = (sums == kSumsReduced) ? p.updbuf[((size_t)q * D + d) * (T + 2) + t] : chunk_column_sum<16>(p, q, d, T, D, t, nchunks);
     __syncthreads();
-    // from_partials == 2 (weights_update_kernel): the sums carry unnormalised weights; divide by their total, which is
-    // also what the read-backs of the probabilities divide by
-    const double psum = (from_partials == 2) ? s_cols[T + 1] : 1.0;
-    if (from_partials == 2 && threadIdx.x == 0) p.wpart[((size_t)q * D + d) * p.wblocks_cap] = psum;
+    // unnormalised weights (weights_update_kernel, weights_update_peer_kernel): divide by their total, which is also what
+    // the read-backs of the probabilities divide by
+    const bool unnormalised = sums == kSumsPartialsUnnormalised || sums == kSumsRanksUnnormalised;
+    const double psum = unnormalised ? s_cols[T + 1] : 1.0;
+    if (unnormalised && threadIdx.x == 0) p.wpart[((size_t)q * D + d) * p.wblocks_cap] = psum;
     if (p.Mproj) {
         // parameter_updates_.row(0) = projection_matrix_ * row(0) (PolicyImprovement.cpp:706): normalise the row in
         // place first (the branch below then sees the finished row), every thread then forms its own dot product
         __syncthreads();
         for (int t = threadIdx.x; t < T; t += blockDim.x) {
             double u = s_cols[t];
-            if (from_partials == 2) u = u / psum;
+            if (unnormalised) u = u / psum;
             u *= 1.0;
             u /= 1.0;
             s_cols[t] = u;
@@ -2472,7 +2625,7 @@ __device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, in
     }
     for (int t = threadIdx.x; t < T + 1; t += blockDim.x) {
         double u = s_cols[t];
-        if (from_partials == 2 && !(p.Mproj && t < T)) u = u / psum;
+        if (unnormalised && !(p.Mproj && t < T)) u = u / psum;
         if (t < T) {
             if (p.Mproj) {
                 const double* mrow = p.Mproj + (size_t)t * T;
@@ -2490,7 +2643,7 @@ __device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, in
             *th = updated;
             if (p.nl_sums_next) s_cols[(T + 2) + kPad + t] = updated;       // the updated row, staged for its control costs below
         } else if (p.use_noise_adaptation) {
-            const double denom = (from_partials == 2) ? s_cols[T + 1] / psum : s_cols[T + 1];
+            const double denom = unnormalised ? s_cols[T + 1] / psum : s_cols[T + 1];
             p.fprob_sum[(size_t)q * D + d] = denom;
             const double frob_stddev = sqrt(u / (denom * T));
             const double update_rate = 0.2;
@@ -2539,255 +2692,13 @@ __device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, in
 
 // dynamic shared memory: T + 2 + N doubles
 __global__ void __launch_bounds__(256)
-apply_update_kernel(const __grid_constant__ LoopParams p, int from_partials, int nchunks)
+apply_update_kernel(const __grid_constant__ LoopParams p, int sums, int nchunks)     // sums: UpdateSums
 {
     extern __shared__ double smem[];
     const int d = blockIdx.x, q = blockIdx.y;
     if (query_frozen(p, q)) return;
     TimelineScope tls(p, 4);
-    apply_update_body(p, q, d, from_partials, nchunks, smem);
-    tls.end();
-}
-
-// =====================================================================================================
-// Rollout sharding without a collective library on the data path (SURVEY.md 8e, DESIGN.md 8).  Every rank maps the
-// other ranks' MAILBOX (cudaIpc, engine.cu: setup_peer_exchange) and the two exchanges of an iteration happen inside ONE
-// kernel, weights_update_peer_kernel, as plain stores over NVLink and spins on the rank's own memory:
-//   A. the min / max of cumulative_costs_[d] over the rank's own rollouts (2 doubles per joint) -> every rank takes the
-//      min / max over the ranks: the same two numbers the single-GPU scan finds, so the weights are bit-identical;
-//   B. the rank's unnormalised partial sums [T + 2] per joint (update row, adaptation numerator, sum of the weights) ->
-//      every rank adds the rows in RANK ORDER (deterministic, identical on all ranks) and applies the update.
-// Transport: every double travels as two self-validating 8-byte words {epoch : 32 | half of the bits : 32} (the "LL"
-// scheme: an aligned 8-byte store is atomic, so a word whose tag equals the exchange's epoch IS the data).  No fence, no
-// separate flag, no release / acquire pair: one NVLink crossing per exchange.  (The first version — data, then
-// __threadfence_system, then a release flag — cost 13 us per iteration on two B200s: MEMBAR.SYS is slow.)  The epoch is
-// one per iteration, the same on every rank; slots are double buffered by its parity (a rank reaches exchange A of epoch
-// e + 2 only after every rank has published B of e + 1, i.e. after it finished reading epoch e).  A spin that lasts 4 s
-// sets the error flag, which every later wait honours: a missing rank costs seconds, never a hung GPU.
-// Mailbox layout (bytes from the base; W ranks, D joints, T time steps):
-//   A [2][W][D][2 doubles as 4 words] | B [2][W][D][T + 2 doubles as 2 (T + 2) words] | barrier [W] u32
-// =====================================================================================================
-constexpr int kMaxPeers = 8;
-struct PeerExchange {
-    unsigned char* box[kMaxPeers];   // mailbox of every rank, own included (own: plain device memory)
-    int32_t world, rank;
-    uint32_t epoch;                  // this iteration's exchange number (>= 1) unless epoch_ptr is set
-    const uint32_t* epoch_ptr;       // device-side epoch (iterations replayed from a CUDA graph), or null
-    int32_t* error;                  // device flag: a wait timed out
-    int32_t D, T;
-};
-__host__ __device__ inline size_t peer_off_b(int W, int D) { return (size_t)2 * W * D * 32; }
-__host__ __device__ inline size_t peer_off_barrier(int W, int D, int T) { return peer_off_b(W, D) + (size_t)2 * W * D * (T + 2) * 16; }
-__host__ __device__ inline size_t peer_box_bytes(int W, int D, int T) { return peer_off_barrier(W, D, T) + 64; }
-
-__device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* p)
-{
-    uint32_t v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_sys(uint32_t* p, uint32_t v)
-{
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-// waits until *flag has reached `epoch`; false (and the error flag) after 4 s, or at once when the flag is already set
-__device__ __forceinline__ bool peer_wait(const uint32_t* flag, uint32_t epoch, int32_t* error)
-{
-    unsigned long long t0 = 0;
-    int polls = 0;
-    while ((int32_t)(ld_acquire_sys(flag) - epoch) < 0) {
-        if (++polls == 256) {
-            polls = 0;
-            if (*(volatile int32_t*)error) return false;
-            const unsigned long long now = global_timer_ns();
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ull) { atomicExch(error, 1); return false; }
-        }
-    }
-    return true;
-}
-// one double as two tagged words, 16 bytes at dst (16-byte aligned)
-__device__ __forceinline__ void ll_store(unsigned char* dst, double v, uint32_t epoch)
-{
-    const unsigned long long bits = (unsigned long long)__double_as_longlong(v), tag = (unsigned long long)epoch << 32;
-    const unsigned long long w0 = tag | (bits & 0xffffffffull), w1 = tag | (bits >> 32);
-    asm volatile("st.volatile.global.v2.u64 [%0], {%1, %2};" ::"l"(dst), "l"(w0), "l"(w1) : "memory");
-}
-// spins until both words at src carry `epoch`; 0.0 (and the error flag) after 4 s
-__device__ __forceinline__ double ll_load(const unsigned char* src, uint32_t epoch, int32_t* error)
-{
-    unsigned long long w0, w1, t0 = 0;
-    int polls = 0;
-    for (;;) {
-        asm volatile("ld.volatile.global.v2.u64 {%0, %1}, [%2];" : "=l"(w0), "=l"(w1) : "l"(src) : "memory");
-        if ((uint32_t)(w0 >> 32) == epoch && (uint32_t)(w1 >> 32) == epoch) break;
-        if (++polls == 256) {
-            polls = 0;
-            if (*(volatile int32_t*)error) return 0.0;
-            const unsigned long long now = global_timer_ns();
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ull) { atomicExch(error, 1); return 0.0; }
-        }
-    }
-    return __longlong_as_double((long long)((w1 << 32) | (w0 & 0xffffffffull)));
-}
-
-// all ranks meet on the device (timer brackets of a sharded run start together); one warp
-__global__ void peer_barrier_kernel(const __grid_constant__ PeerExchange px, uint32_t ticket)
-{
-    const int r = threadIdx.x;
-    if (r >= px.world) return;
-    const size_t off = peer_off_barrier(px.world, px.D, px.T);
-    st_release_sys(reinterpret_cast<uint32_t*>(px.box[r] + off) + px.rank, ticket);
-    peer_wait(reinterpret_cast<const uint32_t*>(px.box[px.rank] + off) + r, ticket, px.error);
-}
-
-// K7 + K8 + K9 of a rollout-sharded engine (one query): weights_update_kernel with the two exchanges inside.
-// grid: nchunks * D CTAs in one dimension; the D CTAs that publish exchange A come first in dispatch order and no CTA
-// ever waits for another CTA of its own grid before publishing, so the spins cannot starve a publisher of an SM.
-__global__ void __launch_bounds__(kUpdateThreads)
-weights_update_peer_kernel(const __grid_constant__ LoopParams p, const __grid_constant__ PeerExchange px)
-{
-    extern __shared__ double smem[];   // [chunk] weights, [chunk] weight * quad ; later [T + 2] column sums
-    __shared__ double scratch[32];
-    __shared__ double s_half[128];
-    __shared__ double s_mm[2 * kMaxPeers];
-    __shared__ int s_last;
-    const int q = 0;
-    pdl_trigger_and_wait();
-    if (p.counters && blockIdx.x == 0 && threadIdx.x == 0) p.counters[0] += 1u;              // next iteration number (graph replay)
-    if (query_frozen(p, q)) return;
-    TimelineScope tls(p, 3);
-    const int T = p.T, D = p.D, tid = threadIdx.x, W = px.world, rank = px.rank;
-    const int nchunks = p.nchunks;
-    int c, d;
-    if ((int)blockIdx.x < D) { c = 0; d = blockIdx.x; }
-    else { const int r = blockIdx.x - D; d = r / (nchunks - 1); c = 1 + (r - d * (nchunks - 1)); }
-    const uint32_t epoch = px.epoch_ptr ? __ldcg(px.epoch_ptr) : px.epoch;
-    const int parity = (int)(epoch & 1u);
-    const int half = tid >> 7, lt = tid & 127;
-    const int k_begin = c * p.chunk, k_end = min(p.num_local, (c + 1) * p.chunk);
-    const int nk = k_end - k_begin;
-    double* sp = smem;
-    double* sq = smem + p.chunk;
-    if (c == 0 && d == 0 && p.noiseless_slot >= 0) materialise_noiseless(p, q, tid, blockDim.x);
-
-    // ---- min / max of cumulative_costs_[d] over this rank's rollouts; exchange A ----
-    const double* S = p.s_compact + (size_t)q * p.gslots;
-    const double* C = p.c_compact + ((size_t)q * D + d) * p.gslots;
-    const double* nl = p.nl_sums + (size_t)q * p.sumw;
-    auto cum_of = [&](int g) { return (g == p.noiseless_gslot) ? 1.0 * (nl[0] + nl[1 + d]) : 1.0 * (S[g] + C[g]); };
-    double mn = 1e300, mx = -1e300;
-#pragma unroll 8
-    for (int k = tid; k < p.num_gen; k += kUpdateThreads) {
-        const double cum = cum_of(p.gen_offset + k);
-        mn = fmin(mn, cum); mx = fmax(mx, cum);
-    }
-    if (tid == 0 && p.noiseless_gslot >= 0) { const double cum = cum_of(p.noiseless_gslot); mn = fmin(mn, cum); mx = fmax(mx, cum); }
-    mn = block_reduce<1>(mn, scratch); mx = block_reduce<2>(mx, scratch);
-    const size_t slot_mine = ((size_t)parity * W + rank) * D + d;
-    if (c == 0 && tid < W && tid != rank) {
-        unsigned char* dst = px.box[tid] + slot_mine * 32;
-        ll_store(dst, mn, epoch);
-        ll_store(dst + 16, mx, epoch);
-    }
-    if (tid < W) {
-        double vmn = mn, vmx = mx;
-        if (tid != rank) {
-            const unsigned char* src = px.box[rank] + (((size_t)parity * W + tid) * D + d) * 32;
-            vmn = ll_load(src, epoch, px.error);
-            vmx = ll_load(src + 16, epoch, px.error);
-        }
-        s_mm[2 * tid] = vmn; s_mm[2 * tid + 1] = vmx;
-    }
-    __syncthreads();
-    for (int r = 0; r < W; ++r) { mn = fmin(mn, s_mm[2 * r]); mx = fmax(mx, s_mm[2 * r + 1]); }
-    double den = mx - mn;
-    if (den < 1e-8) den = 1e-8;
-    const double h = p.cost_scaling_h;
-
-    // ---- unnormalised weights of this chunk ----
-    double psum_part = 0.0;
-    for (int k = k_begin + tid; k < k_end; k += blockDim.x) {
-        const int g = (k == p.noiseless_slot) ? p.noiseless_gslot : p.gen_offset + k;
-        const double pr = 1.0 * exp(((-h) * (cum_of(g) - mn)) / den);      // importance_weight_ = 1
-        const size_t o = ((size_t)q * p.gslots + g) * D + d;
-        p.prob[o] = pr;
-        p.fprob[o] = pr;
-        // the noise-less rollout is replicated on every rank: only the first rank counts it in the sum of the weights
-        if (!(k == p.noiseless_slot && rank != 0)) psum_part += pr;
-        double w = pr, fq = 0.0;
-        if (k == p.noiseless_slot) w = 0.0;       // zero noise: contributes nothing (PolicyImprovement.cpp:407-410)
-        else if (p.use_noise_adaptation) fq = pr * p.sums[((size_t)q * p.gslots + g) * p.sumw + 1 + 2 * D + d];
-        sp[k - k_begin] = w;
-        sq[k - k_begin] = fq;
-        if (d == 0) {   // total_cost_ (:451-462)
-            const double* s = cost_row(p, q, g);
-            double cost = s[0];
-            for (int dd = 0; dd < D; ++dd) cost += s[1 + dd];
-            p.total_cost[(size_t)q * p.gslots + g] = cost;
-        }
-    }
-    __syncthreads();
-    double* out = p.partial + (((size_t)q * nchunks + c) * D + d) * (T + 2);
-    for (int t0 = 0; t0 < T; t0 += 128) {
-        const int t = t0 + lt;
-        double acc = 0.0;
-        if (t < T) {
-            const bool from_rollouts = p.noise_from_rollouts != 0;
-            const double* nz = (from_rollouts ? p.rollouts : p.noise) + (((size_t)q * p.slots + k_begin) * D + d) * T + t;
-            const double th_t = from_rollouts ? p.theta_all[((size_t)q * D + d) * p.N + kPad + t] : 0.0;
-            const size_t stride = (size_t)D * T;
-            double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-            int k = half;
-            for (; k + 30 < nk; k += 32) {       // rows k, k+2, ..., k+30
-                double v[16];
-#pragma unroll
-                for (int u = 0; u < 16; ++u) v[u] = nz[(size_t)(k + 2 * u) * stride] - th_t;
-#pragma unroll
-                for (int u = 0; u < 16; u += 4) {
-                    a0 += v[u] * sp[k + 2 * u]; a1 += v[u + 1] * sp[k + 2 * u + 2];
-                    a2 += v[u + 2] * sp[k + 2 * u + 4]; a3 += v[u + 3] * sp[k + 2 * u + 6];
-                }
-            }
-            for (; k < nk; k += 2) a0 += (nz[(size_t)k * stride] - th_t) * sp[k];
-            acc = (a0 + a1) + (a2 + a3);
-        }
-        if (half == 1) s_half[lt] = acc;
-        __syncthreads();
-        if (half == 0 && t < T) out[t] = acc + s_half[lt];
-        __syncthreads();
-    }
-    double numer = 0.0;
-    for (int k = tid; k < nk; k += blockDim.x) numer += sq[k];
-    numer = block_reduce<0>(numer, scratch);
-    psum_part = block_reduce<0>(psum_part, scratch);
-    if (tid == 0) { out[T] = numer; out[T + 1] = psum_part; }
-
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) s_last = (atomicAdd(p.done_counter + (size_t)q * D + d, 1u) == (unsigned)nchunks - 1u) ? 1 : 0;
-    __syncthreads();
-    if (s_last) {
-        __threadfence();
-        // ---- exchange B: this rank's sums in chunk order -> every mailbox; then all ranks' rows in rank order ----
-        const size_t offb = peer_off_b(W, D);
-        for (int t = tid; t < T + 2; t += blockDim.x) {
-            double mine = 0.0;
-            const double* col = p.partial + ((size_t)q * nchunks * D + d) * (T + 2) + t;
-            const size_t stride = (size_t)D * (T + 2);
-#pragma unroll 8
-            for (int cc = 0; cc < nchunks; ++cc) mine += __ldcg(col + (size_t)cc * stride);
-            for (int r = 0; r < W; ++r)
-                if (r != rank) ll_store(px.box[r] + offb + (slot_mine * (T + 2) + t) * 16, mine, epoch);
-            double u = 0.0;
-            for (int r = 0; r < W; ++r)
-                u += (r == rank) ? mine : ll_load(px.box[rank] + offb + ((((size_t)parity * W + r) * D + d) * (T + 2) + t) * 16, epoch, px.error);
-            smem[t] = u;
-        }
-        apply_update_body(p, q, d, 3, nchunks, smem);
-        if (tid == 0) p.done_counter[(size_t)q * D + d] = 0u;
-    }
+    apply_update_body(p, q, d, (UpdateSums)sums, nchunks, smem);
     tls.end();
 }
 

@@ -64,6 +64,11 @@ def test_invalid_configurations_are_rejected_before_touching_the_device():
     assert L.stomp_b200_create(ctypes.byref(cfg), ctypes.byref(h)) == binding.ERR_UNSUPPORTED
     cfg.use_cumulative_costs, cfg.shard_mode = 1, 7       # no such sharding mode
     assert L.stomp_b200_create(ctypes.byref(cfg), ctypes.byref(h)) == -1
+    cfg.shard_mode, cfg.world_size, cfg.rank = 0, 2, 0    # rollout sharding ...
+    cfg.min_rollouts, cfg.max_rollouts, cfg.num_rollouts_per_iteration = 4, 8, 4   # ... with rollout reuse
+    assert L.stomp_b200_create(ctypes.byref(cfg), ctypes.byref(h)) == binding.ERR_UNSUPPORTED
+    cfg.min_rollouts, cfg.max_rollouts, cfg.num_rollouts_per_iteration = 5, 5, 5   # ... with shards of unequal size
+    assert L.stomp_b200_create(ctypes.byref(cfg), ctypes.byref(h)) == binding.ERR_UNSUPPORTED
     assert L.stomp_b200_status_string(-2).decode().startswith("no CUDA device")
 
 

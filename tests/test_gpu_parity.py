@@ -528,16 +528,24 @@ def test_trajectory_lengths_cover_every_kernel_variant(T):
 def test_unfused_weights_and_update_kernels_match_the_fused_kernel(monkeypatch):
     """Single-GPU runs use weights_update_kernel (K7-K9 in one launch); multi-GPU, rollout reuse and the per-kernel
     profiling pass use rollout_weights_kernel -> weighted_update_kernel -> apply_update_kernel.  K' = 1101 makes the
-    unfused weights kernel run three CTAs per joint (partial sums in wpart) and the update nine chunks."""
+    unfused weights kernel run three CTAs per joint (partial sums in wpart) and the update nine chunks.  With
+    STOMP_B200_FUSE_WEIGHTS=0 the apply step rides on weighted_update_kernel's last chunk CTA; profiling splits it off
+    into apply_update_kernel, which adds the same partials in the same chunk order: bit-identical."""
     pb = P.single_arm_problem(K=1100, T=40, sdf_n=64)
     fused = binding.engine_for_problem(pb, keep_debug_tensors=True)
     monkeypatch.setenv("STOMP_B200_FUSE_WEIGHTS", "0")
     unfused = binding.engine_for_problem(pb, keep_debug_tensors=True)
     monkeypatch.delenv("STOMP_B200_FUSE_WEIGHTS")
-    fused.begin_solve(); unfused.begin_solve()
+    profiled = binding.engine_for_problem(pb, keep_debug_tensors=True)
+    profiled.set_profiling(True)
+    fused.begin_solve(); unfused.begin_solve(); profiled.begin_solve()
     for it in range(4):
         c1, v1, s1 = fused.iterate(it)
         c2, v2, s2 = unfused.iterate(it)
+        c3, v3, s3 = profiled.iterate(it)
+        for name in ("epsilon", "verdicts", "total_cost", "probabilities", "full_probabilities", "updates", "parameters", "stddevs"):
+            np.testing.assert_array_equal(profiled.tensor(name)[0], unfused.tensor(name)[0], err_msg=name)
+        np.testing.assert_array_equal(c3, c2)
         np.testing.assert_array_equal(fused.tensor("epsilon")[0], unfused.tensor("epsilon")[0])
         np.testing.assert_array_equal(fused.tensor("verdicts")[0], unfused.tensor("verdicts")[0])
         for name in ("total_cost", "probabilities", "full_probabilities", "updates", "parameters", "stddevs"):

@@ -3,15 +3,16 @@
 // One engine = one GPU; a main stream plus two helper streams for the fallback paths (control-cost rows beside the state
 // kernel; a two-kernel noise-less rollout under the next iteration's sampling).  The per-iteration sequence mirrors
 // stomp::Stomp::runSingleIteration (reference src/planners/stomp/src/Stomp.cpp:274-301); shipped loop first, fallbacks after |:
-//   doGenRollouts      -> [reuse_rollouts_kernel] sample_rollouts_banded_kernel (recurrence through the banded L^-1, control-cost
-//                         rows fused; draws before it waits for the previous update kernel) | sample_rollouts_dmma_kernel
-//                         (injected epsilon, factors without a band table) | sample_rollouts_kernel | shift_rollouts_kernel
+//   doGenRollouts      -> [reuse_rollouts_kernel], then launch_generate_stage, in the shape generate_shape classifies the
+//                         iteration into: sample_rollouts_banded_kernel (recurrence through the banded L^-1, control-cost rows
+//                         fused; draws before it waits for the previous update kernel) | sample_rollouts_dmma_kernel (injected
+//                         epsilon, factors without a band table) | shift_rollouts_kernel (injected unit noise)
 //   doExecuteRollouts  -> a state pass (launch_state_pass, also for the noise-less rollout and stomp_b200_evaluate_states):
 //                         stomp_b200_states_specialised (generated, state_codegen.hpp; static spheres once per scene by
 //                         stomp_b200_static_spheres) | rollout_states_kernel; states_self_collision_kernel / the generated
 //                         pair-rule kernel with a sphere-pair list; then state_cost_extras_kernel for the alternative costs
-//   setRolloutCosts    -> inside the sampler | control_rows_tile_kernel | control_rows_fast_kernel | control_rows_kernel
-//                         [reused_control_cost_kernel]
+//   setRolloutCosts    -> inside the sampler | launch_generate_stage: control_rows_tile_kernel | control_rows_fast_kernel |
+//                         control_rows_kernel, behind project_noise_dmma_kernel with use_projection; [reused_control_cost_kernel]
 //   improvePolicy + updateParameters
 //                      -> launch_update_stage, in the shape update_shape classifies the iteration into: weights_update_kernel on
 //                         one GPU, weights_update_peer_kernel (both exchanges over NVLink mailboxes) on rollout shards | with the
@@ -101,6 +102,10 @@ NcclApi g_nccl;
 
 struct ProfiledLaunch { int kernel; cudaEvent_t a, b; };
 
+// STOMP_B200_SAMPLER at creation: "dmma" the contraction for on-device noise too, "banded" the recurrence for injected
+// epsilon too; unset or any other value the default (generate_shape)
+enum class SamplerSwitch { kDefault, kContraction, kRecurrence };
+
 }  // namespace
 
 struct stomp_b200_engine {
@@ -136,7 +141,7 @@ struct stomp_b200_engine {
     LoopParams base;                // pointers + constants; per-iteration fields filled in iterate
     double* proj2[2] = {nullptr, nullptr};
     double* d_Lband = nullptr;               // [T][8] rows of L^-1 for the recurrence sampler
-    int sampler_mode = 0;                    // 0 recurrence (default), 1 DMMA contraction, 2 FMA-pipe contraction (STOMP_B200_SAMPLER)
+    SamplerSwitch sampler_switch = SamplerSwitch::kDefault;
     double* d_Mproj = nullptr; double* d_Minv = nullptr;   // projection_matrix_ / its inverse (use_projection only)
     double* state2[2] = {nullptr, nullptr};
     uint8_t* verdict2[2] = {nullptr, nullptr};
@@ -144,7 +149,6 @@ struct stomp_b200_engine {
     int32_t* d_order = nullptr;
     int max_chunks = 1;
     int num_sms = 148;
-    bool use_dmma = true;                    // STOMP_B200_SAMPLER=simt selects the FMA-pipe contraction
     cudaStream_t side_stream = nullptr;      // noise-less rollout, overlapped with the next iteration's sampling + costs
     cudaEvent_t ev_applied = nullptr, ev_noiseless = nullptr;
     cudaStream_t rows_stream = nullptr;      // control-cost rows, side by side with the state kernel
@@ -402,16 +406,27 @@ size_t dmma_smem_bytes(int T)
     return sizeof(double) * (size_t)dmma_slab_rows(T) * dmma_slab_stride(dmma_tiles_for(T));
 }
 
-// FP64 tensor-core contraction (DMMA); used whenever the Lt slab fits in shared memory
+// Raises a kernel's limit of dynamic shared memory to `bytes`, once per engine: the attribute belongs to the device, and one
+// engine is one device.
+cudaError_t opt_in_smem(stomp_b200_engine* e, const void* kernel, int bytes)
+{
+    if (e->smem_opted_in.count(kernel)) return cudaSuccess;
+    const cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (err == cudaSuccess) e->smem_opted_in.insert(kernel);
+    return err;
+}
+
+// The Lt slab of the contraction sampler fits at every T a configuration may have: dmma_slab_rows(T) rows of at most
+// kSlabTilesMax n8 tiles, 217,088 B (212 KB) at T = STOMP_B200_MAX_TIME_STEPS = 256.
+constexpr int kDmmaSmemOptIn = 225 * 1024;
+static_assert(sizeof(double) * dmma_slab_rows(STOMP_B200_MAX_TIME_STEPS) * dmma_slab_stride(kSlabTilesMax) <= kDmmaSmemOptIn,
+              "the contraction sampler's Lt slab must fit in shared memory at every trajectory length");
+
+// FP64 tensor-core contraction (DMMA)
 template <int kTiles, bool kPhilox>
 int launch_sample_dmma_t(stomp_b200_engine* e, const LoopParams& lp)
 {
-    // the attribute is per device: remembered per engine (one engine = one device), not per process
-    const void* fn = (const void*)sample_rollouts_dmma_kernel<kTiles, kPhilox>;
-    if (!e->smem_opted_in.count(fn)) {
-        CUDA_TRY(e, cudaFuncSetAttribute(sample_rollouts_dmma_kernel<kTiles, kPhilox>, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024));
-        e->smem_opted_in.insert(fn);
-    }
+    CUDA_TRY(e, opt_in_smem(e, (const void*)sample_rollouts_dmma_kernel<kTiles, kPhilox>, kDmmaSmemOptIn));
     const long long total_cols = (long long)lp.Q * lp.num_gen * lp.D;
     const int ntiles = (int)((total_cols + 7) / 8);
     const int nslabs = (lp.T + 8 * kTiles - 1) / (8 * kTiles);
@@ -434,21 +449,20 @@ int launch_sample_dmma(stomp_b200_engine* e, const LoopParams& lp)
     }
 }
 
+// recurrence sampler (L^-1 is banded); fuse: control-cost sums + n^T R n in the same pass
 template <bool kPhilox>
-int launch_sample(stomp_b200_engine* e, const LoopParams& lp)
+int launch_sample_banded(stomp_b200_engine* e, const LoopParams& lp, bool fuse)
 {
-    if (e->use_dmma && dmma_smem_bytes(lp.T) <= 220 * 1024) return launch_sample_dmma<kPhilox>(e, lp);
-    const int ncols = lp.num_gen * lp.D;
-    dim3 grid((ncols + 63) / 64, lp.Q);
-    const int need = (lp.T + 15) / 16;
+    const int band = lp.lband_halfwidth <= 4 ? 4 : 6;
+    const void* kernel = band == 4 ? (fuse ? (const void*)sample_rollouts_banded_kernel<4, kPhilox, true> : (const void*)sample_rollouts_banded_kernel<4, kPhilox, false>)
+                                   : (fuse ? (const void*)sample_rollouts_banded_kernel<6, kPhilox, true> : (const void*)sample_rollouts_banded_kernel<6, kPhilox, false>);
+    const size_t smem = sizeof(double) * banded_sampler_smem_doubles(lp.T, lp.N, band);
+    if (smem > 48 * 1024) CUDA_TRY(e, opt_in_smem(e, kernel, 120 * 1024));      // long trajectories: the 32 x T tile passes 48 KB
+    const int nkb = (lp.num_gen + 31) / 32;
     Scope s(e, STOMP_B200_KERNEL_SAMPLE);
-    if (need <= 2) sample_rollouts_kernel<2, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    else if (need <= 4) sample_rollouts_kernel<4, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    else if (need <= 7) sample_rollouts_kernel<7, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    else if (need <= 10) sample_rollouts_kernel<10, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    else if (need <= 13) sample_rollouts_kernel<13, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    else sample_rollouts_kernel<16, kPhilox><<<grid, 256, 0, e->stream>>>(lp, e->limits);
-    return check_launch(e, "sample_rollouts_kernel");
+    void* args[] = {const_cast<LoopParams*>(&lp), &e->limits};
+    CUDA_TRY(e, launch_dependent(e, 0, kernel, dim3((unsigned)(nkb * lp.D), (unsigned)lp.Q), dim3(kBandedThreads), smem, e->stream, args));
+    return check_launch(e, "sample_rollouts_banded_kernel");
 }
 
 enum NoiseMode { kNoisePhilox = 0, kNoiseUnit = 1, kNoiseEpsilon = 2 };
@@ -466,28 +480,6 @@ RowsShape rows_shape(const stomp_b200_engine* e, const LoopParams& lp)
     return lp.rband_halfwidth <= 4 ? kRowsTile : kRowsWindow;
 }
 
-// recurrence sampler (L^-1 is banded); fuse: control-cost sums + n^T R n in the same pass
-template <bool kPhilox>
-int launch_sample_banded(stomp_b200_engine* e, const LoopParams& lp, bool fuse)
-{
-    const int nkb = (lp.num_gen + 31) / 32;
-    const dim3 grid((unsigned)(nkb * lp.D), (unsigned)lp.Q);
-    const size_t smem = sizeof(double) * banded_sampler_smem_doubles(lp.T, lp.N, lp.lband_halfwidth <= 4 ? 4 : 6);
-    auto launch = [&](auto kernel) -> int {
-        const void* fn = (const void*)kernel;
-        if (smem > 48 * 1024 && !e->smem_opted_in.count(fn)) {       // long trajectories: the 32 x T tile passes 48 KB
-            CUDA_TRY(e, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024));
-            e->smem_opted_in.insert(fn);
-        }
-        Scope s(e, STOMP_B200_KERNEL_SAMPLE);
-        void* args[] = {const_cast<LoopParams*>(&lp), &e->limits};
-        CUDA_TRY(e, launch_dependent(e, 0, (const void*)kernel, grid, dim3(kBandedThreads), smem, e->stream, args));
-        return check_launch(e, "sample_rollouts_banded_kernel");
-    };
-    if (lp.lband_halfwidth <= 4) return fuse ? launch(sample_rollouts_banded_kernel<4, kPhilox, true>) : launch(sample_rollouts_banded_kernel<4, kPhilox, false>);
-    return fuse ? launch(sample_rollouts_banded_kernel<6, kPhilox, true>) : launch(sample_rollouts_banded_kernel<6, kPhilox, false>);
-}
-
 // one Stomp::runSingleIteration for all local queries, queued on the stream (no host synchronisation)
 // eight-rows-per-warp control-cost kernel (kernels.cuh): instantiated for the group counts of the usual T
 template <int kGroups>
@@ -495,14 +487,10 @@ bool launch_rows_tile_g(stomp_b200_engine* e, const LoopParams& lp, int rows, cu
 {
     const size_t smem = sizeof(double) * (size_t)kTileWarps * 8 * tile_noise_stride(kGroups);
     const dim3 grid((rows + kTileWarps * 8 - 1) / (kTileWarps * 8), lp.Q);
-    const void* fn = (const void*)control_rows_tile_kernel<kGroups, false>;      // per engine = per device
-    if (!e->smem_opted_in.count(fn)) {
-        if (cudaFuncSetAttribute(control_rows_tile_kernel<kGroups, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(control_rows_tile_kernel<kGroups, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
-            (void)cudaGetLastError();
-            return false;
-        }
-        e->smem_opted_in.insert(fn);
+    if (opt_in_smem(e, (const void*)control_rows_tile_kernel<kGroups, false>, 200 * 1024) != cudaSuccess ||
+        opt_in_smem(e, (const void*)control_rows_tile_kernel<kGroups, true>, 200 * 1024) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return false;     // the caller launches control_rows_fast_kernel instead
     }
     if (smem > 200 * 1024) return false;
     // (Capping this grid's residency so that it shares every SM with the state kernel was tried — 32 KB of shared memory
@@ -757,6 +745,108 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
     return 0;
 }
 
+// The generate stage (K1-K3: sampling; K5, K6: the control costs and n^T R n of the generated rows) in the shape
+// generate_shape classifies an iteration into.
+enum class Sampler {
+    kRecurrence,    // sample_rollouts_banded_kernel through the banded L^-1: on-device noise, or STOMP_B200_SAMPLER=banded
+    kContraction,   // sample_rollouts_dmma_kernel with the caller's L: injected epsilon, no band table, or STOMP_B200_SAMPLER=dmma
+    kShift,         // shift_rollouts_kernel: injected unit noise
+};
+enum class RowsWork {
+    kNone,          // the fused recurrence sampler left C_d and n^T R n, and no per-time-step control cost is kept
+    kStore,         // the fused recurrence sampler left the sums; the row kernel stores only the per-time-step control costs
+                    // that read-backs and the per-time-step mode need (rows_mask 0)
+    kRows,          // the row kernel computes the control costs and n^T R n
+    kProjection,    // project_noise_dmma_kernel, then a row pass for the control costs and one for n^T R n
+};
+struct GenerateShape {
+    Sampler sampler;
+    bool philox;            // on-device noise (else the caller's epsilon or unit noise)
+    bool fused_rows;        // the recurrence sampler computes the control-cost sums and n^T R n itself
+    RowsWork rows;
+    RowsShape rows_kind;
+    bool overlap;           // the rows run on rows_stream beside the state kernel
+};
+
+// Reads the engine only, not an iteration's parameters, so that iterate_async can ask before it builds them.  Projection
+// is tested as base.Mproj != nullptr rather than cfg.use_projection: an iteration runs only once the control-cost matrices
+// are set (ready_to_solve), and stomp_b200_set_control_cost_matrices sets Mproj exactly when use_projection is on.
+GenerateShape generate_shape(const stomp_b200_engine* e, int mode)
+{
+    const LoopParams& b = e->base;
+    GenerateShape g;
+    g.philox = mode == kNoisePhilox;
+    const bool recurrence = b.Lband != nullptr && (e->sampler_switch == SamplerSwitch::kRecurrence ||
+                                                   (g.philox && e->sampler_switch == SamplerSwitch::kDefault));
+    g.sampler = mode == kNoiseUnit ? Sampler::kShift : (recurrence ? Sampler::kRecurrence : Sampler::kContraction);
+    g.rows_kind = rows_shape(e, b);
+    g.fused_rows = g.sampler == Sampler::kRecurrence && !b.Mproj && g.rows_kind == kRowsTile;
+    if (b.Mproj) g.rows = RowsWork::kProjection;
+    else if (g.fused_rows) g.rows = b.control_costs ? RowsWork::kStore : RowsWork::kNone;
+    else g.rows = RowsWork::kRows;
+    // the rows and the state costs (K4) are independent of each other (different columns of `sums`) and both latency-bound
+    // at < 50 % occupancy: side by side on two streams, serial on the main stream while per-kernel profiling is on
+    g.overlap = g.rows != RowsWork::kNone && !e->profiling && e->rows_stream != nullptr;
+    return g;
+}
+
+// K1-K6 of an iteration in shape g: the padding-only control-cost rows when the policy changed, the sampler, then the rows
+// of the generated rollouts.  With g.overlap the rows go to rows_stream and ev_rows marks their end; the caller makes the
+// main stream wait for it after the state pass.
+int launch_generate_stage(stomp_b200_engine* e, const LoopParams& lp, const GenerateShape& g)
+{
+    // padding-only rows of the control costs: constants of a solve, needed by the fused sampler and the row kernels
+    if (e->edge_dirty && lp.num_rules == 1) {
+        edge_rows_kernel<<<e->Q, 64, 0, e->stream>>>(lp);
+        e->launch_count++;
+        if (int rc = check_launch(e, "edge_rows_kernel")) return rc;
+        e->edge_dirty = false;
+    }
+    switch (g.sampler) {
+    case Sampler::kRecurrence:
+        if (int rc = g.philox ? launch_sample_banded<true>(e, lp, g.fused_rows) : launch_sample_banded<false>(e, lp, g.fused_rows)) return rc;
+        break;
+    case Sampler::kContraction:
+        if (int rc = g.philox ? launch_sample_dmma<true>(e, lp) : launch_sample_dmma<false>(e, lp)) return rc;
+        break;
+    case Sampler::kShift: {
+        Scope sc(e, STOMP_B200_KERNEL_SAMPLE);
+        const int per_query = lp.num_gen * e->D * e->T;
+        shift_rollouts_kernel<<<dim3(std::min(1024, (per_query + 255) / 256), e->Q), 256, 0, e->stream>>>(lp, e->limits);
+        if (int rc = check_launch(e, "shift_rollouts_kernel")) return rc;
+        break;
+    }
+    }
+    if (g.rows == RowsWork::kNone) return 0;
+    cudaStream_t rows_stream = g.overlap ? e->rows_stream : e->stream;
+    if (g.overlap) {
+        CUDA_TRY(e, cudaEventRecord(e->ev_sampled, e->stream));
+        CUDA_TRY(e, cudaStreamWaitEvent(rows_stream, e->ev_sampled, 0));
+    }
+    {
+        const int rows = lp.num_gen * e->D;
+        Scope sc(e, STOMP_B200_KERNEL_ROWS);
+        if (g.rows == RowsWork::kProjection) {
+            // M-projection (PolicyImprovement.cpp:421-440): noise_projected_ = M * noise_ for the generated rollouts, then
+            // the control costs from parameters_ + noise_projected_ (:812-817) and n^T R n from noise_ (:656-663)
+            project_noise_dmma_kernel<<<dim3((rows + 31) / 32, (e->T + 63) / 64, e->Q), 128, 0, rows_stream>>>(lp);
+            e->launch_count++;
+            if (int rc = check_launch(e, "project_noise_dmma_kernel")) return rc;
+            LoopParams cpass = lp; cpass.rows_noise = lp.noise_proj; cpass.rows_mask = 1;
+            if (int rc = launch_rows(e, cpass, g.rows_kind, rows, rows_stream)) return rc;
+            LoopParams qpass = lp; qpass.rows_noise = lp.noise; qpass.rows_mask = 2; qpass.control_costs = nullptr;
+            e->launch_count++;
+            if (int rc = launch_rows(e, qpass, g.rows_kind, rows, rows_stream)) return rc;
+        } else if (g.rows == RowsWork::kStore) {
+            LoopParams store = lp; store.rows_mask = 0;
+            if (int rc = launch_rows(e, store, g.rows_kind, rows, rows_stream)) return rc;
+        } else if (int rc = launch_rows(e, lp, g.rows_kind, rows, rows_stream)) {
+            return rc;
+        }
+    }
+    if (g.overlap) CUDA_TRY(e, cudaEventRecord(e->ev_rows, rows_stream));
+    return 0;
+}
 
 // The update stage (K7-K9: computeRolloutProbabilities, computeParameterUpdates, updateParameters) takes one of four shapes.
 // Every rank of a sharded engine classifies alike: the fields involved are set alike on all ranks.
@@ -934,77 +1024,14 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
         e->base.proj = lp.proj; e->base.state_costs = lp.state_costs; e->base.verdicts = lp.verdicts;
     }
 
-    // padding-only rows of the control costs: constants of a solve, needed by the fused sampler and the row kernels
-    if (e->edge_dirty && lp.num_rules == 1) {
-        edge_rows_kernel<<<e->Q, 64, 0, e->stream>>>(lp);
-        e->launch_count++;
-        if (int rc = check_launch(e, "edge_rows_kernel")) return rc;
-        e->edge_dirty = false;
-    }
-    // ---- generate (K1-K3) ----
-    // on-device noise goes through the recurrence sampler (L^-1 is banded) with the control-cost rows fused in; injected
-    // epsilon goes through the contraction with the caller's L (parity mode) unless STOMP_B200_SAMPLER=banded
-    const bool banded = lp.Lband != nullptr && mode != kNoiseUnit &&
-                        ((mode == kNoisePhilox && (e->sampler_mode == 0 || e->sampler_mode == 3)) || (mode == kNoiseEpsilon && e->sampler_mode == 3));
-    const RowsShape rows_kind = rows_shape(e, lp);
-    const bool fused_rows = banded && !lp.Mproj && rows_kind == kRowsTile;
+    // ---- generate (K1-K6) ----
+    const GenerateShape gen_shape = generate_shape(e, mode);
     // the shipped large-K loop (fused sampler, fused weights / update kernel, nothing reads `noise` back): the noise
     // tensor is not materialised — the update kernel subtracts theta from the rollout rows it streams
     const UpdateShape shape = update_shape(e, world);
     const bool one_update_launch = shape == UpdateShape::kFused || shape == UpdateShape::kPeer;
-    lp.noise_from_rollouts = (fused_rows && one_update_launch && !c.keep_debug_tensors && !lp.control_costs && !lp.proj) ? 1 : 0;
-    if (banded) {
-        if (int rc = (mode == kNoisePhilox ? launch_sample_banded<true>(e, lp, fused_rows) : launch_sample_banded<false>(e, lp, fused_rows))) return rc;
-    } else if (mode == kNoiseUnit) {
-        Scope sc(e, STOMP_B200_KERNEL_SAMPLE);
-        const int per_query = gen_local * e->D * e->T;
-        dim3 grid(std::min(1024, (per_query + 255) / 256), e->Q);
-        shift_rollouts_kernel<<<grid, 256, 0, e->stream>>>(lp, e->limits);
-        if (int rc = check_launch(e, "shift_rollouts_kernel")) return rc;
-    } else if (mode == kNoiseEpsilon) {
-        if (int rc = launch_sample<false>(e, lp)) return rc;
-    } else {
-        if (int rc = launch_sample<true>(e, lp)) return rc;
-    }
-
-    // ---- control costs + n^T R n of the generated rows (K5, K6) and the state costs (K4): independent of each
-    // other (different columns of `sums`), both latency-bound at < 50 % occupancy -> run side by side on two
-    // streams; serial on the main stream while per-kernel profiling is on ----
-    const bool rows_needed = !(fused_rows && !lp.control_costs);      // the fused sampler already left C_d and n^T R n
-    const bool overlap_rows = !e->profiling && e->rows_stream != nullptr && rows_needed;
-    cudaStream_t rows_stream = overlap_rows ? e->rows_stream : e->stream;
-    if (overlap_rows) {
-        CUDA_TRY(e, cudaEventRecord(e->ev_sampled, e->stream));
-        CUDA_TRY(e, cudaStreamWaitEvent(rows_stream, e->ev_sampled, 0));
-    }
-    {
-        const int rows = gen_local * e->D;
-        Scope sc(e, STOMP_B200_KERNEL_ROWS);
-        if (lp.Mproj) {
-            // M-projection (PolicyImprovement.cpp:421-440): noise_projected_ = M * noise_ for the generated rollouts, then
-            // the control costs from parameters_ + noise_projected_ (:812-817) and n^T R n from noise_ (:656-663)
-            project_noise_dmma_kernel<<<dim3((rows + 31) / 32, (e->T + 63) / 64, e->Q), 128, 0, rows_stream>>>(lp);
-            e->launch_count++;
-            if (int rc = check_launch(e, "project_noise_dmma_kernel")) return rc;
-            LoopParams cpass = lp; cpass.rows_noise = lp.noise_proj; cpass.rows_mask = 1;
-            if (int rc = launch_rows(e, cpass, rows_kind, rows, rows_stream)) return rc;
-            LoopParams qpass = lp; qpass.rows_noise = lp.noise; qpass.rows_mask = 2; qpass.control_costs = nullptr;
-            e->launch_count++;
-            if (int rc = launch_rows(e, qpass, rows_kind, rows, rows_stream)) return rc;
-        } else if (fused_rows) {
-            // the sampler left C_d and n^T R n; only the per-time-step control costs (read-backs, per-time-step mode) are missing
-            if (lp.control_costs) {
-                LoopParams store = lp; store.rows_mask = 0;
-                if (int rc = launch_rows(e, store, rows_kind, rows, rows_stream)) return rc;
-            } else {
-                e->kernel_launches[STOMP_B200_KERNEL_ROWS]--;     // nothing launched in this scope
-                e->launch_count--;
-            }
-        } else {
-            if (int rc = launch_rows(e, lp, rows_kind, rows, rows_stream)) return rc;
-        }
-    }
-    if (overlap_rows) CUDA_TRY(e, cudaEventRecord(e->ev_rows, rows_stream));
+    lp.noise_from_rollouts = (gen_shape.rows == RowsWork::kNone && one_update_launch && !c.keep_debug_tensors && !lp.proj) ? 1 : 0;
+    if (int rc = launch_generate_stage(e, lp, gen_shape)) return rc;
     {
         const int states = gen_local * e->T;
         Scope sc(e, STOMP_B200_KERNEL_COST);
@@ -1017,7 +1044,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
             e->launch_count += 2;
         }
     }
-    if (overlap_rows) CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_rows, 0));
+    if (gen_shape.overlap) CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_rows, 0));
     // ---- the noise-less rollout of the previous iteration is needed from here on ----
     if (e->noiseless_pending) {
         CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_noiseless, 0));
@@ -1097,10 +1124,11 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
     const stomp_b200_config& c = e->cfg;
     const int world = c.shard_mode == 0 ? c.world_size : 1;
     const UpdateShape shape = update_shape(e, world);
-    bool eligible = allow_graph && e->graphs_allowed && e->d_counters && mode == kNoisePhilox && !e->timeline_on &&
+    const GenerateShape gen_shape = generate_shape(e, mode);
+    bool eligible = allow_graph && e->graphs_allowed && e->d_counters && !e->timeline_on &&
+                    gen_shape.philox && gen_shape.sampler == Sampler::kRecurrence && gen_shape.rows != RowsWork::kProjection &&
                     (shape == UpdateShape::kFused || shape == UpdateShape::kPeer) &&
-                    e->noiseless_valid && !c.keep_debug_tensors && !e->edge_dirty && !c.use_projection && !e->extras_on &&
-                    e->base.Lband != nullptr && (e->sampler_mode == 0 || e->sampler_mode == 3) &&
+                    e->noiseless_valid && !c.keep_debug_tensors && !e->edge_dirty && !e->extras_on &&
                     !e->noiseless_pending && (!e->nl_deferred || e->nl_lp.honour_stop == honour_stop);
     eligible = eligible && noiseless_tail_available(e);      // the side-stream rollout bakes per-iteration state into its parameters
     // A sampler that is launched as a programmatic dependent of the previous iteration's update kernel draws its noise beside
@@ -1607,9 +1635,10 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
         cudaDeviceProp prop;
         CREATE_CUDA(cudaGetDeviceProperties(&prop, cfg->device));
         e->num_sms = prop.multiProcessorCount;
-        const char* sampler = std::getenv("STOMP_B200_SAMPLER");
-        e->use_dmma = !(sampler && std::string(sampler) == "simt");
-        e->sampler_mode = !sampler ? 0 : (std::string(sampler) == "dmma" ? 1 : (std::string(sampler) == "simt" ? 2 : (std::string(sampler) == "banded" ? 3 : 0)));
+    }
+    if (const char* s = std::getenv("STOMP_B200_SAMPLER")) {
+        if (std::strcmp(s, "dmma") == 0) e->sampler_switch = SamplerSwitch::kContraction;
+        else if (std::strcmp(s, "banded") == 0) e->sampler_switch = SamplerSwitch::kRecurrence;
     }
     CREATE_CUDA(cudaFuncSetAttribute(noiseless_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     CREATE_CUDA(cudaFuncSetAttribute(reuse_rollouts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));

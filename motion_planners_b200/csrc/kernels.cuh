@@ -297,109 +297,13 @@ __device__ __forceinline__ void shift_clamp_store(const LoopParams& p, const Joi
     }
 }
 
-// Contraction N^T[c][t] = sum_u E^T[c][u] * Lt[u][t] over the G*D columns c = (k, d) of one query, all T
-// rows at once, fused with the epilogue above.  256 threads: ty = tid/16 owns 4 columns, tx = tid%16 owns the
-// time steps tx + 16*j, j < NT.  Lt is upper triangular: chunk kc of the u loop only touches j >= kc.
-template <int NT, bool kPhilox>
-__global__ void __launch_bounds__(256)
-sample_rollouts_kernel(const __grid_constant__ LoopParams p, const __grid_constant__ JointLimits robot)
-{
-    constexpr int BM = 64, BK = 16, BN = NT * 16;
-    __shared__ double As[BK][BM + 2];
-    __shared__ double Bs[BK][BN];
-    const int q = blockIdx.y;
-    if (query_frozen(p, q)) return;
-    TimelineScope tls(p, 0);
-    const int T = p.T, D = p.D;
-    const int ncols = p.num_gen * D;
-    const int c0 = blockIdx.x * BM;
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-
-    double acc[4][NT];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < NT; ++j) acc[i][j] = 0.0;
-
-    const int nchunks = (T + BK - 1) / BK;
-    const int lc = tid >> 2;              // column of the tile this thread fills
-    const int lu = (tid & 3) * 4;         // first of its 4 u rows
-    for (int kc = 0; kc < nchunks; ++kc) {
-        const int u0 = kc * BK;
-        // ---- A tile: 64 columns x 16 u ----
-        {
-            const int c = c0 + lc;
-            double z[4] = {0.0, 0.0, 0.0, 0.0};
-            if (c < ncols) {
-                const int k = c / D, d = c - k * D;
-                if (kPhilox) {
-                    const uint32_t gcol = (uint32_t)((((size_t)(p.query_offset + q)) * p.gen_global + (p.gen_offset + k)) * D + d);
-                    philox_normals(p.seed, (uint32_t)p.iteration, gcol, (uint32_t)((u0 + lu) >> 2), z);
-                    if (p.store_unit) {
-#pragma unroll
-                        for (int m = 0; m < 4; ++m)
-                            if (u0 + lu + m < T) p.epsilon[(((size_t)q * p.num_gen + k) * D + d) * T + u0 + lu + m] = z[m];
-                    }
-                } else {
-#pragma unroll
-                    for (int m = 0; m < 4; ++m)
-                        if (u0 + lu + m < T) z[m] = p.epsilon[(((size_t)q * p.num_gen + k) * D + d) * T + u0 + lu + m];
-                }
-#pragma unroll
-                for (int m = 0; m < 4; ++m)
-                    if (u0 + lu + m >= T) z[m] = 0.0;
-            }
-#pragma unroll
-            for (int m = 0; m < 4; ++m) As[lu + m][lc] = z[m];
-        }
-        // ---- B tile: 16 u x BN t of Lt (zero outside the matrix) ----
-        for (int e = tid; e < BK * BN; e += 256) {
-            const int u = e / BN, t = e - u * BN;
-            double v = 0.0;
-            if (u0 + u < T && t < T && t >= u0 + u) v = p.Lt[(size_t)(u0 + u) * T + t];
-            Bs[u][t] = v;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int u = 0; u < BK; ++u) {
-            double a[4], b[NT];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) a[i] = As[u][ty * 4 + i];
-#pragma unroll
-            for (int j = 0; j < NT; ++j)
-                if (j >= kc) b[j] = Bs[u][tx + 16 * j];
-#pragma unroll
-            for (int j = 0; j < NT; ++j)
-                if (j >= kc) {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-                }
-        }
-        __syncthreads();
-    }
-    // ---- epilogue ----
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int c = c0 + ty * 4 + i;
-        if (c >= ncols) continue;
-        const int k = c / D, d = c - k * D;
-#pragma unroll
-        for (int j = 0; j < NT; ++j) {
-            const int t = tx + 16 * j;
-            if (t >= T) continue;
-            if (p.store_unit) p.unit_noise[(((size_t)q * p.num_gen + k) * D + d) * T + t] = acc[i][j];
-            shift_clamp_store(p, robot, q, k, d, t, acc[i][j]);
-        }
-    }
-    tls.end();
-}
-
 // ---------------------------------------------------------------------------------------------------
-// The same contraction on the FP64 tensor path (mma.sync.m8n8k4.f64 -> DMMA.8x8x4, the only FP64 MMA shape the
-// hardware has: ptxas splits m16n8k16 into eight of them).  Measured on B200 (tools/fp64_peak.cu,
-// profiles/r1_fp64_peak_b200.json): DMMA 37.0 TFLOP/s vs 35.0 TFLOP/s on the FMA pipe — the same peak, but one DMMA
-// carries the work of eight DFMA warp-instructions, and ncu showed the SIMT kernel above issue-bound, i.e. the
-// case BASELINE.json's north_star reserves tensor cores for.
+// Contraction N^T[c][t] = sum_u E^T[c][u] * Lt[u][t] over the G*D columns c = (k, d) of a query, fused with the
+// epilogue above, on the FP64 tensor path (mma.sync.m8n8k4.f64 -> DMMA.8x8x4, the only FP64 MMA shape the hardware has:
+// ptxas splits m16n8k16 into eight of them).  Measured on B200 (tools/fp64_peak.cu, profiles/r1_fp64_peak_b200.json):
+// DMMA 37.0 TFLOP/s vs 35.0 TFLOP/s on the FMA pipe — the same peak, but one DMMA carries the work of eight DFMA
+// warp-instructions, and ncu showed the earlier FMA-pipe version of this contraction issue-bound, i.e. the case
+// BASELINE.json's north_star reserves tensor cores for.
 //
 // Per warp: one m8 tile = 8 columns (k, d) x all time steps of a 104-wide slab of t; C = 13 n8 tiles in registers;
 // B = the Lt slab, resident in shared memory for the whole kernel; tiles handed out by an atomic counter (reset
@@ -421,7 +325,7 @@ constexpr int kDmmaWarps = 8;
 constexpr int kSlabTilesMax = 13;
 __host__ __device__ constexpr int dmma_slab_stride(int tiles) { return 8 * tiles + 2; }     // == 2 (mod 4)
 
-__host__ __device__ inline int dmma_slab_rows(int T) { return (T + 15) & ~15; }
+__host__ __device__ constexpr int dmma_slab_rows(int T) { return (T + 15) & ~15; }
 
 __device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b)
 {

@@ -622,9 +622,8 @@ def test_smallest_shapes(K, T):
 
 def test_longest_trajectory_and_the_fallback_kernels(monkeypatch):
     """T = STOMP_B200_MAX_TIME_STEPS = 256: three slabs in the DMMA sampler, and N = 268 is past the control-cost tile
-    kernel's instantiations, so control_rows_fast_kernel runs.  Then T = 100 with the FMA-pipe sampler
-    (STOMP_B200_SAMPLER=simt) and the generic state kernel (STOMP_B200_STATES=generic): the fallbacks agree with the
-    oracle like the default kernels do."""
+    kernel's instantiations, so control_rows_fast_kernel runs.  Then T = 100 with the generic state kernel
+    (STOMP_B200_STATES=generic): the fallback agrees with the oracle like the default kernel does."""
     def check(pb, iterations):
         D, K, T = pb.chain.num_dimensions, pb.num_rollouts, pb.num_time_steps
         o, e, pol = _pair(pb)
@@ -640,7 +639,6 @@ def test_longest_trajectory_and_the_fallback_kernels(monkeypatch):
             _compare_iteration(o, e, cost, valid)
         return e
     check(P.single_arm_problem(K=3, T=256, sdf_n=64), 2)
-    monkeypatch.setenv("STOMP_B200_SAMPLER", "simt")
     monkeypatch.setenv("STOMP_B200_STATES", "generic")
     e = check(P.single_arm_problem(K=10, T=100, sdf_n=64), 2)
     assert e.state_kernel_kind()[0] == "generic"
@@ -933,6 +931,70 @@ def test_fused_control_cost_sums_of_the_recurrence_sampler(monkeypatch):
                     np.testing.assert_allclose(eng.tensor("parameters")[0], o.parameters(), rtol=RTOL, atol=1e-12)
                     np.testing.assert_allclose(eng.tensor("stddevs")[0], o.stddevs(), rtol=RTOL)
                     np.testing.assert_allclose(c, cost, rtol=RTOL)
+
+
+# The shapes of the generate stage (engine.cu: generate_shape): noise source, STOMP_B200_SAMPLER, T (odd: the row kernels
+# cannot be fused into the recurrence sampler), debug tensors (the fused sampler then leaves the per-time-step store to the
+# row kernel), use_projection; and launch_count() added by each of three iterate() calls, the owed noise-less rollout that
+# the call's read-back launches included.  The counts pin what the stage launches in each shape (bench.py reports them
+# per step).
+_GENERATE_SHAPES = {
+    "philox-recurrence-fused-lean": ("philox", None, 40, False, False, (7, 4, 4)),
+    "philox-recurrence-fused-store": ("philox", None, 40, True, False, (8, 5, 5)),
+    "philox-recurrence-unfused": ("philox", None, 41, True, False, (8, 5, 5)),
+    "philox-contraction": ("philox", "dmma", 40, False, False, (8, 5, 5)),
+    "epsilon-contraction": ("epsilon", None, 40, True, False, (8, 5, 5)),
+    "epsilon-recurrence": ("epsilon", "banded", 40, True, False, (8, 5, 5)),
+    "unit-noise-shift": ("unit", None, 40, True, False, (8, 5, 5)),
+    "philox-projection": ("philox", None, 40, True, True, (10, 7, 7)),
+}
+
+
+def _generate_shape_iterations(case, monkeypatch):
+    """Three iterations of one generate shape; returns the launch_count() each added.  The two shapes no other test holds
+    to the oracle, injected epsilon through the recurrence sampler and on-device noise under the M-projection, are
+    compared with it here, replayed from the engine's unit noise."""
+    noise, sampler, T, debug, projection = _GENERATE_SHAPES[case][:5]
+    pb = P.single_arm_problem(K=24, T=T, sdf_n=64)
+    D, K = pb.chain.num_dimensions, pb.num_rollouts
+    compare = case in ("epsilon-recurrence", "philox-projection")
+    okw = {"use_projection": True} if projection else {}
+    if sampler:
+        monkeypatch.setenv("STOMP_B200_SAMPLER", sampler)
+    if compare:
+        o, e, pol = _projection_pair(pb, **okw)
+        o.begin_solve()
+    else:
+        e = binding.engine_for_problem(pb, keep_debug_tensors=debug, **okw)
+        pol = e.policy
+    monkeypatch.delenv("STOMP_B200_SAMPLER", raising=False)
+    e.begin_solve()
+    rng = np.random.default_rng(600 + T)
+    added = []
+    for it in range(3):
+        kw = {}
+        if noise == "epsilon":
+            kw["epsilon"] = rng.standard_normal((1, K, D, T))
+        elif noise == "unit":
+            kw["noise"] = np.einsum("tu,kdu->kdt", pol["L"], rng.standard_normal((K, D, T)))[None]
+        before = e.launch_count()
+        cost, valid, _ = e.iterate(it, **kw)
+        added.append(e.launch_count() - before)
+        if compare:
+            unit = e.tensor("unit_noise")[0]
+            ref = np.einsum("tu,kdu->kdt", pol["L"], e.tensor("epsilon")[0])
+            assert abs(unit - ref).max() <= 4e-9 * abs(ref).max()      # recurrence sampler: limited by the accuracy of L itself
+            o.iterate(it, noise=unit)
+            if projection:
+                ref = o.field("noise_projected")
+                np.testing.assert_allclose(e.tensor("noise_projected")[0], ref, rtol=RTOL, atol=1e-13 * abs(ref).max())
+            _compare_iteration(o, e, cost, valid)
+    return added
+
+
+@pytest.mark.parametrize("case", list(_GENERATE_SHAPES))
+def test_each_generate_shape_keeps_its_launch_count(case, monkeypatch):
+    assert _generate_shape_iterations(case, monkeypatch) == list(_GENERATE_SHAPES[case][5])
 
 
 def test_forward_cumulation_variant():

@@ -145,7 +145,6 @@ struct stomp_b200_engine {
     double* d_Mproj = nullptr; double* d_Minv = nullptr;   // projection_matrix_ / its inverse (use_projection only)
     double* state2[2] = {nullptr, nullptr};
     uint8_t* verdict2[2] = {nullptr, nullptr};
-    int cur = 0;
     int32_t* d_order = nullptr;
     int max_chunks = 1;
     int num_sms = 148;
@@ -153,31 +152,44 @@ struct stomp_b200_engine {
     cudaEvent_t ev_applied = nullptr, ev_noiseless = nullptr;
     cudaStream_t rows_stream = nullptr;      // control-cost rows, side by side with the state kernel
     cudaEvent_t ev_sampled = nullptr, ev_rows = nullptr;
-    bool noiseless_pending = false;          // ev_noiseless recorded and not yet waited for by the main stream
-    // The noise-less rollout of iteration i is LAUNCHED at the start of iteration i + 1 (or by the first call that needs its
-    // result), not at the end of i: on the device nothing changes — it still runs on the side stream under the next
-    // sampling — but an iteration then has the fork / join shape [noise-less of i-1 || sample, cost of i] -> update of i
-    // that a CUDA graph can hold.
-    bool nl_deferred = false;
-    LoopParams nl_lp;                        // parameters of the iteration whose noise-less rollout is owed
     // With the run-time specialised state kernel the owed rollout needs no kernel of its own: its control costs are
     // computed by the update kernel's last CTA per joint (apply_update_body), its T states ride on the next state kernel
     // launch as a tail (kinematics.cuh: NoiselessTail), whose last thread does the bookkeeping and the stop rule.  The
     // record of the rollout is double buffered: the update of iteration i writes the one iteration i + 1 reads.
     double* nl_sums2[2] = {nullptr, nullptr};
-    int nl_parity = 0;                       // nl_sums2[nl_parity] is what the next iteration reads
     uint32_t* d_nl_counter = nullptr;        // [Q] packed hit / finished-state counters of the tail
-    // steady-state iterations replayed from CUDA graphs (iterate_async): one per (honour_stop, noise-less rollout owed)
+
+    // The host state an iteration (iterate_body) reads and writes, statistics and configuration aside.  Whole, so that a
+    // CUDA graph replay can set it as the captured iteration left it and an abandoned capture can put it back (iterate_async).
+    struct LoopState {
+        // PolicyImprovement bookkeeping (PolicyImprovement.cpp:170-186) and what read-backs need of the last iteration
+        int num_rollouts = 0;                    // num_rollouts_ after the previous iteration (global)
+        int last_gen = 0, last_local = 0, last_noiseless_slot = -1;
+        int last_wblocks = 1;                    // partial sums of the weights left in wpart by the last iteration
+        bool last_noise_from_rollouts = false;   // the last iteration did not write `noise` (read-backs say so)
+        bool noiseless_valid = false, adapted_valid = false;
+        // The noise-less rollout of iteration i is LAUNCHED at the start of iteration i + 1 (or by the first call that needs
+        // its result), not at the end of i: on the device nothing changes — it still runs on the side stream under the next
+        // sampling — but an iteration then has the fork / join shape [noise-less of i-1 || sample, cost of i] -> update of i
+        // that a CUDA graph can hold.
+        bool nl_deferred = false;
+        LoopParams nl_lp;                        // parameters of the iteration whose noise-less rollout is owed
+        int nl_parity = 0;                       // nl_sums2[nl_parity] is what the next iteration reads
+        bool noiseless_pending = false;          // ev_noiseless recorded and not yet waited for by the main stream
+        int cur = 0;                             // proj2 / state2 / verdict2[cur] hold the last iteration's rollouts (reuse)
+        bool edge_dirty = true;                  // edge_cost has to be recomputed (the policy was uploaded since)
+        bool tables_gathered = true;             // rollout-indexed tables complete on this rank (peer mode gathers them lazily for read-backs)
+        uint32_t peer_epoch = 0;                 // epoch of the last exchange queued (PeerExchange::epoch, LoopParams::counters[1])
+    };
+    LoopState loop;
+    // steady-state iterations replayed from CUDA graphs (iterate_async): one per (honour_stop, record parity)
     struct IterationGraph {
         cudaGraphExec_t exec = nullptr;
-        int gen = -1, n = -1;                            // shape the graph was captured for
         unsigned long long config_epoch = 0;
         int64_t launches = 0;                            // kernel nodes (what a replay adds to launch_count)
-        int num_rollouts = 0, last_gen = 0, last_local = 0, last_noiseless_slot = -1, last_wblocks = 1;   // host bookkeeping after the iteration
-        bool last_noise_from_rollouts = false, peer = false;
-        LoopParams nl_lp;
+        LoopState after;                                 // the loop state the captured iteration left
     };
-    IterationGraph graphs[2][2][2];          // [honour_stop][noise-less rollout owed][record parity]
+    IterationGraph graphs[2][2];             // [honour_stop][record parity]
     unsigned long long config_epoch = 1;     // bumped by every setter whose values are baked into kernel parameters
     // STOMP_B200_PDL=<mask> at creation: bit 0 sampler, 1 state kernel, 2 weights / update kernel launched as programmatic
     // dependents of the kernel before them (0: ordinary launches).  Default 5: the state kernel is NOT made a dependent of the
@@ -197,15 +209,8 @@ struct stomp_b200_engine {
     int64_t graph_launches = 0;
     double* d_theta_all_init = nullptr;   // policy as uploaded by set_policy (restored by begin_solve? no: the policy persists)
 
-    // PolicyImprovement bookkeeping (PolicyImprovement.cpp:170-186)
     bool solving = false;
-    int num_rollouts = 0;           // num_rollouts_ after the previous iteration (global)
-    int last_gen = 0, last_local = 0, last_noiseless_slot = -1;
-    bool last_noise_from_rollouts = false;   // the last iteration did not write `noise` (read-backs say so)
-    int last_wblocks = 1;           // partial sums of the weights left in wpart by the last iteration
     bool fuse_weights_allowed = true;   // STOMP_B200_FUSE_WEIGHTS=0 at creation keeps K7 / K8 / K9 as separate kernels
-    bool noiseless_valid = false, adapted_valid = false;
-    bool edge_dirty = true;         // edge_cost has to be recomputed (the policy was uploaded since)
     // state kernel specialised to the robot structure (state_codegen.hpp); resolved at the first iteration after
     // the chain / spheres / SDF changed
     const codegen::SpecialisedKernel* spec = nullptr;
@@ -251,12 +256,11 @@ struct stomp_b200_engine {
     // read-back gather and the fallback (STOMP_B200_EXCHANGE=nccl, or cudaIpc unavailable)
     PeerExchange px;
     bool peer_ready = false;
-    uint32_t peer_epoch = 0, barrier_ticket = 0;
+    uint32_t barrier_ticket = 0;
     void* peer_box_own = nullptr;
     std::vector<void*> peer_opened;
     int32_t* d_peer_error = nullptr; int32_t* h_peer_error = nullptr;
     std::string exchange_note = "single GPU: no exchange";
-    bool tables_gathered = true;             // rollout-indexed tables complete on this rank (peer mode gathers them lazily for read-backs)
 
     // grow-only scratch of stomp_b200_evaluate_states
     double* eval_theta = nullptr; double* eval_cost = nullptr; uint8_t* eval_verdict = nullptr; uint8_t* eval_valid = nullptr;
@@ -647,7 +651,7 @@ StateKernelArgs noiseless_state_args(stomp_b200_engine* e, const LoopParams& lp,
     a.stop = lp.stop; a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.honour_stop = lp.honour_stop;
     if (tail) {
         a.num_gen = 0; a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
-        fill_noiseless_tail(e, lp, e->nl_sums2[e->nl_parity], a.nl);
+        fill_noiseless_tail(e, lp, e->nl_sums2[e->loop.nl_parity], a.nl);
     } else {
         a.rollouts = lp.theta_all + kPad; a.state_costs = lp.nl_state; a.verdicts = lp.nl_verdict; a.validity = lp.nl_valid;
         a.num_gen = 1; a.row_stride = lp.N; a.rollout_stride = (int64_t)lp.D * lp.N;
@@ -712,15 +716,15 @@ int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream
     return check_launch(e, "rollout_states_kernel");
 }
 
-// the noise-less rollout of the iteration recorded in e->nl_lp (K10 + the wrapper's stop rule): a state pass over its T states,
+// the noise-less rollout of the iteration recorded in e->loop.nl_lp (K10 + the wrapper's stop rule): a state pass over its T states,
 // then noiseless_rollout_kernel unless the pass was the tail of the specialised kernel, which finishes the record itself.  On
 // the side stream behind everything queued on the main stream so far; on_main_stream: the caller is about to wait for the
 // result (a join), nothing is there to overlap with — queue behind the update kernel directly; the cross-stream hand-over
 // alone cost 13 us of every isolated iteration
 int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
 {
-    const LoopParams& lp = e->nl_lp;
-    e->nl_deferred = false;
+    const LoopParams& lp = e->loop.nl_lp;
+    e->loop.nl_deferred = false;
     const bool tail = noiseless_tail_available(e);     // first: resolving may queue the static-sphere kernel on the main stream
     cudaStream_t st = on_main_stream ? e->stream : e->side_stream;
     if (!on_main_stream) {
@@ -740,7 +744,7 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
     }
     if (!on_main_stream) {
         CUDA_TRY(e, cudaEventRecord(e->ev_noiseless, e->side_stream));
-        e->noiseless_pending = true;
+        e->loop.noiseless_pending = true;
     }
     return 0;
 }
@@ -796,11 +800,11 @@ GenerateShape generate_shape(const stomp_b200_engine* e, int mode)
 int launch_generate_stage(stomp_b200_engine* e, const LoopParams& lp, const GenerateShape& g)
 {
     // padding-only rows of the control costs: constants of a solve, needed by the fused sampler and the row kernels
-    if (e->edge_dirty && lp.num_rules == 1) {
+    if (e->loop.edge_dirty && lp.num_rules == 1) {
         edge_rows_kernel<<<e->Q, 64, 0, e->stream>>>(lp);
         e->launch_count++;
         if (int rc = check_launch(e, "edge_rows_kernel")) return rc;
-        e->edge_dirty = false;
+        e->loop.edge_dirty = false;
     }
     switch (g.sampler) {
     case Sampler::kRecurrence:
@@ -890,9 +894,9 @@ int launch_update_stage(stomp_b200_engine* e, LoopParams& lp, UpdateShape shape,
     switch (shape) {
     case UpdateShape::kPeer: {
         lp.wblocks = 1;
-        e->px.epoch = ++e->peer_epoch;
+        e->px.epoch = ++e->loop.peer_epoch;
         e->px.epoch_ptr = on_graph ? e->d_counters + 1 : nullptr;
-        e->tables_gathered = false;
+        e->loop.tables_gathered = false;
         Scope sc(e, STOMP_B200_KERNEL_UPDATE);
         void* args[] = {&lp, &e->px};
         CUDA_TRY(e, launch_dependent(e, 2, (const void*)weights_update_peer_kernel, dim3(lp.nchunks * e->D), dim3(kUpdateThreads), update_smem, e->stream, args));
@@ -924,7 +928,7 @@ int launch_update_stage(stomp_b200_engine* e, LoopParams& lp, UpdateShape shape,
     case UpdateShape::kSeparate: {
         const bool nccl = world > 1;
         if (nccl) {     // ---- exchange 1: per-rollout cost scalars (SURVEY.md §8e) ----
-            e->tables_gathered = true;
+            e->loop.tables_gathered = true;
             const size_t count = (size_t)lp.num_gen * e->sumw;
             NCCL_TRY(e, g_nccl.AllGather(lp.sums + (size_t)c.rank * count, lp.sums, count, ncclFloat64, e->comm, e->stream));
         }
@@ -951,23 +955,34 @@ int launch_update_stage(stomp_b200_engine* e, LoopParams& lp, UpdateShape shape,
     return 0;
 }
 
+// PolicyImprovement::generateRollouts bookkeeping (PolicyImprovement.cpp:170-186): the rollouts the next iteration generates,
+// in all and on this rank, and the ones it keeps from the last
+struct RolloutPlan { int gen, gen_local, reused; };
+RolloutPlan plan_rollouts(const stomp_b200_engine* e)
+{
+    const stomp_b200_config& c = e->cfg;
+    const int prev = e->loop.num_rollouts;
+    RolloutPlan p;
+    p.gen = c.num_rollouts_per_iteration;
+    if (prev + p.gen < c.min_rollouts) p.gen = c.min_rollouts - prev;
+    p.reused = prev;
+    if (prev + p.gen > c.max_rollouts) p.reused = prev - (prev + p.gen - c.max_rollouts);
+    if (p.reused < 0) p.reused = 0;
+    p.gen_local = p.gen / (c.shard_mode == 0 ? c.world_size : 1);
+    return p;
+}
+
 int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop, bool on_graph)
 {
     const stomp_b200_config& c = e->cfg;
     const int world = c.shard_mode == 0 ? c.world_size : 1;
-    // ---- PolicyImprovement::generateRollouts bookkeeping (PolicyImprovement.cpp:170-186) ----
-    const int prev = e->num_rollouts;
-    int gen = c.num_rollouts_per_iteration;
-    int reused = prev;
-    if (prev + gen < c.min_rollouts) gen = c.min_rollouts - prev;
-    if (prev + gen > c.max_rollouts) reused = prev - (prev + gen - c.max_rollouts);
-    if (reused < 0) reused = 0;
+    const int prev = e->loop.num_rollouts;
+    const auto [gen, gen_local, reused] = plan_rollouts(e);
     if (world > 1 && (reused != 0 || gen % world != 0))
         return fail(e, STOMP_B200_ERR_UNSUPPORTED, "rollout sharding needs min = max = per-iteration rollouts, divisible by world_size");
     if (!e->reuse_possible && reused != 0) return fail(e, STOMP_B200_ERR_UNSUPPORTED, "internal: reuse without reuse buffers");
-    const int gen_local = gen / world;
     int n = reused + gen;
-    const bool have_nl = e->noiseless_valid;
+    const bool have_nl = e->loop.noiseless_valid;
     const int nl_gslot = have_nl ? n : -1;
     if (have_nl) ++n;
 
@@ -984,13 +999,13 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     lp.store_unit = c.keep_debug_tensors;
     lp.counters = on_graph ? e->d_counters : nullptr;
     lp.early_sampler = e->early_sampler ? 1 : 0;
-    lp.nl_sums = e->nl_sums2[e->nl_parity];
-    lp.nl_sums_next = e->nl_sums2[e->nl_parity ^ 1];
+    lp.nl_sums = e->nl_sums2[e->loop.nl_parity];
+    lp.nl_sums_next = e->nl_sums2[e->loop.nl_parity ^ 1];
     // the noise-less rollout of the previous iteration: a tail of this iteration's state kernel launch when that kernel is the
     // specialised one, else two kernels on the side stream, under this iteration's sampling and costs
     bool tail_in_state_kernel = false;
-    if (e->nl_deferred) {
-        if (noiseless_tail_available(e)) { tail_in_state_kernel = true; e->nl_deferred = false; }
+    if (e->loop.nl_deferred) {
+        if (noiseless_tail_available(e)) { tail_in_state_kernel = true; e->loop.nl_deferred = false; }
         else if (int rc = launch_noiseless(e, false)) return rc;
     }
     if (e->timeline_on) {
@@ -999,7 +1014,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     }
 
     // ---- noise magnitude (Stomp.cpp:179, PolicyImprovement.cpp:162-163) ----
-    if (!e->adapted_valid) {
+    if (!e->loop.adapted_valid) {
         SigmaIt s;
         for (int d = 0; d < e->D; ++d) s.v[d] = c.noise_stddev[d] * std::pow(c.noise_decay[d], iteration - 1);
         Scope sc(e, STOMP_B200_KERNEL_APPLY);
@@ -1009,7 +1024,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
 
     // ---- reused rollouts (PolicyImprovement.cpp:188-255) ----
     if (e->reuse_possible) {
-        const int src = e->cur, dst = 1 - e->cur;
+        const int src = e->loop.cur, dst = 1 - e->loop.cur;
         lp.proj = e->proj2[dst]; lp.state_costs = e->state2[dst]; lp.verdicts = e->verdict2[dst];
         if (reused > 0) {
             ReuseParams rp;
@@ -1020,7 +1035,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
             reuse_rollouts_kernel<<<e->Q, 256, sizeof(double) * (size_t)prev, e->stream>>>(lp, rp);
             if (int rc = check_launch(e, "reuse_rollouts_kernel")) return rc;
         }
-        e->cur = dst;
+        e->loop.cur = dst;
         e->base.proj = lp.proj; e->base.state_costs = lp.state_costs; e->base.verdicts = lp.verdicts;
     }
 
@@ -1046,9 +1061,9 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     }
     if (gen_shape.overlap) CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_rows, 0));
     // ---- the noise-less rollout of the previous iteration is needed from here on ----
-    if (e->noiseless_pending) {
+    if (e->loop.noiseless_pending) {
         CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_noiseless, 0));
-        e->noiseless_pending = false;
+        e->loop.noiseless_pending = false;
     }
     if (reused > 0) {
         const int warps = 8;
@@ -1060,20 +1075,21 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
     }
 
     if (int rc = launch_update_stage(e, lp, shape, world, on_graph)) return rc;
-    e->last_wblocks = lp.wblocks;
-    e->last_noise_from_rollouts = lp.noise_from_rollouts != 0;
+    stomp_b200_engine::LoopState& s = e->loop;
+    s.last_wblocks = lp.wblocks;
+    s.last_noise_from_rollouts = lp.noise_from_rollouts != 0;
     // ---- noise-less rollout (K10): owed; launched on the side stream by the next iteration or the next join ----
-    e->nl_lp = lp;
-    e->nl_deferred = true;
-    e->nl_parity ^= 1;                            // the record this iteration's update wrote is what the next one reads
-    if (on_graph && shape != UpdateShape::kPeer) ++e->peer_epoch;       // the sampler advances counters[1] on every replayed iteration: keep the host's mirror in step
+    s.nl_lp = lp;
+    s.nl_deferred = true;
+    s.nl_parity ^= 1;                             // the record this iteration's update wrote is what the next one reads
+    if (on_graph && shape != UpdateShape::kPeer) ++s.peer_epoch;        // the sampler advances counters[1] on every replayed iteration: keep the host's mirror in step
 
-    e->num_rollouts = n;
-    e->last_gen = gen_local;
-    e->last_local = lp.num_local;
-    e->last_noiseless_slot = lp.noiseless_slot;
-    e->noiseless_valid = true;
-    if (c.use_noise_adaptation) e->adapted_valid = true;
+    s.num_rollouts = n;
+    s.last_gen = gen_local;
+    s.last_local = lp.num_local;
+    s.last_noiseless_slot = lp.noiseless_slot;
+    s.noiseless_valid = true;
+    if (c.use_noise_adaptation) s.adapted_valid = true;
     return 0;
 }
 
@@ -1085,38 +1101,13 @@ __global__ void set_counters_kernel(uint32_t* counters, uint32_t iteration, uint
     counters[3] = 0u;
 }
 
-// host state an iteration changes (restored when a capture has to be abandoned)
-struct HostIterationState {
-    int num_rollouts, last_gen, last_local, last_noiseless_slot, last_wblocks, cur, nl_parity;
-    bool last_noise_from_rollouts, noiseless_valid, adapted_valid, nl_deferred, noiseless_pending, edge_dirty, tables_gathered;
-    uint32_t peer_epoch;
-    int64_t launch_count;
-    LoopParams nl_lp, base;
-    void save(const stomp_b200_engine* e)
-    {
-        num_rollouts = e->num_rollouts; last_gen = e->last_gen; last_local = e->last_local; last_noiseless_slot = e->last_noiseless_slot;
-        last_wblocks = e->last_wblocks; cur = e->cur; nl_parity = e->nl_parity; last_noise_from_rollouts = e->last_noise_from_rollouts;
-        noiseless_valid = e->noiseless_valid; adapted_valid = e->adapted_valid; nl_deferred = e->nl_deferred;
-        noiseless_pending = e->noiseless_pending; edge_dirty = e->edge_dirty; tables_gathered = e->tables_gathered;
-        peer_epoch = e->peer_epoch; launch_count = e->launch_count; nl_lp = e->nl_lp; base = e->base;
-    }
-    void restore(stomp_b200_engine* e) const
-    {
-        e->num_rollouts = num_rollouts; e->last_gen = last_gen; e->last_local = last_local; e->last_noiseless_slot = last_noiseless_slot;
-        e->last_wblocks = last_wblocks; e->cur = cur; e->nl_parity = nl_parity; e->last_noise_from_rollouts = last_noise_from_rollouts;
-        e->noiseless_valid = noiseless_valid; e->adapted_valid = adapted_valid; e->nl_deferred = nl_deferred;
-        e->noiseless_pending = noiseless_pending; e->edge_dirty = edge_dirty; e->tables_gathered = tables_gathered;
-        e->peer_epoch = peer_epoch; e->launch_count = launch_count; e->nl_lp = nl_lp; e->base = base;
-    }
-};
-
 // One Stomp::runSingleIteration for all local queries, queued on the stream (no host synchronisation).  Steady-state
 // iterations of the shipped large-K loop — on-device sampler, fused weights / update kernel (single GPU or peer exchange),
 // no rollout reuse, nothing per-iteration left in the kernel parameters — are captured ONCE into a CUDA graph with the shape
 //     [noise-less rollout of the previous iteration || sampler -> state kernel] -> weights / update
-// and replayed with one cudaGraphLaunch: the kernel-to-kernel launch gaps and the host's per-launch cost (which bounds a
-// rollout shard of a few hundred rollouts) go away.  The iteration number and the exchange epoch are device-side counters
-// then (LoopParams::counters).  Everything else runs iterate_body directly.
+// per (honour_stop, record parity), and replayed with one cudaGraphLaunch: the kernel-to-kernel launch gaps and the host's
+// per-launch cost (which bounds a rollout shard of a few hundred rollouts) go away.  The iteration number and the exchange
+// epoch are device-side counters then (LoopParams::counters).  Everything else runs iterate_body directly.
 int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop, bool allow_graph = true)
 {
     e->scalars_fresh = false; e->solution_fresh = false;
@@ -1125,11 +1116,14 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
     const int world = c.shard_mode == 0 ? c.world_size : 1;
     const UpdateShape shape = update_shape(e, world);
     const GenerateShape gen_shape = generate_shape(e, mode);
+    // nl_deferred: the first iteration after a join (the owed rollout was flushed for the caller) happens once per call, not
+    // worth a capture (~0.15 ms) of its own
     bool eligible = allow_graph && e->graphs_allowed && e->d_counters && !e->timeline_on &&
+                    e->loop.nl_deferred && e->loop.nl_lp.honour_stop == honour_stop &&
                     gen_shape.philox && gen_shape.sampler == Sampler::kRecurrence && gen_shape.rows != RowsWork::kProjection &&
                     (shape == UpdateShape::kFused || shape == UpdateShape::kPeer) &&
-                    e->noiseless_valid && !c.keep_debug_tensors && !e->edge_dirty && !e->extras_on &&
-                    !e->noiseless_pending && (!e->nl_deferred || e->nl_lp.honour_stop == honour_stop);
+                    e->loop.noiseless_valid && !c.keep_debug_tensors && !e->loop.edge_dirty && !e->extras_on &&
+                    !e->loop.noiseless_pending;
     eligible = eligible && noiseless_tail_available(e);      // the side-stream rollout bakes per-iteration state into its parameters
     // A sampler that is launched as a programmatic dependent of the previous iteration's update kernel draws its noise beside
     // it (LoopParams::early_sampler); a graph boundary is a full dependency and would undo that.  On one GPU with a grid that
@@ -1139,10 +1133,7 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
         const long long sampler_ctas = (long long)((c.num_rollouts_per_iteration / world + 31) / 32) * e->D * e->Q;
         if (sampler_ctas >= 5LL * e->num_sms) eligible = false;
     }
-    // the first iteration after a join (the owed rollout was flushed for the caller) happens once per call: not worth a
-    // capture (~0.15 ms) of its own
-    eligible = eligible && e->nl_deferred;
-    if (eligible && !e->adapted_valid)          // sigma is a per-iteration kernel parameter unless it does not decay
+    if (eligible && !e->loop.adapted_valid)     // sigma is a per-iteration kernel parameter unless it does not decay
         for (int d = 0; d < e->D; ++d) eligible = eligible && c.noise_decay[d] == 1.0;
     if (!eligible) return iterate_body(e, iteration, mode, honour_stop, false);
     if (e->streak_epoch != e->config_epoch) { e->streak_epoch = e->config_epoch; e->eligible_streak = 0; }
@@ -1150,17 +1141,17 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
         e->eligible_streak++;
         return iterate_body(e, iteration, mode, honour_stop, false);
     }
-    const int gen = c.num_rollouts_per_iteration, n = gen + 1;
-    stomp_b200_engine::IterationGraph& g = e->graphs[honour_stop ? 1 : 0][e->nl_deferred ? 1 : 0][e->nl_parity];
-    if (e->dev_iteration_next != iteration || e->dev_epoch_next != (long long)e->peer_epoch) {
-        set_counters_kernel<<<1, 1, 0, e->stream>>>(e->d_counters, (uint32_t)iteration, e->peer_epoch);
+    stomp_b200_engine::IterationGraph& g = e->graphs[honour_stop ? 1 : 0][e->loop.nl_parity];
+    if (e->dev_iteration_next != iteration || e->dev_epoch_next != (long long)e->loop.peer_epoch) {
+        set_counters_kernel<<<1, 1, 0, e->stream>>>(e->d_counters, (uint32_t)iteration, e->loop.peer_epoch);
         e->launch_count++;
         if (int rc = check_launch(e, "set_counters_kernel")) return rc;
     }
-    if (!g.exec || g.config_epoch != e->config_epoch || g.gen != gen || g.n != n) {
+    if (!g.exec || g.config_epoch != e->config_epoch) {
         if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
-        HostIterationState before;
-        before.save(e);
+        const stomp_b200_engine::LoopState loop_before = e->loop;
+        const LoopParams base_before = e->base;
+        const int64_t launches_before = e->launch_count;
         cudaGraph_t graph = nullptr;
         cudaError_t err = cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal);
         int rc = 0;
@@ -1173,36 +1164,30 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
         if (err != cudaSuccess || rc != 0) {    // no graph on this engine: run the iteration directly from the saved state
             (void)cudaGetLastError();
             if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
-            before.restore(e);
+            e->loop = loop_before; e->base = base_before; e->launch_count = launches_before;
             e->graphs_allowed = false;
             e->dev_iteration_next = e->dev_epoch_next = -1;
             return iterate_body(e, iteration, mode, honour_stop, false);
         }
-        g.config_epoch = e->config_epoch; g.gen = gen; g.n = n;
-        g.launches = e->launch_count - before.launch_count;
-        g.num_rollouts = e->num_rollouts; g.last_gen = e->last_gen; g.last_local = e->last_local;
-        g.last_noiseless_slot = e->last_noiseless_slot; g.last_wblocks = e->last_wblocks;
-        g.last_noise_from_rollouts = e->last_noise_from_rollouts; g.peer = world > 1;
-        g.nl_lp = e->nl_lp;
+        g.config_epoch = e->config_epoch;
+        g.launches = e->launch_count - launches_before;
+        g.after = e->loop;
     } else {
-        // replay: the host bookkeeping the body would have done
-        ++e->peer_epoch;
+        // Replay.  The iteration leaves the loop state it left in the capture, but for the exchange epoch and the owed
+        // rollout's iteration number, which advance: nl_parity and honour_stop are the graph's key; without rollout reuse
+        // (which eligibility implies) `cur` never moves and the rollout record is the same in every iteration; edge_dirty
+        // and noiseless_pending are false by eligibility; tables_gathered is false on the peer shape and always true on one
+        // GPU; adapted_valid is false without noise adaptation and true after its first iteration with it.
+        const uint32_t epoch = e->loop.peer_epoch + 1;
+        e->loop = g.after;
+        e->loop.peer_epoch = epoch;
+        e->loop.nl_lp.iteration = iteration;
         e->launch_count += g.launches;
-        e->num_rollouts = g.num_rollouts; e->last_gen = g.last_gen; e->last_local = g.last_local;
-        e->last_noiseless_slot = g.last_noiseless_slot; e->last_wblocks = g.last_wblocks;
-        e->last_noise_from_rollouts = g.last_noise_from_rollouts;
-        if (g.peer) e->tables_gathered = false;
-        e->noiseless_valid = true;
-        if (c.use_noise_adaptation) e->adapted_valid = true;
-        e->noiseless_pending = false;
-        e->nl_lp = g.nl_lp; e->nl_lp.iteration = iteration;
-        e->nl_deferred = true;
-        e->nl_parity ^= 1;
     }
     CUDA_TRY(e, cudaGraphLaunch(g.exec, e->stream));
     e->graph_launches++;
     e->dev_iteration_next = (long long)iteration + 1;
-    e->dev_epoch_next = (long long)e->peer_epoch;
+    e->dev_epoch_next = (long long)e->loop.peer_epoch;
     return 0;
 }
 
@@ -1211,16 +1196,16 @@ int iterate_async(stomp_b200_engine* e, int iteration, int mode, int honour_stop
 // (every rank asks for the same tensors in the same order; tests and bench.py's parity check do).
 int gather_tables_for_readback(stomp_b200_engine* e)
 {
-    if (e->tables_gathered || !e->comm) return 0;
+    if (e->loop.tables_gathered || !e->comm) return 0;
     const stomp_b200_config& c = e->cfg;
-    const size_t gl = (size_t)e->last_gen;
+    const size_t gl = (size_t)e->loop.last_gen;
     const LoopParams& b = e->base;
     NCCL_TRY(e, g_nccl.AllGather(b.sums + (size_t)c.rank * gl * e->sumw, b.sums, gl * e->sumw, ncclFloat64, e->comm, e->stream));
     NCCL_TRY(e, g_nccl.AllGather(b.prob + (size_t)c.rank * gl * e->D, b.prob, gl * e->D, ncclFloat64, e->comm, e->stream));
     NCCL_TRY(e, g_nccl.AllGather(b.fprob + (size_t)c.rank * gl * e->D, b.fprob, gl * e->D, ncclFloat64, e->comm, e->stream));
     NCCL_TRY(e, g_nccl.AllGather(b.total_cost + (size_t)c.rank * gl, b.total_cost, gl, ncclFloat64, e->comm, e->stream));
     CUDA_TRY(e, cudaStreamSynchronize(e->stream));
-    e->tables_gathered = true;
+    e->loop.tables_gathered = true;
     return 0;
 }
 
@@ -1305,7 +1290,7 @@ int setup_peer_exchange(stomp_b200_engine* e)
     }
     e->px.world = W; e->px.rank = c.rank; e->px.epoch = 0; e->px.epoch_ptr = nullptr; e->px.error = e->d_peer_error;
     e->px.D = e->D; e->px.T = e->T;
-    e->peer_epoch = 0; e->barrier_ticket = 0;
+    e->loop.peer_epoch = 0; e->barrier_ticket = 0;
     e->peer_ready = true;
     e->exchange_note = "peer mailboxes over NVLink (cudaIpc), both exchanges inside weights_update_peer_kernel";
     return 0;
@@ -1322,11 +1307,11 @@ int ready_to_solve(stomp_b200_engine* e)
 
 int join_side_stream(stomp_b200_engine* e)
 {
-    if (e->nl_deferred)
+    if (e->loop.nl_deferred)
         if (int rc = launch_noiseless(e, true)) return rc;
-    if (e->noiseless_pending) {
+    if (e->loop.noiseless_pending) {
         CUDA_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_noiseless, 0));
-        e->noiseless_pending = false;
+        e->loop.noiseless_pending = false;
     }
     return 0;
 }
@@ -1660,10 +1645,9 @@ int stomp_b200_destroy(stomp_b200_engine* e)
     if (e->rows_stream) cudaStreamSynchronize(e->rows_stream);
     if (e->stream) cudaStreamSynchronize(e->stream);
     resolve_profile(e);
-    for (auto& plane : e->graphs)
-        for (auto& row : plane)
-            for (auto& g : row)
-                if (g.exec) cudaGraphExecDestroy(g.exec);
+    for (auto& row : e->graphs)
+        for (auto& g : row)
+            if (g.exec) cudaGraphExecDestroy(g.exec);
     release_peer_exchange(e);
     if (e->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(e->comm);
     for (void* p : e->allocations) cudaFree(p);
@@ -2282,7 +2266,7 @@ int stomp_b200_set_policies(stomp_b200_engine* e, int32_t first_query, int32_t c
         CUDA_TRY(e, cudaMemcpy(d_mincc, min_control_cost, sizeof(double) * nm * count, cudaMemcpyHostToDevice));
     }
     for (int q = first_query; q < first_query + count; ++q) e->have_policy[q] = 1;
-    e->edge_dirty = true;
+    e->loop.edge_dirty = true;
     return STOMP_B200_OK;
 }
 
@@ -2323,12 +2307,12 @@ int stomp_b200_begin_solve(stomp_b200_engine* e)
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (int rc = ready_to_solve(e)) return rc;
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
-    e->num_rollouts = 0;
-    e->noiseless_valid = false;
-    e->adapted_valid = false;
-    e->last_gen = 0; e->last_local = 0; e->last_noiseless_slot = -1;
+    e->loop.num_rollouts = 0;
+    e->loop.noiseless_valid = false;
+    e->loop.adapted_valid = false;
+    e->loop.last_gen = 0; e->loop.last_local = 0; e->loop.last_noiseless_slot = -1;
     if (int rc = join_side_stream(e)) return rc;
-    e->nl_deferred = false;
+    e->loop.nl_deferred = false;
     e->scalars_fresh = false; e->solution_fresh = false;
     if (e->h_note) {
         // the progress words are reset from the host: no kernel that could still write them may be in flight (after a
@@ -2343,7 +2327,7 @@ int stomp_b200_begin_solve(stomp_b200_engine* e)
     reset_solve_state_kernel<<<(e->Q + 127) / 128, 128, 0, e->stream>>>(e->base);
     e->launch_count++;
     if (int rc = check_launch(e, "reset_solve_state_kernel")) return rc;
-    e->edge_dirty = true;
+    e->loop.edge_dirty = true;
     e->solving = true;
     return STOMP_B200_OK;
 }
@@ -2351,11 +2335,7 @@ int stomp_b200_begin_solve(stomp_b200_engine* e)
 int32_t stomp_b200_next_num_generated(const stomp_b200_engine* e)
 {
     if (!e) return 0;
-    const stomp_b200_config& c = e->cfg;
-    int gen = c.num_rollouts_per_iteration;
-    if (e->num_rollouts + gen < c.min_rollouts) gen = c.min_rollouts - e->num_rollouts;
-    const int world = c.shard_mode == 0 ? c.world_size : 1;
-    return gen / world;
+    return plan_rollouts(e).gen_local;
 }
 
 int stomp_b200_iterate(stomp_b200_engine* e, int32_t iteration, const double* unit_noise, const double* epsilon,
@@ -2495,8 +2475,8 @@ int stomp_b200_finish_solve(stomp_b200_engine* e, double* solution, int32_t* sta
 int stomp_b200_num_rollouts(const stomp_b200_engine* e, int32_t* num_rollouts, int32_t* num_generated)
 {
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
-    if (num_rollouts) *num_rollouts = e->num_rollouts;
-    if (num_generated) *num_generated = e->last_gen;
+    if (num_rollouts) *num_rollouts = e->loop.num_rollouts;
+    if (num_generated) *num_generated = e->loop.last_gen;
     return STOMP_B200_OK;
 }
 
@@ -2512,8 +2492,8 @@ int stomp_b200_get_tensor(stomp_b200_engine* e, int32_t tensor, void* out, size_
         tensor == STOMP_B200_PROBABILITIES || tensor == STOMP_B200_FULL_PROBABILITIES)
         if (int rc = gather_tables_for_readback(e)) return rc;
     const size_t Q = e->Q, T = e->T, D = e->D, N = e->N;
-    const size_t nl = e->last_local;      // local rollouts of the last iteration
-    const size_t ng = e->num_rollouts;    // rollouts in the rollout-indexed tables
+    const size_t nl = e->loop.last_local;     // local rollouts of the last iteration
+    const size_t ng = e->loop.num_rollouts;   // rollouts in the rollout-indexed tables
     // copy `rows` rows of `row_bytes` per query out of a [Q][stride_rows] table
     auto per_query = [&](const void* src, size_t rows, size_t stride_rows, size_t row_bytes) -> int {
         if (out_bytes != Q * rows * row_bytes) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "out_bytes does not match the tensor size");
@@ -2543,7 +2523,7 @@ int stomp_b200_get_tensor(stomp_b200_engine* e, int32_t tensor, void* out, size_
     switch (tensor) {
         case STOMP_B200_ROLLOUTS: return per_query(b.rollouts, nl * D, (size_t)e->slots * D, T * sizeof(double));
         case STOMP_B200_NOISE:
-            if (e->last_noise_from_rollouts) return fail(e, STOMP_B200_ERR_NOT_READY, "noise_ was not materialised in this configuration (keep_debug_tensors keeps it)");
+            if (e->loop.last_noise_from_rollouts) return fail(e, STOMP_B200_ERR_NOT_READY, "noise_ was not materialised in this configuration (keep_debug_tensors keeps it)");
             return per_query(b.noise, nl * D, (size_t)e->slots * D, T * sizeof(double));
         case STOMP_B200_STATE_COSTS: return per_query(b.state_costs, nl, e->slots, T * sizeof(double));
         case STOMP_B200_VERDICTS: return per_query(b.verdicts, nl, e->slots, T);
@@ -2566,7 +2546,7 @@ int stomp_b200_get_tensor(stomp_b200_engine* e, int32_t tensor, void* out, size_
             std::vector<double> pr(Q * e->gslots * D), part(Q * D * b.wblocks_cap);
             CUDA_TRY(e, cudaMemcpy(pr.data(), b.prob, sizeof(double) * pr.size(), cudaMemcpyDeviceToHost));
             CUDA_TRY(e, cudaMemcpy(part.data(), b.wpart, sizeof(double) * part.size(), cudaMemcpyDeviceToHost));
-            const int wblocks = e->last_wblocks;   // as launched
+            const int wblocks = e->loop.last_wblocks;   // as launched
             double* o = static_cast<double*>(out);
             for (size_t q = 0; q < Q; ++q)
                 for (size_t d = 0; d < D; ++d) {
@@ -2592,15 +2572,15 @@ int stomp_b200_get_tensor(stomp_b200_engine* e, int32_t tensor, void* out, size_
             const size_t cap = (size_t)std::max(e->cfg.num_rollouts_per_iteration, e->cfg.min_rollouts) / (e->cfg.shard_mode == 0 ? e->cfg.world_size : 1) + 1;
             (void)cap;
             // staging layout is [Q][G][D][T] with G = rollouts generated in the last iteration (dense)
-            if (out_bytes != Q * e->last_gen * D * T * sizeof(double)) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "out_bytes does not match the tensor size");
+            if (out_bytes != Q * e->loop.last_gen * D * T * sizeof(double)) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "out_bytes does not match the tensor size");
             CUDA_TRY(e, cudaMemcpy(out, b.unit_noise, out_bytes, cudaMemcpyDeviceToHost));
             return 0;
         }
         case STOMP_B200_EPSILON:
-            if (out_bytes != Q * e->last_gen * D * T * sizeof(double)) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "out_bytes does not match the tensor size");
+            if (out_bytes != Q * e->loop.last_gen * D * T * sizeof(double)) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "out_bytes does not match the tensor size");
             CUDA_TRY(e, cudaMemcpy(out, b.epsilon, out_bytes, cudaMemcpyDeviceToHost));
             return 0;
-        case STOMP_B200_ROLLOUT_VALIDITY: return per_query(b.validity, e->last_gen, e->slots, 1);
+        case STOMP_B200_ROLLOUT_VALIDITY: return per_query(b.validity, e->loop.last_gen, e->slots, 1);
         case STOMP_B200_NOISE_PROJECTED:
             if (!b.noise_proj) return fail(e, STOMP_B200_ERR_NOT_READY, "noise_projected_ exists with use_projection only (it is noise_ otherwise)");
             return per_query(b.noise_proj, nl * D, (size_t)e->slots * D, T * sizeof(double));

@@ -1102,27 +1102,52 @@ def test_sampler_that_draws_before_it_waits_changes_nothing(monkeypatch):
             np.testing.assert_array_equal(a, b)
 
 
+# launch_count() added by the run sequence of the test below and graph_replays() after it, per (STOMP_B200_GRAPH,
+# STOMP_B200_PDL), as measured on an NVIDIA B200 (1000 W): a replay counts the kernels of the iteration it captured, and
+# each time the device-side iteration counter is set from the host, set_counters_kernel adds one launch
+_REPLAY_SEQUENCE_COUNTS = {("1", "13"): (50, 9), ("0", "0"): (48, 0), ("1", "0"): (50, 9), ("0", "13"): (48, 0)}
+
+
+def _last_iteration_record(e):
+    """What the engine reports of its last iteration: the rollout counts and the read-backs that follow the host's record of
+    it (noise: the array, or the error when the loop did not materialise it)."""
+    record = [e.num_rollouts(), e.next_num_generated()]
+    record += [e.tensor(name).copy() for name in ("rollouts", "total_cost", "probabilities", "rollout_validity", "noiseless_state_costs")]
+    try:
+        record.append(e.tensor("noise").copy())
+    except binding.StompB200Error as err:
+        record.append(str(err))
+    return record
+
+
 def test_graph_replay_and_dependent_launch_change_nothing(medium_problem, monkeypatch):
     """Steady iterations replay from CUDA graphs (device-side iteration counter, double-buffered noise-less record) and the
     sampler / update kernels are launched as programmatic dependents: the same kernels on the same data, so the whole solve
-    is bit for bit the one plain launches give — parameters, noise-less cost, iteration count, stop behaviour."""
+    is bit for bit the one plain launches give — parameters, noise-less cost, iteration count, stop behaviour — and a replay
+    leaves the host's record of the iteration as the iteration itself would: rollout counts and read-backs."""
     pb = medium_problem
-    results, replays = [], []
-    for graph, pdl in (("1", "13"), ("0", "0"), ("1", "0"), ("0", "13")):
+    results, records = [], []
+    for graph, pdl in _REPLAY_SEQUENCE_COUNTS:
         monkeypatch.setenv("STOMP_B200_GRAPH", graph)
         monkeypatch.setenv("STOMP_B200_PDL", pdl)
         e = binding.engine_for_problem(pb)
         e.begin_solve()
+        before = e.launch_count()
         e.run(0, 7)                      # queued back to back: graphs from the fourth iteration on
         e.run(7, 1)                      # a lone iteration: plain launches, the noise-less tail launched alone at the join
         e.run(8, 6, honour_stop=True)
-        replays.append(e.graph_replays())
+        counts = (e.launch_count() - before, e.graph_replays())
+        assert counts == _REPLAY_SEQUENCE_COUNTS[(graph, pdl)]
         r = e.finish_solve()
         results.append((r["solution"].copy(), r["cost"].copy(), r["iterations"].copy(), e.tensor("stddevs").copy()))
+        records.append(_last_iteration_record(e))
         e.close()
-    assert replays[0] > 0 and replays[2] > 0 and replays[1] == 0 and replays[3] == 0
     for other in results[1:]:
         for a, b in zip(results[0], other):
+            np.testing.assert_array_equal(a, b)
+    for other in records[1:]:
+        assert len(other) == len(records[0])
+        for a, b in zip(records[0], other):
             np.testing.assert_array_equal(a, b)
     # and the device-side solve loop on top of graphs: same answer as the host-paced loop without them
     monkeypatch.setenv("STOMP_B200_GRAPH", "1"); monkeypatch.setenv("STOMP_B200_PDL", "13")

@@ -528,7 +528,8 @@ def test_trajectory_lengths_cover_every_kernel_variant(T):
 def test_unfused_weights_and_update_kernels_match_the_fused_kernel(monkeypatch):
     """Single-GPU runs use weights_update_kernel (K7-K9 in one launch); multi-GPU, rollout reuse and the per-kernel
     profiling pass use rollout_weights_kernel -> weighted_update_kernel -> apply_update_kernel.  K' = 1101 makes the
-    unfused weights kernel run three CTAs per joint (partial sums in wpart) and the update nine chunks.  With
+    unfused weights kernel run three CTAs per joint (partial sums in wpart) and the update 35 chunks of 32 rollouts
+    (the chunk stomp_b200_create picks for 1101 slots, 7 joints and one query on a 148-SM B200).  With
     STOMP_B200_FUSE_WEIGHTS=0 the apply step rides on weighted_update_kernel's last chunk CTA; profiling splits it off
     into apply_update_kernel, which adds the same partials in the same chunk order: bit-identical."""
     pb = P.single_arm_problem(K=1100, T=40, sdf_n=64)

@@ -12,7 +12,9 @@
 //                         stomp_b200_static_spheres) | rollout_states_kernel; states_self_collision_kernel / the generated
 //                         pair-rule kernel with a sphere-pair list; then state_cost_extras_kernel for the alternative costs
 //   setRolloutCosts    -> inside the sampler | launch_generate_stage: control_rows_tile_kernel | control_rows_fast_kernel |
-//                         control_rows_kernel, behind project_noise_dmma_kernel with use_projection; [reused_control_cost_kernel]
+//                         control_rows_kernel, behind project_noise_dmma_kernel with use_projection; [reused_control_cost_kernel];
+//                         all of them form rows, n^T R n terms and sums with the same functions (kernels.cuh: band_row_cost,
+//                         interior_row_cost, quad_term, edge_cost_sum, store_row_sums)
 //   improvePolicy + updateParameters
 //                      -> launch_update_stage, in the shape update_shape classifies the iteration into: weights_update_kernel on
 //                         one GPU, weights_update_peer_kernel (both exchanges over NVLink mailboxes) on rollout shards | with the
@@ -478,57 +480,50 @@ enum RowsShape { kRowsGeneric, kRowsWindow, kRowsTile };
 
 RowsShape rows_shape(const stomp_b200_engine* e, const LoopParams& lp)
 {
-    if (!(lp.st_n > 0 && lp.num_rules == 1 && (lp.r_toeplitz || !lp.use_noise_adaptation) && e->T % 2 == 0 && e->N >= 12)) return kRowsGeneric;
-    for (int j = 0; j < lp.st_n; ++j)
-        if (!(lp.st_off[j] > -3 && lp.st_off[j] < 3)) return kRowsWindow;
+    if (!(lp.st_uniform && (lp.r_toeplitz || !lp.use_noise_adaptation) && e->T % 2 == 0 && e->N >= 12)) return kRowsGeneric;
+    if (lp.st_dense[0] != 0.0 || lp.st_dense[6] != 0.0) return kRowsWindow;
     return lp.rband_halfwidth <= 4 ? kRowsTile : kRowsWindow;
 }
 
-// one Stomp::runSingleIteration for all local queries, queued on the stream (no host synchronisation)
-// eight-rows-per-warp control-cost kernel (kernels.cuh): instantiated for the group counts of the usual T
+// eight-rows-per-warp control-cost kernel (kernels.cuh), instantiated for the group counts of the usual T.  Its shared memory
+// stays under the default 48 KB: 15,488 B at 14 groups.
+// (Capping this grid's residency so that it shares every SM with the state kernel was tried — 32 KB of shared memory per
+// one-warp CTA, 7 per SM — and lost: a tile's latency is ~10 us whatever runs beside it, so 3.5 waves of 7 warps took 42 us.
+// The two kernels overlap only at their tails.)
 template <int kGroups>
-bool launch_rows_tile_g(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream)
+void launch_rows_tile(const LoopParams& lp, dim3 grid, cudaStream_t stream)
 {
-    const size_t smem = sizeof(double) * (size_t)kTileWarps * 8 * tile_noise_stride(kGroups);
-    const dim3 grid((rows + kTileWarps * 8 - 1) / (kTileWarps * 8), lp.Q);
-    if (opt_in_smem(e, (const void*)control_rows_tile_kernel<kGroups, false>, 200 * 1024) != cudaSuccess ||
-        opt_in_smem(e, (const void*)control_rows_tile_kernel<kGroups, true>, 200 * 1024) != cudaSuccess) {
-        (void)cudaGetLastError();
-        return false;     // the caller launches control_rows_fast_kernel instead
-    }
-    if (smem > 200 * 1024) return false;
-    // (Capping this grid's residency so that it shares every SM with the state kernel was tried — 32 KB of shared memory
-    // per one-warp CTA, 7 per SM — and lost: a tile's latency is ~10 us whatever runs beside it, so 3.5 waves of 7 warps
-    // took 42 us.  The two kernels overlap only at their tails.)
+    constexpr size_t smem = sizeof(double) * kTileWarps * 8 * tile_noise_stride(kGroups);
+    static_assert(smem <= 48 * 1024, "the tile kernel launches without a shared-memory opt-in");
     if (lp.control_costs) control_rows_tile_kernel<kGroups, true><<<grid, kTileWarps * 32, smem, stream>>>(lp);
     else control_rows_tile_kernel<kGroups, false><<<grid, kTileWarps * 32, smem, stream>>>(lp);
-    return true;
 }
 
-bool launch_rows_tile(stomp_b200_engine* e, const LoopParams& lp, int rows, cudaStream_t stream)
-{
-    const int g = tile_groups(lp.N);
-    if (g <= 2) return launch_rows_tile_g<2>(e, lp, rows, stream);
-    if (g <= 4) return launch_rows_tile_g<4>(e, lp, rows, stream);
-    if (g <= 7) return launch_rows_tile_g<7>(e, lp, rows, stream);
-    if (g <= 11) return launch_rows_tile_g<11>(e, lp, rows, stream);
-    if (g <= 14) return launch_rows_tile_g<14>(e, lp, rows, stream);
-    return false;
-}
-
-// control costs + n^T R n of `rows` (rollout, joint) rows with the kernel the shape allows (the tile kernel where its shared
-// memory can be had, else the register-window kernel), then the per-time-step costs when they are kept
+// control costs + n^T R n of `rows` (rollout, joint) rows with the kernel of the operator's shape (kRowsTile: the tile kernel
+// up to 14 groups, N <= 224, beyond that the register-window kernel for five taps), then the fold of the padding rows into
+// the per-time-step costs when they are kept
 int launch_rows(stomp_b200_engine* e, const LoopParams& rl, RowsShape shape, int rows, cudaStream_t stream)
 {
-    if (shape == kRowsGeneric) {
+    const dim3 grid8((rows + 7) / 8, e->Q);     // eight rows per warp (tile kernel) or per CTA (window kernel)
+    const int groups = tile_groups(e->N);
+    const char* name = "control_rows_tile_kernel";
+    if (shape == kRowsTile && groups <= 2) launch_rows_tile<2>(rl, grid8, stream);
+    else if (shape == kRowsTile && groups <= 4) launch_rows_tile<4>(rl, grid8, stream);
+    else if (shape == kRowsTile && groups <= 7) launch_rows_tile<7>(rl, grid8, stream);
+    else if (shape == kRowsTile && groups <= 11) launch_rows_tile<11>(rl, grid8, stream);
+    else if (shape == kRowsTile && groups <= 14) launch_rows_tile<14>(rl, grid8, stream);
+    else if (shape == kRowsTile) {
+        control_rows_fast_kernel<true, true><<<grid8, 256, 0, stream>>>(rl);
+        name = "control_rows_fast_kernel<true, true>";
+    } else if (shape == kRowsWindow) {
+        control_rows_fast_kernel<false, false><<<grid8, 256, 0, stream>>>(rl);
+        name = "control_rows_fast_kernel<false, false>";
+    } else {
         const size_t row_smem = sizeof(double) * (size_t)kRowWarps * (control_row_x_stride(e->N) + control_row_n_stride(e->T));
         control_rows_kernel<<<dim3((rows + kRowWarps - 1) / kRowWarps, e->Q), kRowWarps * 32, row_smem, stream>>>(rl);
-    } else if (!(shape == kRowsTile && launch_rows_tile(e, rl, rows, stream))) {
-        const dim3 grid((rows + 7) / 8, e->Q);
-        if (shape == kRowsTile) control_rows_fast_kernel<true, true><<<grid, 256, 0, stream>>>(rl);
-        else control_rows_fast_kernel<false, false><<<grid, 256, 0, stream>>>(rl);
+        name = "control_rows_kernel";
     }
-    if (int rc = check_launch(e, "control_rows_kernel")) return rc;
+    if (int rc = check_launch(e, name)) return rc;
     if (rl.control_costs) {
         fold_control_costs_kernel<<<dim3((rows + 127) / 128, e->Q), 128, 0, stream>>>(rl);
         if (int rc = check_launch(e, "fold_control_costs_kernel")) return rc;
@@ -1578,14 +1573,8 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
                 b.num_rules++;
             }
         }
-        b.st_n = 0;
-        if (b.num_rules == 1 && e->N >= 8) {
-            const double* row = band.data() + ((size_t)b.rule_id[0] * N + 3) * 7;   // any interior row
-            for (int o = 0; o < 7; ++o) {
-                b.st_dense[o] = row[o];
-                if (row[o] != 0.0) { b.st_off[b.st_n] = o - 3; b.st_coef[b.st_n] = row[o]; b.st_n++; }
-            }
-        }
+        b.st_uniform = b.num_rules == 1 && e->N >= 8;
+        if (b.st_uniform) std::copy_n(band.data() + ((size_t)b.rule_id[0] * N + 3) * 7, 7, b.st_dense);   // any interior row
         CREATE_TRY(dev_alloc(e, &tmp, band.size())); b.diff_band = tmp;
         CREATE_CUDA(cudaMemcpyAsync(tmp, band.data(), sizeof(double) * band.size(), cudaMemcpyHostToDevice, e->stream));
         CREATE_TRY(dev_alloc(e, &tmp, D)); b.min_stddev = tmp;

@@ -94,11 +94,10 @@ struct LoopParams {
     int32_t num_rules;
     int32_t rule_id[kMaxRules];
     double rule_sqrt_w[kMaxRules];
-    // interior rows of the single active rule as a tap list (non-zero coefficients only), see load_stencil
-    int32_t st_n;
-    int32_t st_off[7];
-    double st_coef[7];
-    double st_dense[7];       // the same taps as a dense row, offsets -3 .. +3 (zeros included)
+    // one active rule, whose interior rows (3 <= i < N-3) all carry the taps st_dense (offsets -3 .. +3, zeros included):
+    // interior_row_cost; otherwise every row walks the band table (band_row_cost) and st_dense is zero
+    int32_t st_uniform;
+    double st_dense[7];
     // recurrence sampler (sample_rollouts_banded_kernel): rows of L^-1, which is banded — see the kernel's comment
     const double* Lband;      // [T][8]: [0] = 1 / B[t][t], [o] = B[t][t-o] / B[t][t] for o = 1 .. 6 (zero beyond the band / before row 0), [7] unused
     int32_t lband_halfwidth;  // band of B = L^-1 below the diagonal (4 for the acceleration rule); 0 = table not available
@@ -579,6 +578,117 @@ project_noise_dmma_kernel(const __grid_constant__ LoopParams p)
     }
 }
 
+// ---- control costs: CovariantMovementPrimitive::computeControlCosts (stomp/src/CovariantMovementPrimitive.cpp:
+// 363-377): costs_all[i] = sum_rules dt*w*(Ax*Ax), Ax = (D_rule x)[i] * sqrt(w_rule).  Every kernel that forms a row, an
+// n^T R n term or a write-back of the sums does it through the functions of this section.
+// Band-table row i: every active rule, columns max(0, i-3) .. min(N-1, i+3) in order.  x(j) = x_all[j] (a shared-memory or a
+// global row).
+template <class X>
+__device__ __forceinline__ double band_row_cost(const LoopParams& p, int i, X x)
+{
+    const double dtw = p.dt * p.control_cost_weight;
+    double c = 0.0;
+    for (int r = 0; r < p.num_rules; ++r) {
+        const double* band = p.diff_band + ((size_t)p.rule_id[r] * p.N + i) * 7;
+        double s = 0.0;
+        const int lo = max(0, i - 3), hi = min(p.N - 1, i + 3);
+        for (int j = lo; j <= hi; ++j) s += __ldg(band + (j - i + 3)) * x(j);
+        const double Ax = s * p.rule_sqrt_w[r];
+        c += dtw * (Ax * Ax);
+    }
+    return c;
+}
+
+// Interior row (3 <= i < N-3) of the single active rule (p.st_uniform): the taps st_dense[kLo .. kHi], the others being
+// zero, multiplied then added in column order — the reference's arithmetic; a zero tap adds an exact zero, so any kLo / kHi
+// that covers the non-zero taps gives the same bits.  x(o) = x_all[i - 3 + o].
+template <int kLo, int kHi, class X>
+__device__ __forceinline__ double interior_row_cost(const LoopParams& p, X x)
+{
+    double s = 0.0;
+#pragma unroll
+    for (int o = kLo; o <= kHi; ++o) s += p.st_dense[o] * x(o);
+    const double Ax = s * p.rule_sqrt_w[0];
+    return (p.dt * p.control_cost_weight) * (Ax * Ax);
+}
+
+// either of the two above, for row i of a row held in memory (x[j] = x_all[j])
+__device__ __forceinline__ double control_cost_row(const LoopParams& p, const double* x, int i)
+{
+    if (p.st_uniform && i >= 3 && i < p.N - 3) return interior_row_cost<0, 6>(p, [&](int o) { return x[i - 3 + o]; });
+    return band_row_cost(p, i, [&](int j) { return x[j]; });
+}
+
+// The n^T R n term of time step t (PolicyImprovement.cpp:656-663): n_t (R_tt n_t + 2 sum_{o=1..kB} R_{t,t+o} n_{t+o}); R is
+// symmetric and banded, so each pair counts once.  r[o] = R_{t,t+o}: the Toeplitz diagonals r_diag or the row of Rband at t;
+// n(o) = noise[t + o], zero outside [0, T).
+template <int kB, class Nz>
+__device__ __forceinline__ double quad_term(const double* r, Nz n)
+{
+    double s = 0.0;
+#pragma unroll
+    for (int o = 1; o <= kB; ++o) s += r[o] * n(o);
+    return n(0) * (r[0] * n(0) + 2.0 * s);
+}
+
+// the six padding-only rows of (query, joint), summed (edge_rows_kernel leaves them in edge_cost)
+__device__ __forceinline__ double edge_cost_sum(const LoopParams& p, int q, int d)
+{
+    const double* ec = p.edge_cost + ((size_t)q * p.D + d) * 6;
+    return ((ec[0] + ec[1]) + (ec[2] + ec[3])) + (ec[4] + ec[5]);
+}
+
+// C_d and n^T R n of generated rollout k into `sums` (and C_d into c_compact), as far as rows_mask asks
+__device__ __forceinline__ void store_row_sums(const LoopParams& p, int q, int k, int d, double C_d, double quad)
+{
+    double* srow = p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw;
+    if (p.rows_mask & 1) {
+        srow[1 + d] = C_d;
+        if (p.c_compact) p.c_compact[((size_t)q * p.D + d) * p.gslots + (p.gen_offset + k)] = C_d;
+    }
+    if (p.rows_mask & 2) srow[1 + 2 * p.D + d] = p.use_noise_adaptation ? quad : 0.0;
+}
+
+// One (rollout, joint) row for one warp: C_d = sum of the per-timestep control costs (padding rows folded into
+// the first / last free step, i.e. simply included in the sum) and cum_d = sum_t (state + control).
+// x: padded trajectory of this (rollout, joint) in shared memory; state: state costs [T] in shared memory.
+__device__ __forceinline__ void control_cost_sums(const LoopParams& p, const double* x, const double* state, int lane,
+                                                  double& C_d, double& cum_d)
+{
+    const int T = p.T, N = p.N;
+    double c_sum = 0.0, s_sum = 0.0;
+    for (int i = lane; i < N; i += 32) {
+        c_sum += control_cost_row(p, x, i);
+        if (state && i < T) s_sum += state[i];
+    }
+    c_sum = warp_sum(c_sum);
+    s_sum = warp_sum(s_sum);
+    C_d = c_sum;
+    cum_d = s_sum + c_sum;
+}
+
+// per-timestep control costs in the reference's layout and folding order (:363-377); read-backs / noise-less record
+__device__ __forceinline__ void control_cost_store(const LoopParams& p, const double* x, int lane, double* control_out /*[T]*/)
+{
+    const int T = p.T, N = p.N;
+    for (int t = lane; t < T; t += 32) control_out[t] = control_cost_row(p, x, kPad + t);
+    // the 2 * kPad padding rows: one lane each (twelve dependent table walks on one lane were most of the noise-less
+    // kernel's time), then lane 0 adds them in the reference's order
+    double v = 0.0;
+    if (lane < 2 * kPad) v = control_cost_row(p, x, lane < kPad ? lane : N - (lane - kPad + 1));
+    __syncwarp();
+    double first = (lane == 0) ? control_out[0] : 0.0, last = (lane == 0) ? control_out[T - 1] : 0.0;
+#pragma unroll
+    for (int i = 0; i < kPad; ++i) {
+        first += __shfl_sync(0xffffffffu, v, i);
+        last += __shfl_sync(0xffffffffu, v, kPad + i);
+    }
+    if (lane == 0) {
+        control_out[0] = first;
+        control_out[T - 1] = last;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------
 // The same sample without the contraction.  L = chol(R^-1) (MultivariateGaussian.hpp:81) is dense, but its INVERSE is
 // banded: factor the banded R = U U^T with U UPPER triangular (a Cholesky factorisation run from the last row up; U has R's
@@ -916,16 +1026,11 @@ sample_rollouts_banded_kernel(const __grid_constant__ LoopParams p, const __grid
         const int k = k0 + lane;
         double* srow = p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw;
         if (kFuse) {
-            const double* ec = p.edge_cost + ((size_t)q * D + d) * 6;
-            const double edge = ((ec[0] + ec[1]) + (ec[2] + ec[3])) + (ec[4] + ec[5]);
             const double sw = p.rule_sqrt_w[0];
             const double kappa = (p.dt * p.control_cost_weight) * (sw * sw);
             const double ss_all = (s_part[lane] + s_part[32 + lane]) + (s_part[64 + lane] + s_part[96 + lane]);
             const double quad_all = (s_part[128 + lane] + s_part[160 + lane]) + (s_part[192 + lane] + s_part[224 + lane]);
-            const double C_d = kappa * ss_all + edge;
-            srow[1 + d] = C_d;
-            if (p.c_compact) p.c_compact[((size_t)q * D + d) * p.gslots + (p.gen_offset + k)] = C_d;
-            srow[1 + 2 * D + d] = p.use_noise_adaptation ? quad_all : 0.0;
+            store_row_sums(p, q, k, d, kappa * ss_all + edge_cost_sum(p, q, d), quad_all);   // rows_mask is 3 here
         }
         if (d == 0) {                   // S_k = sum_t state cost is accumulated with atomics by the state kernel: zeroed here
             srow[0] = 0.0;
@@ -976,148 +1081,6 @@ __device__ __forceinline__ bool state_collides(const RobotParams& robot, const S
     return hit;
 }
 
-// ---- control costs: CovariantMovementPrimitive::computeControlCosts (stomp/src/CovariantMovementPrimitive.cpp:
-// 363-377): costs_all[i] = sum_rules dt*w*(Ax*Ax), Ax = (D_rule x)[i] * sqrt(w_rule).
-// Interior rows (3 <= i < N-3) of a differentiation matrix all carry the same coefficients; with one active
-// rule (the shipped task: acceleration only) the host passes them as a list of non-zero taps (a zero
-// coefficient contributes an exact zero).  Boundary rows and multi-rule
-// configurations read the band table in column order.
-__device__ __forceinline__ double control_cost_row_table(const LoopParams& p, const double* x, int i)
-{
-    const double dtw = p.dt * p.control_cost_weight;
-    double c = 0.0;
-    for (int r = 0; r < p.num_rules; ++r) {
-        const double* band = p.diff_band + ((size_t)p.rule_id[r] * p.N + i) * 7;
-        double s = 0.0;
-        const int lo = max(0, i - 3), hi = min(p.N - 1, i + 3);
-        for (int j = lo; j <= hi; ++j) s += __ldg(band + (j - i + 3)) * x[j];
-        const double Ax = s * p.rule_sqrt_w[r];
-        c += dtw * (Ax * Ax);
-    }
-    return c;
-}
-
-__device__ __forceinline__ double control_cost_row(const LoopParams& p, const double* x, int i)
-{
-    if (p.st_n > 0 && i >= 3 && i < p.N - 3) {
-        double s = 0.0;
-        for (int j = 0; j < p.st_n; ++j) s += p.st_coef[j] * x[i + p.st_off[j]];   // mul then add, column order: the reference's arithmetic
-        const double Ax = s * p.rule_sqrt_w[0];
-        return (p.dt * p.control_cost_weight) * (Ax * Ax);
-    }
-    return control_cost_row_table(p, x, i);
-}
-
-// Register-resident coefficients of one (rollout, joint) row pass: the 7 interior taps of the single active
-// rule (zeros included: c*x with c == 0 adds an exact zero, so the sum is the reference's) and the diagonals of R.
-struct RowCoefficients {
-    double c[7];
-    double r[kRBand + 1];
-    double sqrt_w, dtw;
-    bool fast;
-};
-
-__device__ __forceinline__ RowCoefficients load_row_coefficients(const LoopParams& p)
-{
-    RowCoefficients rc;
-    rc.fast = p.st_n > 0;
-#pragma unroll
-    for (int o = 0; o < 7; ++o) rc.c[o] = 0.0;
-    for (int j = 0; j < p.st_n; ++j) {
-        const int o = p.st_off[j] + 3;
-#pragma unroll
-        for (int u = 0; u < 7; ++u)
-            if (u == o) rc.c[u] = p.st_coef[j];
-    }
-#pragma unroll
-    for (int o = 0; o <= kRBand; ++o) rc.r[o] = p.r_diag[o];
-    rc.sqrt_w = p.rule_sqrt_w[0];
-    rc.dtw = p.dt * p.control_cost_weight;
-    return rc;
-}
-
-// One (rollout, joint) row for one warp: C_d = sum of the per-timestep control costs (padding rows folded into
-// the first / last free step, i.e. simply included in the sum) and cum_d = sum_t (state + control).
-// x: padded trajectory of this (rollout, joint) in shared memory; state: state costs [T] in shared memory.
-__device__ __forceinline__ void control_cost_sums(const LoopParams& p, const RowCoefficients& rc, const double* x,
-                                                  const double* state, int lane, double& C_d, double& cum_d)
-{
-    const int T = p.T, N = p.N;
-    double c_sum = 0.0, s_sum = 0.0;
-    for (int i = lane; i < N; i += 32) {
-        double c;
-        if (rc.fast && i >= 3 && i < N - 3) {
-            const double* xi = x + i - 3;
-            double s = 0.0;
-#pragma unroll
-            for (int o = 0; o < 7; ++o) s += rc.c[o] * xi[o];
-            const double Ax = s * rc.sqrt_w;
-            c = rc.dtw * (Ax * Ax);
-        } else {
-            c = control_cost_row_table(p, x, i);
-        }
-        c_sum += c;
-        if (state && i < T) s_sum += state[i];
-    }
-    c_sum = warp_sum(c_sum);
-    s_sum = warp_sum(s_sum);
-    C_d = c_sum;
-    cum_d = s_sum + c_sum;
-}
-
-// per-timestep control costs in the reference's layout and folding order (:363-377); read-backs / noise-less record
-__device__ __forceinline__ void control_cost_store(const LoopParams& p, const double* x, int lane, double* control_out /*[T]*/)
-{
-    const int T = p.T, N = p.N;
-    for (int t = lane; t < T; t += 32) control_out[t] = control_cost_row(p, x, kPad + t);
-    // the 2 * kPad padding rows: one lane each (twelve dependent table walks on one lane were most of the noise-less
-    // kernel's time), then lane 0 adds them in the reference's order
-    double v = 0.0;
-    if (lane < 2 * kPad) v = control_cost_row(p, x, lane < kPad ? lane : N - (lane - kPad + 1));
-    __syncwarp();
-    double first = (lane == 0) ? control_out[0] : 0.0, last = (lane == 0) ? control_out[T - 1] : 0.0;
-#pragma unroll
-    for (int i = 0; i < kPad; ++i) {
-        first += __shfl_sync(0xffffffffu, v, i);
-        last += __shfl_sync(0xffffffffu, v, kPad + i);
-    }
-    if (lane == 0) {
-        control_out[0] = first;
-        control_out[T - 1] = last;
-    }
-}
-
-// n^T R n of one (rollout, joint) row for the noise adaptation (PolicyImprovement.cpp:656-663), by the warp that
-// holds the row x = theta + noise in shared memory.  The row is overwritten in place by noise = x - theta with a
-// zero tail; R is symmetric and banded: sum_t n_t (R_tt n_t + 2 sum_{o>0} R_{t,t+o} n_{t+o}).
-__device__ __forceinline__ double noise_quadratic_form(const LoopParams& p, const RowCoefficients& rc, double* x,
-                                                       const double* theta_row, int lane)
-{
-    const int T = p.T;
-    __syncwarp();
-    for (int t = lane; t < T + kPad; t += 32) x[kPad + t] = (t < T) ? x[kPad + t] - theta_row[kPad + t] : 0.0;
-    __syncwarp();
-    const double* n = x + kPad;
-    double quad = 0.0;
-    if (p.r_toeplitz) {
-        for (int t = lane; t < T; t += 32) {
-            double s = 0.0;
-#pragma unroll
-            for (int o = 1; o <= kRBand; ++o) s += rc.r[o] * n[t + o];
-            quad += n[t] * (rc.r[0] * n[t] + 2.0 * s);
-        }
-    } else {
-        const int hw = p.rband_halfwidth;
-        for (int t = lane; t < T; t += 32) {
-            const double* rb = p.Rband + (size_t)t * (2 * kRBand + 1) + kRBand;
-            double s = 0.0;
-            for (int o = 1; o <= hw; ++o) s += __ldg(rb + o) * n[t + o];
-            quad += n[t] * (__ldg(rb) * n[t] + 2.0 * s);
-        }
-    }
-    return warp_sum(quad);
-}
-
 // K5 + K6: PolicyImprovement::computeRolloutControlCosts / computeRolloutCumulativeCosts
 // (PolicyImprovement.cpp:442-495) and the n^T R n of the noise adaptation (:656-663) for the generated rollouts.
 // One WARP per (rollout, joint) row.  The warp stages the padded trajectory x = theta + noise and the noise in
@@ -1147,16 +1110,6 @@ control_rows_kernel(const __grid_constant__ LoopParams p)
         const double* nz = p.rows_noise + (((size_t)q * p.slots + k) * D + d) * T;
         const double* th = p.theta_all + ((size_t)q * D + d) * N;
         double* cc_out = p.control_costs ? p.control_costs + (((size_t)q * p.slots + k) * D + d) * T : nullptr;
-        const double dtw = p.dt * p.control_cost_weight;
-        const bool fast = p.st_n > 0;
-        double c7[7];
-#pragma unroll
-        for (int o = 0; o < 7; ++o) {
-            c7[o] = 0.0;
-            for (int j = 0; j < p.st_n; ++j)
-                if (p.st_off[j] + 3 == o) c7[o] = p.st_coef[j];
-        }
-        const double sqrt_w = p.rule_sqrt_w[0];
         // ---- stage ----
         for (int i = lane; i < XS; i += 32) {
             const int j = i - 3;
@@ -1181,25 +1134,9 @@ control_rows_kernel(const __grid_constant__ LoopParams p)
             for (int e = 0; e < 4; ++e) {
                 const int i = i0 + e;
                 if (i < N) {
-                    double cost;
-                    if (fast && i >= 3 && i < N - 3) {
-                        double sacc = 0.0;
-#pragma unroll
-                        for (int o = 0; o < 7; ++o) sacc += c7[o] * w[e + o];   // mul then add in column order: the reference's arithmetic
-                        const double Ax = sacc * sqrt_w;
-                        cost = dtw * (Ax * Ax);
-                    } else {
-                        cost = 0.0;
-                        for (int r = 0; r < p.num_rules; ++r) {
-                            const double* band = p.diff_band + ((size_t)p.rule_id[r] * N + i) * 7;
-                            double sacc = 0.0;
-#pragma unroll
-                            for (int o = 0; o < 7; ++o)
-                                if (i - 3 + o >= 0 && i - 3 + o < N) sacc += __ldg(band + o) * w[e + o];
-                            const double Ax = sacc * p.rule_sqrt_w[r];
-                            cost += dtw * (Ax * Ax);
-                        }
-                    }
+                    const double cost = (p.st_uniform && i >= 3 && i < N - 3)
+                                            ? interior_row_cost<0, 6>(p, [&](int o) { return w[e + o]; })
+                                            : band_row_cost(p, i, [&](int j) { return xs[3 + j]; });
                     C_part += cost;
                     // per-timestep layout for read-backs; fold_control_costs_kernel adds the padding rows in the reference's order
                     if (cc_out && i >= kPad && i < kPad + T) cc_out[i - kPad] = cost;
@@ -1218,31 +1155,16 @@ control_rows_kernel(const __grid_constant__ LoopParams p)
                 for (int e = 0; e < 4; ++e) {
                     const int t = t0 + e;
                     if (t < T) {
-                        double sacc = 0.0;
-                        if (p.r_toeplitz) {
-#pragma unroll
-                            for (int o = 1; o <= kRBand; ++o) sacc += p.r_diag[o] * m[e + o];
-                            quad += m[e] * (p.r_diag[0] * m[e] + 2.0 * sacc);
-                        } else {
-                            const double* rb = p.Rband + (size_t)t * (2 * kRBand + 1) + kRBand;
-#pragma unroll
-                            for (int o = 1; o <= kRBand; ++o) sacc += __ldg(rb + o) * m[e + o];
-                            quad += m[e] * (__ldg(rb) * m[e] + 2.0 * sacc);
-                        }
+                        auto nt = [&](int o) { return m[e + o]; };
+                        quad += p.r_toeplitz ? quad_term<kRBand>(p.r_diag, nt)
+                                             : quad_term<kRBand>(p.Rband + (size_t)t * (2 * kRBand + 1) + kRBand, nt);
                     }
                 }
             }
         }
         C_part = warp_sum(C_part);
         quad = warp_sum(quad);
-        if (lane == 0) {
-            double* srow = p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw;
-            if (p.rows_mask & 1) {
-                srow[1 + d] = C_part;
-                if (p.c_compact) p.c_compact[((size_t)q * D + d) * p.gslots + (p.gen_offset + k)] = C_part;
-            }
-            if (p.rows_mask & 2) srow[1 + 2 * D + d] = quad;
-        }
+        if (lane == 0) store_row_sums(p, q, k, d, C_part, quad);
     }
     tls.end();
 }
@@ -1255,16 +1177,8 @@ __global__ void edge_rows_kernel(const __grid_constant__ LoopParams p)
     const int q = blockIdx.x, N = p.N;
     for (int e = threadIdx.x; e < p.D * 6; e += blockDim.x) {
         const int d = e / 6, r = e - d * 6;
-        const int i = r < 3 ? r : N - 6 + r;
         const double* th = p.theta_all + ((size_t)q * p.D + d) * N;
-        const double* band = p.diff_band + ((size_t)p.rule_id[0] * N + i) * 7;
-        double sacc = 0.0;
-        for (int o = 0; o < 7; ++o) {
-            const int j = i - 3 + o;
-            if (j >= 0 && j < N) sacc += band[o] * th[j];
-        }
-        const double Ax = sacc * p.rule_sqrt_w[0];
-        p.edge_cost[(size_t)q * p.D * 6 + e] = (p.dt * p.control_cost_weight) * (Ax * Ax);
+        p.edge_cost[(size_t)q * p.D * 6 + e] = band_row_cost(p, r < 3 ? r : N - 6 + r, [&](int j) { return th[j]; });
     }
 }
 
@@ -1292,13 +1206,12 @@ control_rows_fast_kernel(const __grid_constant__ LoopParams p)
         const double* nz = p.rows_noise + (((size_t)q * p.slots + k) * D + d) * T;
         const double* th = p.theta_all + ((size_t)q * D + d) * N;
         double* cc_out = p.control_costs ? p.control_costs + (((size_t)q * p.slots + k) * D + d) * T : nullptr;
-        const double dtw = p.dt * p.control_cost_weight;
-        const double sqrt_w = p.rule_sqrt_w[0];
         constexpr int kNoisePairs = kRb4 ? 6 : 7;
         constexpr int kBand = kRb4 ? 4 : kRBand;
         double C_part = 0.0, quad = 0.0;
         // band-table rows 0..2 and N-3..N-1 only see the fixed padding: their costs are per (query, joint) constants
-        // of the solve (edge_rows_kernel); six lanes pick them up
+        // of the solve (edge_rows_kernel); six lanes pick them up and add them before the warp sum (not edge_cost_sum: that
+        // order of the additions is this kernel's own)
         const double edge = (lane < 6) ? p.edge_cost[((size_t)q * D + d) * 6 + lane] : 0.0;
         for (int base = 0; base < N; base += 128) {
             const int i0 = base + 4 * lane;
@@ -1325,11 +1238,7 @@ control_rows_fast_kernel(const __grid_constant__ LoopParams p)
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
                 const int i = i0 + e;
-                double sacc = 0.0;
-#pragma unroll
-                for (int o = kTaps5 ? 1 : 0; o < (kTaps5 ? 6 : 7); ++o) sacc += p.st_dense[o] * W[e + o + 1];   // mul then add in column order: the reference's arithmetic
-                const double Ax = sacc * sqrt_w;
-                const double cost = dtw * (Ax * Ax);
+                const double cost = interior_row_cost<kTaps5 ? 1 : 0, kTaps5 ? 5 : 6>(p, [&](int o) { return W[e + o + 1]; });
                 if (i >= 3 && i < N - 3) {
                     C_part += cost;
                     // per-timestep layout for read-backs; fold_control_costs_kernel adds the padding rows in the reference's order
@@ -1339,25 +1248,13 @@ control_rows_fast_kernel(const __grid_constant__ LoopParams p)
             // n^T R n terms of t = i - kPad: n_t (R_tt n_t + 2 sum_{o>0} R_{t,t+o} n_{t+o}), n_t = M[e + 4]
             if (p.use_noise_adaptation) {
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    double sacc = 0.0;
-#pragma unroll
-                    for (int o = 1; o <= kBand; ++o) sacc += p.r_diag[o] * M[e + 4 + o];
-                    quad += M[e + 4] * (p.r_diag[0] * M[e + 4] + 2.0 * sacc);   // zero noise outside [0, T): no guard needed
-                }
+                for (int e = 0; e < 4; ++e) quad += quad_term<kBand>(p.r_diag, [&](int o) { return M[e + 4 + o]; });   // zero noise outside [0, T): no guard needed
             }
         }
         C_part += edge;
         C_part = warp_sum(C_part);
         quad = warp_sum(quad);
-        if (lane == 0) {
-            double* srow = p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw;
-            if (p.rows_mask & 1) {
-                srow[1 + d] = C_part;
-                if (p.c_compact) p.c_compact[((size_t)q * D + d) * p.gslots + (p.gen_offset + k)] = C_part;
-            }
-            if (p.rows_mask & 2) srow[1 + 2 * D + d] = quad;
-        }
+        if (lane == 0) store_row_sums(p, q, k, d, C_part, quad);
     }
     tls.end();
 }
@@ -1425,15 +1322,7 @@ control_rows_tile_kernel(const __grid_constant__ LoopParams p)
     if (c0 < nrows) {          // warp-uniform
         const bool live = c < nrows;
         const int k = live ? c / D : 0, d = live ? c - k * D : 0;
-        const double dtw = p.dt * p.control_cost_weight;
-        const double sqrt_w = p.rule_sqrt_w[0];
-        const double c1 = p.st_dense[1], c2 = p.st_dense[2], c3 = p.st_dense[3], c4 = p.st_dense[4], c5 = p.st_dense[5];
-        const double r0 = p.r_diag[0], r1 = p.r_diag[1], r2 = p.r_diag[2], r3 = p.r_diag[3], r4 = p.r_diag[4];
-        double edge = 0.0;
-        if (live && kq == 0) {
-            const double* ec = p.edge_cost + ((size_t)q * D + d) * 6;
-            edge = ((ec[0] + ec[1]) + (ec[2] + ec[3])) + (ec[4] + ec[5]);
-        }
+        const double edge = (live && kq == 0) ? edge_cost_sum(p, q, d) : 0.0;
         const int i_begin = kq * E;
         const double* nrow = ns + r * NS + i_begin;          // nrow[m] = noise[i_begin + m - 8]
         const double* trow = p.theta_all + ((size_t)q * D + d) * N + i_begin - 2;   // trow[m] = theta_all[i_begin + m - 2] (L1-resident)
@@ -1470,33 +1359,20 @@ control_rows_tile_kernel(const __grid_constant__ LoopParams p)
             }
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
-                // element i + e: taps -2 .. +2 on x_all, mul then add in column order (the reference's arithmetic)
-                double sacc = 0.0;
-                sacc += c1 * xw[e]; sacc += c2 * xw[e + 1]; sacc += c3 * xw[e + 2]; sacc += c4 * xw[e + 3]; sacc += c5 * xw[e + 4];
-                const double Ax = sacc * sqrt_w;
-                double cost = dtw * (Ax * Ax);
+                // element i + e: taps -2 .. +2 on x_all
+                double cost = interior_row_cost<1, 5>(p, [&](int o) { return xw[e + o - 1]; });
                 if ((unsigned)(i + e - 3) >= (unsigned)(N - 6)) cost = 0.0;     // band-table rows and the zero padding beyond N
                 if (e & 1) C1 += cost; else C0 += cost;
                 if (kStore && cc_out && i + e >= kPad && i + e < kPad + T) cc_out[i + e - kPad] = cost;
                 // n^T R n term of t = i + e - 6: n_t = nw[2 + e]; zero outside [0, T), no guard needed
-                const double nt = nw[2 + e];
-                double qs = 0.0;
-                qs += r1 * nw[3 + e]; qs += r2 * nw[4 + e]; qs += r3 * nw[5 + e]; qs += r4 * nw[6 + e];
-                const double term = nt * (r0 * nt + 2.0 * qs);
+                const double term = quad_term<4>(p.r_diag, [&](int o) { return nw[2 + e + o]; });
                 if (e & 1) Q1 += term; else Q0 += term;
             }
         }
         double C_part = (C0 + C1) + edge, quad = Q0 + Q1;
         C_part += __shfl_xor_sync(0xffffffffu, C_part, 1); quad += __shfl_xor_sync(0xffffffffu, quad, 1);
         C_part += __shfl_xor_sync(0xffffffffu, C_part, 2); quad += __shfl_xor_sync(0xffffffffu, quad, 2);
-        if (live && kq == 0) {
-            double* srow = p.sums + ((size_t)q * p.gslots + (p.gen_offset + k)) * p.sumw;
-            if (p.rows_mask & 1) {
-                srow[1 + d] = C_part;
-                if (p.c_compact) p.c_compact[((size_t)q * D + d) * p.gslots + (p.gen_offset + k)] = C_part;
-            }
-            if (p.rows_mask & 2) srow[1 + 2 * D + d] = p.use_noise_adaptation ? quad : 0.0;
-        }
+        if (live && kq == 0) store_row_sums(p, q, k, d, C_part, quad);
     }
     tls.end();
 }
@@ -1516,20 +1392,8 @@ fold_control_costs_kernel(const __grid_constant__ LoopParams p)
     const double* th = p.theta_all + ((size_t)q * D + d) * N;
     double* cc = p.control_costs + (((size_t)q * p.slots + k) * D + d) * T;
     auto xall = [&](int j) { return (j >= kPad && j < kPad + T) ? th[j] + nz[j - kPad] : th[j]; };
-    auto row_cost = [&](int i) {
-        const double dtw = p.dt * p.control_cost_weight;
-        double cost = 0.0;
-        for (int r = 0; r < p.num_rules; ++r) {
-            const double* band = p.diff_band + ((size_t)p.rule_id[r] * N + i) * 7;
-            double s = 0.0;
-            for (int j = max(0, i - 3); j <= min(N - 1, i + 3); ++j) s += __ldg(band + (j - i + 3)) * xall(j);
-            const double Ax = s * p.rule_sqrt_w[r];
-            cost += dtw * (Ax * Ax);
-        }
-        return cost;
-    };
     double first = cc[0], last = cc[T - 1];
-    for (int i = 0; i < kPad; ++i) { first += row_cost(i); last += row_cost(N - (i + 1)); }
+    for (int i = 0; i < kPad; ++i) { first += band_row_cost(p, i, xall); last += band_row_cost(p, N - (i + 1), xall); }
     cc[0] = first;
     cc[T - 1] = last;
 }
@@ -1809,7 +1673,6 @@ reused_control_cost_kernel(const __grid_constant__ LoopParams p, int first, int 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     double* x = smem + (size_t)warp * (N + T);
     double* stc = x + N;
-    const RowCoefficients rc = load_row_coefficients(p);
     for (int task = blockIdx.x * nwarps + warp; task < count * D; task += gridDim.x * nwarps) {
         const int r = task / D, d = task - r * D, k = first + r;
         // control costs see parameters_ + noise_projected_ (PolicyImprovement.cpp:812-817), the quadratic form noise_
@@ -1823,7 +1686,7 @@ reused_control_cost_kernel(const __grid_constant__ LoopParams p, int first, int 
         for (int t = lane; t < T; t += 32) stc[t] = p.state_costs[((size_t)q * p.slots + k) * T + t];
         __syncwarp();
         double C_d, cum_d;
-        control_cost_sums(p, rc, x, stc, lane, C_d, cum_d);
+        control_cost_sums(p, x, stc, lane, C_d, cum_d);
         if (p.control_costs) control_cost_store(p, x, lane, p.control_costs + (((size_t)q * p.slots + k) * D + d) * T);
         double s = 0.0;
         for (int t = lane; t < T; t += 32) s += stc[t];
@@ -1835,7 +1698,18 @@ reused_control_cost_kernel(const __grid_constant__ LoopParams p, int first, int 
                 for (int t = lane; t < T; t += 32)
                     x[kPad + t] = p.theta_all[((size_t)q * D + d) * N + kPad + t] + p.noise[(((size_t)q * p.slots + k) * D + d) * T + t];
             }
-            quad = noise_quadratic_form(p, rc, x, p.theta_all + ((size_t)q * D + d) * N, lane);
+            // x becomes the noise x - theta with a zero tail, in place
+            const double* theta_row = p.theta_all + ((size_t)q * D + d) * N;
+            __syncwarp();
+            for (int t = lane; t < T + kPad; t += 32) x[kPad + t] = (t < T) ? x[kPad + t] - theta_row[kPad + t] : 0.0;
+            __syncwarp();
+            const double* n = x + kPad;
+            for (int t = lane; t < T; t += 32) {
+                auto nt = [&](int o) { return n[t + o]; };
+                quad += p.r_toeplitz ? quad_term<kRBand>(p.r_diag, nt)
+                                     : quad_term<kRBand>(p.Rband + (size_t)t * (2 * kRBand + 1) + kRBand, nt);
+            }
+            quad = warp_sum(quad);
         }
         if (lane == 0) {
             double* o = p.sums + ((size_t)q * p.gslots + k) * p.sumw;
@@ -2565,25 +2439,15 @@ __device__ __forceinline__ void apply_update_body(const LoopParams& p, int q, in
         __syncthreads();
         if (threadIdx.x < 32) {
             const int lane = threadIdx.x;
-            const RowCoefficients rc = load_row_coefficients(p);
             double C_d, cum_d;
-            if (p.control_costs == nullptr && p.num_rules == 1 && rc.fast) {
+            if (p.control_costs == nullptr && p.st_uniform) {
                 // the shipped loop: interior rows from the staged row, the six padding-only rows from edge_cost (constants of
                 // the solve, edge_rows_kernel) — no table walk on the critical path of the update kernel
                 double c_sum = 0.0;
-                for (int i = 3 + lane; i < N - 3; i += 32) {
-                    const double* xi = s_row + i - 3;
-                    double acc = 0.0;
-#pragma unroll
-                    for (int o = 0; o < 7; ++o) acc += rc.c[o] * xi[o];
-                    const double Ax = acc * rc.sqrt_w;
-                    c_sum += rc.dtw * (Ax * Ax);
-                }
-                c_sum = warp_sum(c_sum);
-                const double* ec = p.edge_cost + ((size_t)q * D + d) * 6;
-                C_d = c_sum + (((ec[0] + ec[1]) + (ec[2] + ec[3])) + (ec[4] + ec[5]));
+                for (int i = 3 + lane; i < N - 3; i += 32) c_sum += interior_row_cost<0, 6>(p, [&](int o) { return s_row[i - 3 + o]; });
+                C_d = warp_sum(c_sum) + edge_cost_sum(p, q, d);
             } else {
-                control_cost_sums(p, rc, s_row, nullptr, lane, C_d, cum_d);
+                control_cost_sums(p, s_row, nullptr, lane, C_d, cum_d);
                 control_cost_store(p, s_row, lane, p.nl_control + ((size_t)q * D + d) * T);
             }
             if (lane == 0) {
@@ -2639,11 +2503,10 @@ noiseless_rollout_kernel(const __grid_constant__ LoopParams p, const __grid_cons
         __syncthreads();
     }
     // control costs (noise = 0: parameters + 0.0 is exact) and sums
-    const RowCoefficients rc = load_row_coefficients(p);
     for (int task = warp; task < D + 1; task += nwarps) {
         if (task < D) {
             double C_d, cum_d;
-            control_cost_sums(p, rc, sx + (size_t)task * N, sstate, lane, C_d, cum_d);
+            control_cost_sums(p, sx + (size_t)task * N, sstate, lane, C_d, cum_d);
             control_cost_store(p, sx + (size_t)task * N, lane, p.nl_control + ((size_t)q * D + task) * T);
             if (lane == 0) { ssum[1 + task] = C_d; ssum[1 + D + task] = cum_d; ssum[1 + 2 * D + task] = 0.0; }
         } else {

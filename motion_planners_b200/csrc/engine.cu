@@ -194,11 +194,12 @@ struct stomp_b200_engine {
     IterationGraph graphs[2][2];             // [honour_stop][record parity]
     unsigned long long config_epoch = 1;     // bumped by every setter whose values are baked into kernel parameters
     // STOMP_B200_PDL=<mask> at creation: bit 0 sampler, 1 state kernel, 2 weights / update kernel launched as programmatic
-    // dependents of the kernel before them (0: ordinary launches).  Default 5: the state kernel is NOT made a dependent of the
-    // sampler — its CTAs would become resident beside the sampler's, whose 31 KB of shared memory each keep the SM in its
-    // large-shared-memory / small-L1 split, and the state kernel's gathers then run against a sliver of L1: 16.5 -> 34 us
-    // (profiles/r3r_pdl_edges.txt).  In-process A / B (profiles/r3s_ab_steady.txt): 56.5 us per iteration against 59.6.
-    int pdl_mask = 13;                       // + bit 3: the noise-less tail launched alone at a join (84.8 -> 83.9 us per isolated C3 iteration, profiles/r4j_pdl_tail.txt)
+    // dependents of the kernel before them (0: ordinary launches); bit 3 the noise-less tail launched alone at a join (84.8 ->
+    // 83.9 us per isolated C3 iteration, profiles/r4j_pdl_tail.txt).  Default 15, all four.  The state kernel's edge pays only
+    // with its largest-L1 preference (resolve_state_kernel): without it its CTAs become resident beside the sampler's and run
+    // their gathers against a sliver of L1 (16.5 -> 34 us, profiles/r3r_pdl_edges.txt); with it the sampler -> state gap goes
+    // from 3.1 to 1.1 us and the kernel keeps its 16.9 us (isolated C3 iteration 71.8 -> 69.4 us, profiles/r6a_*).
+    int pdl_mask = 15;
     bool graphs_allowed = true;              // STOMP_B200_GRAPH=0 at creation switches the replay off
     bool timer_armed = false, timer_end_recorded = false;   // stomp_b200_timer_begin .. _end: stomp_b200_run records the end event itself
     bool graph_over_overlap = false;         // STOMP_B200_GRAPH=2: replay graphs even where plain launches would overlap the sampler with the update kernel
@@ -565,6 +566,12 @@ void resolve_state_kernel(stomp_b200_engine* e)
     std::string err;
     e->spec = codegen::specialised_state_kernel(e->robot, state_kernel_options(e), err);
     e->spec_note = e->spec ? std::string() : err;
+    // Largest L1: the walk's SDF gathers want it, and an SM whose split is the sampler's (31 KB of shared memory per CTA)
+    // then takes no state CTA until it has drained.  Without the preference, CTAs launched as programmatic dependents of the
+    // sampler fill the room beside its CTAs and keep that small-L1 split: 16.9 -> 36 us (profiles/r6a_*).  A hint only.
+    if (e->spec && cudaKernelSetAttributeForDevice(e->spec->kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                                   (int)cudaSharedmemCarveoutMaxL1, e->cfg.device) != cudaSuccess)
+        (void)cudaGetLastError();
     if (e->spec && e->spec->static_kernel) {
         // Spheres on the axis of a chain's first joint do not move with the state: one thread walks them here, with the
         // statements the state kernel would have issued, and every state starts from that verdict.  Robot, spheres or scene
@@ -645,6 +652,7 @@ StateKernelArgs noiseless_state_args(stomp_b200_engine* e, const LoopParams& lp,
     StateKernelArgs a{};
     a.stop = lp.stop; a.T = lp.T; a.D = lp.D; a.slots = 1; a.gslots = 1; a.sumw = lp.sumw; a.honour_stop = lp.honour_stop;
     if (tail) {
+        a.timeline = lp.timeline ? lp.timeline + 2 * 5 : nullptr;     // the "noiseless" slot: a launch of its own at a join
         a.num_gen = 0; a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
         fill_noiseless_tail(e, lp, e->nl_sums2[e->loop.nl_parity], a.nl);
     } else {

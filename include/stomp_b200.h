@@ -145,6 +145,25 @@ int stomp_b200_build_sdf_scene(stomp_b200_engine* e, const int32_t dims[3], cons
 int stomp_b200_get_sdf(stomp_b200_engine* e, float* out, size_t count, int32_t dims_out[3], double origin_out[3],
                        double* voxel_size_out);
 
+/* ---- scenes: one distance field each; every local query reads the field of its scene ----------------------------------
+ * A batch can hold queries in different worlds (datasets over many environments, benchmark suites of many scenes, a fleet
+ * of cells with their own obstacles).  An engine starts with scene 0, which every query uses; an engine that never calls
+ * the two functions below behaves exactly as before.
+ * select_scene: set_sdf, build_sdf_primitives / _occupancy / _scene, get_sdf and evaluate_states act on `scene` from now
+ * on.  Indices are dense: 0 <= scene <= current number of scenes (selecting that number creates an empty scene).
+ *   - A scene has its own dims, origin and voxel size.
+ *   - Rebuilding a scene, or reassigning queries to scenes, between solves takes effect from the next iteration, in loops
+ *     replayed from CUDA graphs too.
+ *   - begin_solve, iterate, run and solve return STOMP_B200_ERR_NOT_READY while a local query's scene has no field
+ *     (stomp_b200_last_error names the query and the scene).
+ *   - A bad query range, a negative scene or a scene that does not exist: STOMP_B200_ERR_INVALID_ARGUMENT.
+ *   - Query indices are local, as for policies: under query sharding each rank holds the scenes its caller gives it.
+ * The Philox noise of a query does not depend on its scene: a batch spread over several scenes draws what the same batch
+ * in one scene draws. */
+int stomp_b200_select_scene(stomp_b200_engine* e, int32_t scene);
+/* scene[i] for local queries first_query .. first_query + count - 1 (query-major like stomp_b200_set_policies). */
+int stomp_b200_set_query_scenes(stomp_b200_engine* e, int32_t first_query, int32_t count, const int32_t* scene);
+
 /* ---- policy: the host-computed products of CovariantMovementPrimitive::initialize ----------------------
  * (CovariantMovementPrimitive.cpp:57-74,136-301; computed by stomp_b200_host_policy below or by the
  * C++ stomp::CovariantMovementPrimitive in include/stomp/).  R = control_costs_, Rinv = inv_control_costs_,

@@ -39,6 +39,7 @@ SYMBOLS = [
     "stomp_b200_state_kernel_kind", "stomp_b200_state_kernel_source", "stomp_b200_codegen_selftest",
     "stomp_b200_set_cost_cumulation", "stomp_b200_set_self_collision", "stomp_b200_set_cost_extras",
     "stomp_b200_build_sdf_primitives", "stomp_b200_build_sdf_occupancy", "stomp_b200_build_sdf_scene", "stomp_b200_get_sdf",
+    "stomp_b200_select_scene", "stomp_b200_set_query_scenes",
 ]
 
 
@@ -99,6 +100,8 @@ def lib():
         L.stomp_b200_build_sdf_occupancy.argtypes = [vp, ip, dp, C.c_double, u8p]
         L.stomp_b200_build_sdf_scene.argtypes = [vp, ip, dp, C.c_double, C.c_int32, dp, C.c_int32, C.c_int32, dp, dp, u8p]
         L.stomp_b200_get_sdf.argtypes = [vp, C.POINTER(C.c_float), C.c_size_t, ip, dp, dp]
+        L.stomp_b200_select_scene.argtypes = [vp, C.c_int32]
+        L.stomp_b200_set_query_scenes.argtypes = [vp, C.c_int32, C.c_int32, ip]
         L.stomp_b200_set_control_cost_matrices.argtypes = [vp, dp, dp, dp]
         L.stomp_b200_set_policy.argtypes = [vp, C.c_int32, dp, dp]
         L.stomp_b200_set_policies.argtypes = [vp, C.c_int32, C.c_int32, dp, dp]
@@ -321,6 +324,16 @@ class Engine:
                     "stomp_b200_get_sdf")
         return out, org, vox.value
 
+    def select_scene(self, scene):
+        """The scene the SDF setters, builders, get_sdf and evaluate_states act on from now on; selecting the current
+        number of scenes creates an empty one (stomp_b200_select_scene)."""
+        self._check(lib().stomp_b200_select_scene(self.h, int(scene)), "stomp_b200_select_scene")
+
+    def set_query_scenes(self, first_query, scenes):
+        """scenes[i]: the scene local query first_query + i plans in (stomp_b200_set_query_scenes)."""
+        sc = np.ascontiguousarray(scenes, dtype=np.int32).reshape(-1)
+        self._check(lib().stomp_b200_set_query_scenes(self.h, int(first_query), len(sc), _ip(sc)), "stomp_b200_set_query_scenes")
+
     def set_matrices(self, R, Rinv, L):
         R, L = _c64(R), _c64(L)
         Rinv = None if Rinv is None else _c64(Rinv)
@@ -340,10 +353,18 @@ class Engine:
 
     def set_problem(self, problem, policy=None):
         """Scene + StompPlanner::setStartGoalTrajectory for every local query.  `policy`, when given, is a
-        dict (R, Rinv, L, params_all, mincc) shared with the oracle in parity tests."""
+        dict (R, Rinv, L, params_all, mincc) shared with the oracle in parity tests.  A problem with a list of scenes
+        (problems.batch_problem_scenes) gets one field per scene and each query the scene of its query_scene entry."""
         self.set_chain(problem.chain)
         self.set_spheres(problem.spheres)
-        self.set_sdf(problem.sdf)
+        if problem.scenes:
+            for i, sdf in enumerate(problem.scenes):
+                self.select_scene(i)
+                self.set_sdf(sdf)
+            self.select_scene(0)
+            self.set_query_scenes(0, np.asarray(problem.query_scene)[self.query_offset:self.query_offset + self.Q])
+        else:
+            self.set_sdf(problem.sdf)
         starts = np.atleast_2d(problem.start)
         goals = np.atleast_2d(problem.goal)
         pol = policy

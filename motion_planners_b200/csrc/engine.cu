@@ -122,11 +122,24 @@ struct stomp_b200_engine {
 
     RobotParams robot;
     JointLimits limits;             // robot.lower / upper, for the sampling kernels
-    SdfParams sdf;
-    float* d_sdf = nullptr;
-    size_t sdf_count = 0;
-    double sdf_origin[3] = {0, 0, 0}, sdf_voxel = 0;
-    CostExtras extras;              // stomp_b200_set_cost_extras; all zero: the shipped 0 / 1 state cost
+    // Scenes: one distance field each (stomp_b200_select_scene / stomp_b200_set_query_scenes).  The SDF setters, builders,
+    // get_sdf and evaluate_states act on scenes[selected]; local query q reads scenes[query_scene[q]].  With one scene the
+    // kernels take its SdfParams as their argument, exactly as before scenes existed; with more, the loop's kernels read
+    // their query's record from d_query_sdf (LoopParams / StateKernelArgs::query_sdf).
+    struct Scene {
+        SdfParams sdf{};            // grid == d_grid
+        float* d_grid = nullptr;
+        size_t count = 0;
+        double origin[3] = {0, 0, 0}, voxel = 0;
+        bool have = false;          // the grid holds a field
+    };
+    std::vector<Scene> scenes = std::vector<Scene>(1);
+    int selected = 0;
+    std::vector<int32_t> query_scene;         // [Q]
+    std::vector<SdfParams> query_sdf_staging; // [Q] host side of d_query_sdf
+    SdfParams* d_query_sdf = nullptr;        // [Q] scenes[query_scene[q]].sdf, rewritten on the main stream at every change
+    int32_t* d_query_scene = nullptr;         // [Q]
+    CostExtras extras;             // stomp_b200_set_cost_extras; all zero: the shipped 0 / 1 state cost
     bool extras_on = false;
     SelfPairs self_pairs = {nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0};   // stomp_b200_set_self_collision; n == 0: world collisions only
     std::vector<void*> self_pair_buffers;
@@ -137,7 +150,7 @@ struct stomp_b200_engine {
     const codegen::SpecialisedKernel* spec_self = nullptr;
     bool spec_self_resolved = false;
     std::string spec_self_note;
-    bool have_chain = false, have_spheres = false, have_sdf = false, have_matrices = false;
+    bool have_chain = false, have_spheres = false, have_matrices = false;
     std::vector<uint8_t> have_policy;
 
     LoopParams base;                // pointers + constants; per-iteration fields filled in iterate
@@ -218,7 +231,8 @@ struct stomp_b200_engine {
     // the chain / spheres / SDF changed
     const codegen::SpecialisedKernel* spec = nullptr;
     bool spec_resolved = false;
-    int32_t* d_static_hit = nullptr;         // verdict of the spheres no joint value moves (stomp_b200_static_spheres), rewritten whenever the state kernel is resolved
+    int32_t* d_static_hit = nullptr;         // [scene] verdict of the spheres no joint value moves (stomp_b200_static_spheres), rewritten whenever the state kernel is resolved
+    size_t static_capacity = 0;
     std::string spec_note;          // why the generic kernel is in use, when it is
 
     // pinned host mirrors of the per-query scalars
@@ -535,14 +549,23 @@ int launch_rows(stomp_b200_engine* e, const LoopParams& rl, RowsShape shape, int
 codegen::StateKernelOptions state_kernel_options(const stomp_b200_engine* e)
 {
     codegen::StateKernelOptions opt;
-    opt.wide_index = e->sdf.wide_index != 0;
     // The two bounds below hold for ANY value of a revolute joint, but only inside the limits of a prismatic one — and the
     // noise-less rollout (policy parameters) and stomp_b200_evaluate_states (caller's values) are not clamped to the limits:
     // chains with a prismatic joint keep the index clamps and the saturating conversion.
     bool has_prismatic = false;
     for (int d = 0; d < e->robot.num_joints; ++d) has_prismatic = has_prismatic || e->robot.joint[d].prismatic != 0;
-    opt.magic_floor = !has_prismatic && codegen::magic_floor_is_safe(e->robot, e->sdf);
-    opt.inside_grid = !has_prismatic && codegen::reach_is_inside_grid(e->robot, e->sdf);
+    // One kernel serves every scene: the index width and the two bounds must hold for each field it can be handed
+    opt.per_query_field = e->scenes.size() > 1;
+    std::vector<const SdfParams*> fields;
+    for (const stomp_b200_engine::Scene& s : e->scenes)
+        if (s.have) fields.push_back(&s.sdf);
+    if (fields.empty()) fields.push_back(&e->scenes[0].sdf);     // no field yet: the bounds of the empty geometry
+    opt.magic_floor = opt.inside_grid = !has_prismatic;
+    for (const SdfParams* g : fields) {
+        opt.wide_index = opt.wide_index || g->wide_index != 0;
+        opt.magic_floor = opt.magic_floor && codegen::magic_floor_is_safe(e->robot, *g);
+        opt.inside_grid = opt.inside_grid && codegen::reach_is_inside_grid(e->robot, *g);
+    }
     // links between issuing a link's gathers and comparing them.  With the static spheres out of the walk the 7-joint arm is
     // fastest comparing one link later (16.1 against 16.9 us at lag 2 and 17.7 at lag 0, C3 in the loop; 16.9 / 17.8 / 18.4
     // isolated and flushed), the 14-joint dual arm two links later (41.5 against 44.0 us at lag 1): profiles/r5s_*
@@ -574,16 +597,22 @@ void resolve_state_kernel(stomp_b200_engine* e)
         (void)cudaGetLastError();
     if (e->spec && e->spec->static_kernel) {
         // Spheres on the axis of a chain's first joint do not move with the state: one thread walks them here, with the
-        // statements the state kernel would have issued, and every state starts from that verdict.  Robot, spheres or scene
-        // changing resets spec_resolved (set_chain / set_spheres / the SDF setters and builders), which brings us back here;
-        // the launch is ordered on the main stream behind the copy or build that produced the grid.
+        // statements the state kernel would have issued, and every state starts from that verdict — one per scene, and a
+        // query starts from its scene's.  Robot, spheres or a scene changing resets spec_resolved (set_chain / set_spheres /
+        // select_scene / the SDF setters and builders), which brings us back here; the launches are ordered on the main
+        // stream behind the copies or builds that produced the grids.
         cudaError_t rc = cudaSuccess;
-        if (!e->d_static_hit) {
-            rc = cudaMalloc((void**)&e->d_static_hit, sizeof(int32_t));
-            if (rc == cudaSuccess) e->allocations.push_back(e->d_static_hit);
+        if (e->static_capacity < e->scenes.size()) {
+            if (e->d_static_hit) cudaFree(e->d_static_hit);
+            e->d_static_hit = nullptr;
+            e->static_capacity = 0;
+            rc = cudaMalloc((void**)&e->d_static_hit, sizeof(int32_t) * e->scenes.size());
+            if (rc == cudaSuccess) e->static_capacity = e->scenes.size();
         }
-        if (rc == cudaSuccess) {
-            void* args[] = {&e->robot, &e->sdf, &e->d_static_hit};
+        for (size_t s = 0; s < e->scenes.size() && rc == cudaSuccess; ++s) {
+            if (!e->scenes[s].have) continue;
+            int32_t* out = e->d_static_hit + s;
+            void* args[] = {&e->robot, &e->scenes[s].sdf, &out};
             rc = cudaLaunchKernel((const void*)e->spec->static_kernel, dim3(1), dim3(32), args, 0, e->stream);
             e->launch_count++;
         }
@@ -604,11 +633,12 @@ void resolve_state_kernel(stomp_b200_engine* e)
 // the two arguments of the specialised kernel that come from the engine rather than from the loop: the verdict of the static
 // spheres, and the multiplier that replaces idx / T where the host can prove it exact (M = floor(2^32 / T) + 1 has
 // M T = 2^32 + r with 0 < r <= T, so umulhi(idx, M) = floor(idx / T + idx r / (T 2^32)) = idx / T whenever idx r < 2^32).
-// The static verdict exists once the state kernel is resolved, so that happens here.
-void finish_state_args(stomp_b200_engine* e, StateKernelArgs& a)
+// The static verdict exists once the state kernel is resolved, so that happens here.  `scene`: the field of a pass without
+// a per-query table (a.query_sdf null).
+void finish_state_args(stomp_b200_engine* e, StateKernelArgs& a, int scene)
 {
     resolve_state_kernel(e);
-    a.static_hit = (e->spec && e->spec->static_kernel) ? e->d_static_hit : nullptr;
+    a.static_hit = (e->spec && e->spec->static_kernel) ? e->d_static_hit + (a.query_sdf ? 0 : scene) : nullptr;
     const unsigned long long T = (unsigned long long)std::max(a.T, 0), n = (unsigned long long)std::max(a.num_gen, 0);
     a.t_magic = (T >= 2 && n * T * T < (1ull << 32)) ? (uint32_t)((1ull << 32) / T + 1) : 0u;
 }
@@ -639,8 +669,9 @@ StateKernelArgs rollout_state_args(stomp_b200_engine* e, const LoopParams& lp, b
     a.T = lp.T; a.D = lp.D; a.slots = lp.slots; a.gslots = lp.gslots; a.sumw = lp.sumw; a.num_gen = lp.num_gen;
     a.gen_offset = lp.gen_offset; a.honour_stop = lp.honour_stop;
     a.row_stride = lp.T; a.rollout_stride = (int64_t)lp.D * lp.T;
+    a.query_sdf = lp.query_sdf; a.query_scene = lp.query_scene;
     if (tail) fill_noiseless_tail(e, lp, lp.nl_sums, a.nl);
-    finish_state_args(e, a);
+    finish_state_args(e, a, 0);
     return a;
 }
 
@@ -659,11 +690,12 @@ StateKernelArgs noiseless_state_args(stomp_b200_engine* e, const LoopParams& lp,
         a.rollouts = lp.theta_all + kPad; a.state_costs = lp.nl_state; a.verdicts = lp.nl_verdict; a.validity = lp.nl_valid;
         a.num_gen = 1; a.row_stride = lp.N; a.rollout_stride = (int64_t)lp.D * lp.N;
     }
-    finish_state_args(e, a);
+    a.query_sdf = lp.query_sdf; a.query_scene = lp.query_scene;
+    finish_state_args(e, a, 0);
     return a;
 }
 
-// the caller's trajectories theta [K][D][T] of stomp_b200_evaluate_states, as one query
+// the caller's trajectories theta [K][D][T] of stomp_b200_evaluate_states, as one query in the selected scene
 StateKernelArgs trajectory_state_args(stomp_b200_engine* e, const double* theta, int K, int T, double* costs, uint8_t* verdicts,
                                       uint8_t* validity)
 {
@@ -671,7 +703,7 @@ StateKernelArgs trajectory_state_args(stomp_b200_engine* e, const double* theta,
     a.rollouts = theta; a.state_costs = costs; a.verdicts = verdicts; a.validity = validity;
     a.T = T; a.D = e->D; a.slots = K; a.gslots = 1; a.sumw = 1; a.num_gen = K;
     a.row_stride = T; a.rollout_stride = (int64_t)e->D * T;
-    finish_state_args(e, a);
+    finish_state_args(e, a, e->selected);
     return a;
 }
 
@@ -681,9 +713,10 @@ StateKernelArgs trajectory_state_args(stomp_b200_engine* e, const double* theta,
 // kernels leave out clamps only such values make redundant).  The grids have codegen::kStateThreads threads per CTA; the
 // tail's CTAs come first (state_codegen.hpp).  The caller counts the launch (its profiling Scope, or the noise-less rollout's
 // category).
-int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream_t stream, int queries, int pdl_bit, bool sane)
+int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream_t stream, int queries, int pdl_bit, bool sane, int scene = 0)
 {
     resolve_state_kernel(e);
+    SdfParams sdf = e->scenes[scene].sdf;     // the kernels' argument: read unless a.query_sdf is set
     constexpr int bt = codegen::kStateThreads;
     const unsigned tail_blocks = a.nl.theta ? (unsigned)((a.T + bt - 1) / bt) : 0u;
     const dim3 grid((unsigned)(((long long)a.num_gen * a.T + bt - 1) / bt) + tail_blocks, (unsigned)queries), block(bt);
@@ -692,14 +725,14 @@ int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream
         if (e->spec_self && sane) {
             constexpr int tw = bt / 32;      // time steps per CTA when the lanes of a warp are rollouts
             const dim3 lanes_grid((unsigned)((a.num_gen + 31) / 32) * (unsigned)((a.T + tw - 1) / tw), grid.y);
-            void* args[] = {(void*)&a, &e->robot, &e->sdf, &e->self_pairs, e->self_bands.data()};
+            void* args[] = {(void*)&a, &e->robot, &sdf, &e->self_pairs, e->self_bands.data()};
             (void)cudaLaunchKernel((const void*)e->spec_self->kernel, e->spec_self->rollout_lanes ? lanes_grid : grid, block, args, 0, stream);
             return check_launch(e, "stomp_b200_states_specialised (pair rule)");
         }
         const int S = e->robot.num_spheres;
         auto walk = [&](auto simple_kernel, auto kernel) {
-            if (e->robot.simple_chain) simple_kernel<<<grid, block, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
-            else kernel<<<grid, block, 0, stream>>>(a, e->robot, e->sdf, e->self_pairs);
+            if (e->robot.simple_chain) simple_kernel<<<grid, block, 0, stream>>>(a, e->robot, sdf, e->self_pairs);
+            else kernel<<<grid, block, 0, stream>>>(a, e->robot, sdf, e->self_pairs);
         };
         if (S <= 32) walk(states_self_collision_kernel<32, true>, states_self_collision_kernel<32, false>);
         else if (S <= 64) walk(states_self_collision_kernel<64, true>, states_self_collision_kernel<64, false>);
@@ -707,15 +740,15 @@ int launch_state_pass(stomp_b200_engine* e, const StateKernelArgs& a, cudaStream
         return check_launch(e, "states_self_collision_kernel");
     }
     if (e->spec && sane) {
-        void* args[] = {(void*)&a, &e->robot, &e->sdf};
+        void* args[] = {(void*)&a, &e->robot, &sdf};
         // Only this kernel may be a programmatic dependent: it is the only state kernel that executes griddepcontrol.wait.
         // Any other, launched that way, could read the stop flag and its joint values before the kernel before it wrote them.
         if (pdl_bit >= 0) (void)launch_dependent(e, pdl_bit, (const void*)e->spec->kernel, grid, block, 0, stream, args);
         else (void)cudaLaunchKernel((const void*)e->spec->kernel, grid, block, args, 0, stream);
         return check_launch(e, "stomp_b200_states_specialised");
     }
-    if (e->robot.simple_chain) rollout_states_kernel<true><<<grid, block, 0, stream>>>(a, e->robot, e->sdf);
-    else rollout_states_kernel<false><<<grid, block, 0, stream>>>(a, e->robot, e->sdf);
+    if (e->robot.simple_chain) rollout_states_kernel<true><<<grid, block, 0, stream>>>(a, e->robot, sdf);
+    else rollout_states_kernel<false><<<grid, block, 0, stream>>>(a, e->robot, sdf);
     return check_launch(e, "rollout_states_kernel");
 }
 
@@ -741,7 +774,7 @@ int launch_noiseless(stomp_b200_engine* e, bool on_main_stream)
     e->kernel_launches[STOMP_B200_KERNEL_APPLY]++;
     if (!tail) {
         const size_t smem = sizeof(double) * ((size_t)e->D * e->N + e->T + e->sumw);
-        noiseless_rollout_kernel<<<e->Q, 256, smem, st>>>(lp, e->robot, e->sdf, e->extras);
+        noiseless_rollout_kernel<<<e->Q, 256, smem, st>>>(lp, e->robot, e->scenes[0].sdf, e->extras);
         e->launch_count++;
         if (int rc = check_launch(e, "noiseless_rollout_kernel")) return rc;
     }
@@ -1055,7 +1088,7 @@ int iterate_body(stomp_b200_engine* e, int iteration, int mode, int honour_stop,
         Scope sc(e, STOMP_B200_KERNEL_COST);
         if (int rc = launch_state_pass(e, rollout_state_args(e, lp, tail_in_state_kernel), e->stream, e->Q, 1, true)) return rc;
         if (e->extras_on) {     // alternative state costs: a pass of their own, then S_k in a fixed order
-            state_cost_extras_kernel<<<dim3((states + 127) / 128, e->Q), 128, 0, e->stream>>>(lp, e->robot, e->sdf, e->extras);
+            state_cost_extras_kernel<<<dim3((states + 127) / 128, e->Q), 128, 0, e->stream>>>(lp, e->robot, e->scenes[0].sdf, e->extras);
             if (int rc = check_launch(e, "state_cost_extras_kernel")) return rc;
             state_row_sums_kernel<<<dim3((gen_local + 7) / 8, e->Q), 256, 0, e->stream>>>(lp);
             if (int rc = check_launch(e, "state_row_sums_kernel")) return rc;
@@ -1299,12 +1332,37 @@ int setup_peer_exchange(stomp_b200_engine* e)
     return 0;
 }
 
+// every local query's scene holds a field (begin_solve, iterate, run and solve ask)
+int scenes_ready(stomp_b200_engine* e)
+{
+    for (int q = 0; q < e->Q; ++q)
+        if (!e->scenes[e->query_scene[q]].have) {
+            e->last_error = "query " + std::to_string(q) + " reads scene " + std::to_string(e->query_scene[q]) + ", which has no distance field";
+            return STOMP_B200_ERR_NOT_READY;
+        }
+    return 0;
+}
+
 int ready_to_solve(stomp_b200_engine* e)
 {
-    if (!e->have_chain || !e->have_spheres || !e->have_sdf || !e->have_matrices)
+    if (!e->have_chain || !e->have_spheres || (e->scenes.size() == 1 && !e->scenes[0].have) || !e->have_matrices)
         return fail(e, STOMP_B200_ERR_NOT_READY, "chain, spheres, SDF and control-cost matrices must be set first");
+    if (int rc = scenes_ready(e)) return rc;
     for (int q = 0; q < e->Q; ++q)
         if (!e->have_policy[q]) return fail(e, STOMP_B200_ERR_NOT_READY, "stomp_b200_set_policy missing for a query");
+    return 0;
+}
+
+// the per-query table as the assignment and the scenes are now (engines with several scenes): copied on the main stream,
+// behind every kernel queued there, and waited for, so that the host staging may change again at the next call
+int upload_query_fields(stomp_b200_engine* e)
+{
+    if (e->scenes.size() < 2) return 0;
+    e->query_sdf_staging.resize((size_t)e->Q);
+    for (int q = 0; q < e->Q; ++q) e->query_sdf_staging[q] = e->scenes[e->query_scene[q]].sdf;
+    CUDA_TRY(e, cudaMemcpyAsync(e->d_query_sdf, e->query_sdf_staging.data(), sizeof(SdfParams) * e->Q, cudaMemcpyHostToDevice, e->stream));
+    CUDA_TRY(e, cudaMemcpyAsync(e->d_query_scene, e->query_scene.data(), sizeof(int32_t) * e->Q, cudaMemcpyHostToDevice, e->stream));
+    CUDA_TRY(e, cudaStreamSynchronize(e->stream));
     return 0;
 }
 
@@ -1540,6 +1598,9 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
     CREATE_TRY(dev_alloc(e, &b.old_cost, Q));
     CREATE_TRY(dev_alloc(e, &b.best_cost, Q));
     CREATE_TRY(dev_alloc(e, &e->d_order, Q * S));
+    CREATE_TRY(dev_alloc(e, &e->d_query_sdf, Q));
+    CREATE_TRY(dev_alloc(e, &e->d_query_scene, Q));
+    e->query_scene.assign(Q, 0);
     // rollouts per CTA of the weights / update kernels: the kernels are latency chains (cost scan -> exp -> stream of the
     // chunk's rows -> last-CTA reduction), so shorter chunks finish sooner — as long as the grid stays ONE wave (three
     // 256-thread CTAs per SM at 80 registers).  Measured at K = 4096 on one GPU: 128 -> 14.2 us (231 CTAs), 64 -> 15.4 us
@@ -1626,7 +1687,6 @@ int stomp_b200_create(const stomp_b200_config* cfg, stomp_b200_engine** out)
     CREATE_CUDA(cudaFuncSetAttribute(reuse_rollouts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
     if (const char* f = std::getenv("STOMP_B200_FUSE_WEIGHTS")) e->fuse_weights_allowed = std::strcmp(f, "0") != 0;
     std::memset(&e->robot, 0, sizeof(e->robot));
-    std::memset(&e->sdf, 0, sizeof(e->sdf));
     CREATE_CUDA(cudaStreamSynchronize(e->stream));
 #undef CREATE_TRY
 #undef CREATE_CUDA
@@ -1648,7 +1708,9 @@ int stomp_b200_destroy(stomp_b200_engine* e)
     release_peer_exchange(e);
     if (e->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(e->comm);
     for (void* p : e->allocations) cudaFree(p);
-    if (e->d_sdf) cudaFree(e->d_sdf);
+    for (auto& sc : e->scenes)
+        if (sc.d_grid) cudaFree(sc.d_grid);
+    if (e->d_static_hit) cudaFree(e->d_static_hit);
     for (void* p : e->self_pair_buffers) cudaFree(p);
     if (e->eval_theta) cudaFree(e->eval_theta);
     if (e->eval_cost) cudaFree(e->eval_cost);
@@ -1924,28 +1986,32 @@ int stomp_b200_set_self_collision(stomp_b200_engine* e, int32_t num_pairs, const
     return STOMP_B200_OK;
 }
 
-// (re)allocates the device grid and records its geometry; the caller fills it
+// (re)allocates the selected scene's device grid and records its geometry; the caller fills it
 static int adopt_sdf_geometry(stomp_b200_engine* e, const int32_t dims[3], const double origin[3], double voxel_size)
 {
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
     const size_t count = (size_t)dims[0] * dims[1] * dims[2];
     CUDA_TRY(e, cudaStreamSynchronize(e->stream));
     if (e->side_stream) CUDA_TRY(e, cudaStreamSynchronize(e->side_stream));
-    if (e->d_sdf && e->sdf_count != count) { cudaFree(e->d_sdf); e->d_sdf = nullptr; }
-    if (!e->d_sdf) {
-        e->have_sdf = false;
-        CUDA_TRY(e, cudaMalloc(&e->d_sdf, count * sizeof(float)));
-        e->sdf_count = count;
+    stomp_b200_engine::Scene& sc = e->scenes[e->selected];
+    if (sc.d_grid && sc.count != count) { cudaFree(sc.d_grid); sc.d_grid = nullptr; }
+    if (!sc.d_grid) {
+        sc.have = false;
+        CUDA_TRY(e, cudaMalloc(&sc.d_grid, count * sizeof(float)));
+        sc.count = count;
     }
-    e->sdf.grid = e->d_sdf;
-    e->sdf.nx = dims[0]; e->sdf.ny = dims[1]; e->sdf.nz = dims[2];
-    e->sdf.inv_h = 1.0 / voxel_size;
-    e->sdf.offx = -(origin[0] * e->sdf.inv_h); e->sdf.offy = -(origin[1] * e->sdf.inv_h); e->sdf.offz = -(origin[2] * e->sdf.inv_h);
-    e->sdf.wide_index = count >= ((size_t)1 << 31) ? 1 : 0;
-    e->sdf_origin[0] = origin[0]; e->sdf_origin[1] = origin[1]; e->sdf_origin[2] = origin[2];
-    e->sdf_voxel = voxel_size;
+    SdfParams& g = sc.sdf;
+    g.grid = sc.d_grid;
+    g.nx = dims[0]; g.ny = dims[1]; g.nz = dims[2];
+    g.inv_h = 1.0 / voxel_size;
+    g.offx = -(origin[0] * g.inv_h); g.offy = -(origin[1] * g.inv_h); g.offz = -(origin[2] * g.inv_h);
+    g.wide_index = count >= ((size_t)1 << 31) ? 1 : 0;
+    sc.origin[0] = origin[0]; sc.origin[1] = origin[1]; sc.origin[2] = origin[2];
+    sc.voxel = voxel_size;
     e->spec_resolved = false;
+    e->spec_self_resolved = false;      // the bounds of the generated kernels follow the set of fields
     e->config_epoch++;
+    if (int rc = upload_query_fields(e)) return rc;
     return STOMP_B200_OK;
 }
 
@@ -1954,8 +2020,9 @@ int stomp_b200_set_sdf(stomp_b200_engine* e, const int32_t dims[3], const double
     if (!e || !dims || !origin || !grid || !(voxel_size > 0.0)) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (dims[0] < 1 || dims[1] < 1 || dims[2] < 1) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (int rc = adopt_sdf_geometry(e, dims, origin, voxel_size)) return rc;
-    CUDA_TRY(e, cudaMemcpy(e->d_sdf, grid, e->sdf_count * sizeof(float), cudaMemcpyHostToDevice));
-    e->have_sdf = true;
+    stomp_b200_engine::Scene& sc = e->scenes[e->selected];
+    CUDA_TRY(e, cudaMemcpy(sc.d_grid, grid, sc.count * sizeof(float), cudaMemcpyHostToDevice));
+    sc.have = true;
     return STOMP_B200_OK;
 }
 
@@ -1982,22 +2049,23 @@ int stomp_b200_build_sdf_primitives(stomp_b200_engine* e, const int32_t dims[3],
     cudaError_t err = cudaMemcpy(d_list, &pl, sizeof(PrimitiveList), cudaMemcpyHostToDevice);
     if (err == cudaSuccess) {
         build_sdf_primitives_kernel<<<dim3((dims[0] + 127) / 128, dims[1], dims[2]), 128, 0, e->stream>>>(
-            e->d_sdf, dims[0], dims[1], dims[2], origin[0], origin[1], origin[2], voxel_size, d_list);
+            e->scenes[e->selected].d_grid, dims[0], dims[1], dims[2], origin[0], origin[1], origin[2], voxel_size, d_list);
         e->launch_count++;
         err = cudaGetLastError();
     }
     if (err == cudaSuccess) err = cudaStreamSynchronize(e->stream);
     cudaFree(d_list);
     if (err != cudaSuccess) { e->last_error = std::string("build_sdf_primitives: ") + cudaGetErrorString(err); return STOMP_B200_ERR_CUDA; }
-    e->have_sdf = true;
+    e->scenes[e->selected].have = true;
     return STOMP_B200_OK;
 }
 
-// exact signed Euclidean distance transform of a device occupancy grid into e->d_sdf (geometry already adopted)
+// exact signed Euclidean distance transform of a device occupancy grid into the selected scene's grid (geometry already adopted)
 static int edt_from_device_occupancy(stomp_b200_engine* e, const uint8_t* d_occ, const char* what)
 {
-    const size_t count = e->sdf_count;
-    const int nx = e->sdf.nx, ny = e->sdf.ny, nz = e->sdf.nz;
+    const stomp_b200_engine::Scene& sc = e->scenes[e->selected];
+    const size_t count = sc.count;
+    const int nx = sc.sdf.nx, ny = sc.sdf.ny, nz = sc.sdf.nz;
     int32_t* d_a = nullptr; int32_t* d_b = nullptr; int32_t* d_c = nullptr;
     auto cleanup = [&]() { cudaFree(d_a); cudaFree(d_b); cudaFree(d_c); };
     cudaError_t err = cudaMalloc(&d_a, count * sizeof(int32_t));
@@ -2015,7 +2083,7 @@ static int edt_from_device_occupancy(stomp_b200_engine* e, const uint8_t* d_occ,
         };
         transform(d_a);
         transform(d_b);
-        finish_edt_kernel<<<blocks, 256, 0, e->stream>>>(d_occ, d_a, d_b, e->d_sdf, e->sdf_voxel, count);
+        finish_edt_kernel<<<blocks, 256, 0, e->stream>>>(d_occ, d_a, d_b, sc.d_grid, sc.voxel, count);
         e->launch_count += 8;
         err = cudaGetLastError();
     }
@@ -2045,7 +2113,7 @@ int stomp_b200_build_sdf_scene(stomp_b200_engine* e, const int32_t dims[3], cons
         if (!(leaf_sizes[i] > 0.0) || !(std::fabs(leaf_centres[3 * i]) <= 1e9) || !(std::fabs(leaf_centres[3 * i + 1]) <= 1e9) || !(std::fabs(leaf_centres[3 * i + 2]) <= 1e9))
             return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "octomap leaf: centre not finite or size not positive");
     if (int rc = adopt_sdf_geometry(e, dims, origin, voxel_size)) return rc;
-    const size_t count = e->sdf_count;
+    const size_t count = e->scenes[e->selected].count;
     const int nx = dims[0], ny = dims[1], nz = dims[2];
     uint8_t* d_occ = nullptr; uint8_t* d_out = nullptr; double* d_tri = nullptr; double* d_leaf = nullptr; int* d_flag = nullptr;
     auto cleanup = [&]() { cudaFree(d_occ); cudaFree(d_out); cudaFree(d_tri); cudaFree(d_leaf); cudaFree(d_flag); };
@@ -2098,24 +2166,60 @@ int stomp_b200_build_sdf_scene(stomp_b200_engine* e, const int32_t dims[3], cons
     const int rc = edt_from_device_occupancy(e, d_occ, "build_sdf_scene");
     cleanup();
     if (rc) return rc;
-    e->have_sdf = true;
+    e->scenes[e->selected].have = true;
     return STOMP_B200_OK;
 }
 
 int stomp_b200_get_sdf(stomp_b200_engine* e, float* out, size_t count, int32_t dims_out[3], double origin_out[3], double* voxel_size_out)
 {
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
-    if (!e->have_sdf) return fail(e, STOMP_B200_ERR_NOT_READY, "no distance field set");
-    if (dims_out) { dims_out[0] = e->sdf.nx; dims_out[1] = e->sdf.ny; dims_out[2] = e->sdf.nz; }
-    if (origin_out) { origin_out[0] = e->sdf_origin[0]; origin_out[1] = e->sdf_origin[1]; origin_out[2] = e->sdf_origin[2]; }
-    if (voxel_size_out) *voxel_size_out = e->sdf_voxel;
+    const stomp_b200_engine::Scene& sc = e->scenes[e->selected];
+    if (!sc.have) return fail(e, STOMP_B200_ERR_NOT_READY, "no distance field set");
+    if (dims_out) { dims_out[0] = sc.sdf.nx; dims_out[1] = sc.sdf.ny; dims_out[2] = sc.sdf.nz; }
+    if (origin_out) { origin_out[0] = sc.origin[0]; origin_out[1] = sc.origin[1]; origin_out[2] = sc.origin[2]; }
+    if (voxel_size_out) *voxel_size_out = sc.voxel;
     if (out) {
-        if (count != e->sdf_count) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "count does not match the grid");
+        if (count != sc.count) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "count does not match the grid");
         CUDA_TRY(e, cudaSetDevice(e->cfg.device));
         CUDA_TRY(e, cudaStreamSynchronize(e->stream));
-        CUDA_TRY(e, cudaMemcpy(out, e->d_sdf, count * sizeof(float), cudaMemcpyDeviceToHost));
+        CUDA_TRY(e, cudaMemcpy(out, sc.d_grid, count * sizeof(float), cudaMemcpyDeviceToHost));
     }
     return STOMP_B200_OK;
+}
+
+int stomp_b200_select_scene(stomp_b200_engine* e, int32_t scene)
+{
+    if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
+    if (scene < 0 || (size_t)scene > e->scenes.size())
+        return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "scene out of range: 0 .. number of scenes (which creates one)");
+    if ((size_t)scene == e->scenes.size()) {
+        CUDA_TRY(e, cudaSetDevice(e->cfg.device));
+        e->scenes.emplace_back();
+        // from two scenes on, the loop's kernels read their query's field from the table (the state kernel is generated
+        // with the per-query branch; a noise-less rollout still owed was set up without the table and reads scene 0)
+        e->base.query_sdf = e->d_query_sdf;
+        e->base.query_scene = e->d_query_scene;
+        e->spec_resolved = false;
+        e->spec_self_resolved = false;
+        e->config_epoch++;
+        if (int rc = upload_query_fields(e)) return rc;
+    }
+    e->selected = scene;
+    return STOMP_B200_OK;
+}
+
+int stomp_b200_set_query_scenes(stomp_b200_engine* e, int32_t first_query, int32_t count, const int32_t* scene)
+{
+    if (!e || !scene) return STOMP_B200_ERR_INVALID_ARGUMENT;
+    if (count < 1 || first_query < 0 || first_query > e->Q - count) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "query range out of bounds");
+    for (int i = 0; i < count; ++i)
+        if (scene[i] < 0 || (size_t)scene[i] >= e->scenes.size())
+            return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, ("query " + std::to_string(first_query + i) + ": scene " + std::to_string(scene[i]) + " does not exist").c_str());
+    CUDA_TRY(e, cudaSetDevice(e->cfg.device));
+    if (int rc = join_side_stream(e)) return rc;      // an owed noise-less rollout belongs to the assignment as it was
+    std::copy(scene, scene + count, e->query_scene.begin() + first_query);
+    e->config_epoch++;
+    return upload_query_fields(e);
 }
 
 // Rows of B = L^-1 for the recurrence sampler (kernels.cuh: sample_rollouts_banded_kernel).  R = U U^T with U upper
@@ -2340,6 +2444,7 @@ int stomp_b200_iterate(stomp_b200_engine* e, int32_t iteration, const double* un
 {
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (!e->solving) return fail(e, STOMP_B200_ERR_NOT_READY, "stomp_b200_begin_solve first");
+    if (int rc = scenes_ready(e)) return rc;
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
     const size_t count = (size_t)e->Q * stomp_b200_next_num_generated(e) * e->D * e->T;
     int mode = kNoisePhilox;
@@ -2364,6 +2469,7 @@ int stomp_b200_run(stomp_b200_engine* e, int32_t first_iteration, int32_t num_it
 {
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (!e->solving) return fail(e, STOMP_B200_ERR_NOT_READY, "stomp_b200_begin_solve first");
+    if (int rc = scenes_ready(e)) return rc;
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
     // a lone iteration whose end the caller waits for: three plain launches start sooner than one graph launch (an isolated
     // C3 iteration: 88 us against 97 us); queued back to back the graph wins (57 against 61 us per iteration)
@@ -2388,6 +2494,7 @@ int stomp_b200_solve(stomp_b200_engine* e, int32_t max_iterations, int32_t poll_
 {
     if (!e || max_iterations < 0) return STOMP_B200_ERR_INVALID_ARGUMENT;
     if (!e->solving) return fail(e, STOMP_B200_ERR_NOT_READY, "stomp_b200_begin_solve first");
+    if (int rc = scenes_ready(e)) return rc;
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
     if (poll_every <= 0) poll_every = 8;
     int done = 0;
@@ -2621,7 +2728,7 @@ int stomp_b200_evaluate_states(stomp_b200_engine* e, const double* theta, int32_
                                double* state_costs, uint8_t* verdicts, uint8_t* validity)
 {
     if (!e || !theta || num_trajectories < 1 || num_steps < 1) return STOMP_B200_ERR_INVALID_ARGUMENT;
-    if (!e->have_chain || !e->have_spheres || !e->have_sdf) return fail(e, STOMP_B200_ERR_NOT_READY, "chain, spheres and SDF must be set first");
+    if (!e->have_chain || !e->have_spheres || !e->scenes[e->selected].have) return fail(e, STOMP_B200_ERR_NOT_READY, "chain, spheres and SDF must be set first");
     CUDA_TRY(e, cudaSetDevice(e->cfg.device));
     const size_t states = (size_t)num_trajectories * num_steps;
     if (states > (size_t)0x7fffff00) return fail(e, STOMP_B200_ERR_INVALID_ARGUMENT, "too many states for one call");
@@ -2635,10 +2742,10 @@ int stomp_b200_evaluate_states(stomp_b200_engine* e, const double* theta, int32_
     {
         Scope sc(e, STOMP_B200_KERNEL_COST);
         const StateKernelArgs a = trajectory_state_args(e, d_theta, num_trajectories, num_steps, d_cost, d_verdict, d_valid);
-        if (int rc = launch_state_pass(e, a, e->stream, 1, -1, sane)) return rc;
+        if (int rc = launch_state_pass(e, a, e->stream, 1, -1, sane, e->selected)) return rc;
     }
     if (e->extras_on) {
-        evaluate_extras_kernel<<<(unsigned)((states + 127) / 128), 128, 0, e->stream>>>(e->robot, e->sdf, e->extras, d_theta, num_trajectories, num_steps, d_cost);
+        evaluate_extras_kernel<<<(unsigned)((states + 127) / 128), 128, 0, e->stream>>>(e->robot, e->scenes[e->selected].sdf, e->extras, d_theta, num_trajectories, num_steps, d_cost);
         e->launch_count++;
         if (int rc = check_launch(e, "evaluate_extras_kernel")) return rc;
     }
@@ -2829,7 +2936,9 @@ int stomp_b200_synchronize(stomp_b200_engine* e)
 int32_t stomp_b200_state_kernel_kind(stomp_b200_engine* e, char* note, size_t note_capacity)
 {
     if (!e) return STOMP_B200_ERR_INVALID_ARGUMENT;
-    if (!e->have_chain || !e->have_spheres || !e->have_sdf) return fail(e, STOMP_B200_ERR_NOT_READY, "chain, spheres and SDF come first");
+    bool any_field = false;
+    for (const stomp_b200_engine::Scene& sc : e->scenes) any_field = any_field || sc.have;
+    if (!e->have_chain || !e->have_spheres || !any_field) return fail(e, STOMP_B200_ERR_NOT_READY, "chain, spheres and SDF come first");
     if (cudaSetDevice(e->cfg.device) != cudaSuccess) return fail(e, STOMP_B200_ERR_CUDA, "cudaSetDevice");
     resolve_state_kernel(e);
     if (note && note_capacity) {
@@ -2858,7 +2967,7 @@ int stomp_b200_state_kernel_source(stomp_b200_engine* e, char* buffer, size_t ca
 }
 
 // Needs no device: generates the kernel for a synthetic structure that exercises every template branch (all axis
-// kinds, fixed rotation, prismatic joint, chain restart, every zero mask, wide index) and compiles it to an
+// kinds, fixed rotation, prismatic joint, chain restart, every zero mask, wide index, field per query) and compiles it to an
 // sm_100a cubin with NVRTC.  The "does the generated code build" check of __graft_entry__.build().
 int stomp_b200_codegen_selftest(char* log, size_t log_capacity)
 {
@@ -2888,6 +2997,7 @@ int stomp_b200_codegen_selftest(char* log, size_t log_capacity)
         opt.wide_index = wide != 0;
         opt.magic_floor = wide == 0;
         opt.inside_grid = wide == 0;
+        opt.per_query_field = wide != 0;     // an engine with several scenes: each query reads its own field
         const std::string src = codegen::generate_state_kernel_source(r, opt);
         if (!codegen::compile_to_cubin(src, cubin, clog, err)) {
             all_log += err;
@@ -2897,7 +3007,8 @@ int stomp_b200_codegen_selftest(char* log, size_t log_capacity)
             const size_t at = src.find(" static spheres\n");
             const size_t from = at == std::string::npos ? at : src.rfind("// ", at);
             const std::string statics = from == std::string::npos ? std::string("no static spheres") : src.substr(from + 3, at - from - 3) + " static spheres";
-            all_log += "ok: " + std::to_string(cubin.size()) + " byte cubin (" + codegen::cache().nvrtc.where + "), " + statics + " " + clog + "\n";
+            all_log += "ok: " + std::to_string(cubin.size()) + " byte cubin (" + codegen::cache().nvrtc.where + "), " + statics +
+                       (opt.per_query_field ? ", field per query " : " ") + clog + "\n";
         }
     }
     if (rc == STOMP_B200_OK) {      // the same walk with the sphere-pair rule inside: every sphere of the first chain against every one of the second
@@ -2916,12 +3027,12 @@ int stomp_b200_codegen_selftest(char* log, size_t log_capacity)
         std::vector<char> cubin;
         std::string clog;
         codegen::StateKernelOptions opt;
-        opt.magic_floor = true; opt.inside_grid = true; opt.no_tail = true; opt.self = &sp;
+        opt.magic_floor = true; opt.inside_grid = true; opt.no_tail = true; opt.self = &sp; opt.per_query_field = true;
         if (!codegen::compile_to_cubin(codegen::generate_state_kernel_source(r, opt), cubin, clog, err)) {
             all_log += err;
             rc = STOMP_B200_ERR_CUDA;
         } else {
-            all_log += "ok (pair rule, " + std::to_string(sp.i.size()) + " pairs): " + std::to_string(cubin.size()) + " byte cubin " + clog + "\n";
+            all_log += "ok (pair rule, " + std::to_string(sp.i.size()) + " pairs, field per query): " + std::to_string(cubin.size()) + " byte cubin " + clog + "\n";
         }
     }
     if (log && log_capacity) std::snprintf(log, log_capacity, "%s", all_log.c_str());

@@ -127,6 +127,10 @@ struct LoopParams {
     // them depends on what an iteration computes.  Launched as a programmatic dependent of the weights / update kernel, that
     // part runs beside it (sample_rollouts_banded_kernel)
     int32_t early_sampler;
+    // [Q] the field of each local query's scene and [Q] its scene (StateKernelArgs::query_sdf), or null: one scene, the
+    // kernels' SdfParams argument
+    const SdfParams* query_sdf;
+    const int32_t* query_scene;
 };
 
 // the joint limits of OptimizationTask::filter: all the sampling kernels need of the robot (0.5 KB of kernel parameters
@@ -1414,13 +1418,14 @@ rollout_states_kernel(const __grid_constant__ StateKernelArgs a, const __grid_co
     if (a.tile_counter && blockIdx.x == 0 && q == 0 && threadIdx.x < 4) a.tile_counter[threadIdx.x] = 0u;   // for the next sampling launch
     if (a.honour_stop && a.stop[q] != 0) return;
     TimelineScope tls(a.timeline);
+    const SdfParams field = query_field(a.query_sdf, q, sdf);     // the field of this query's scene
     const int T = a.T;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx < a.num_gen * T) {
         const int k = idx / T, t = idx - k * T;
         const double* xq = a.rollouts + ((size_t)q * a.slots + k) * a.rollout_stride + t;
         const size_t rs = (size_t)a.row_stride;
-        const bool hit = state_collides<kSimple>(robot, sdf, [&](int d) { return xq[(size_t)d * rs]; });
+        const bool hit = state_collides<kSimple>(robot, field, [&](int d) { return xq[(size_t)d * rs]; });
         const size_t o = ((size_t)q * a.slots + k) * T + t;
         if (a.state_costs) a.state_costs[o] = hit ? 1.0 : 0.0;
         if (a.verdicts) a.verdicts[o] = hit ? 1 : 0;
@@ -1493,7 +1498,8 @@ state_cost_extras_kernel(const __grid_constant__ LoopParams p, const __grid_cons
     const int k = idx / T, t = idx - k * T;
     const double* xq = p.rollouts + ((size_t)q * p.slots + k) * D * T + t;
     const size_t o = ((size_t)q * p.slots + k) * T + t;
-    p.state_costs[o] = extra_state_cost(robot, sdf, x, [&](int d) { return xq[(size_t)d * T]; }, p.state_costs[o]);
+    const SdfParams field = query_field(p.query_sdf, q, sdf);
+    p.state_costs[o] = extra_state_cost(robot, field, x, [&](int d) { return xq[(size_t)d * T]; }, p.state_costs[o]);
 }
 
 // S_k = sum_t state_costs[k][t] of the generated rollouts, one warp per rollout, fixed order
@@ -1581,6 +1587,7 @@ states_self_collision_kernel(const __grid_constant__ StateKernelArgs a, const __
         asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t0));
         atomicMin(a.timeline, t0);
     }
+    const SdfParams field = query_field(a.query_sdf, q, sdf);     // the field of this query's scene
     const int T = a.T;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx < a.num_gen * T) {
@@ -1604,7 +1611,7 @@ states_self_collision_kernel(const __grid_constant__ StateKernelArgs a, const __
                 double cx, cy, cz;
                 sphere_centre(f, robot.sphere[s], cx, cy, cz);
                 c[3 * s] = cx; c[3 * s + 1] = cy; c[3 * s + 2] = cz;
-                const double dist = (double)__ldg(sdf.grid + sdf_index(sdf, cx, cy, cz));
+                const double dist = (double)__ldg(field.grid + sdf_index(field, cx, cy, cz));
                 hit |= (dist - robot.sphere[s].r) < 0.0;
             }
         }
@@ -2495,9 +2502,10 @@ noiseless_rollout_kernel(const __grid_constant__ LoopParams p, const __grid_cons
     for (int t = tid; t < T; t += blockDim.x) sstate[t] = p.nl_state[(size_t)q * T + t];
     __syncthreads();
     if (extras.smooth || extras.joint_constraint) {     // alternative state costs of the noise-less states (see CostExtras)
+        const SdfParams field = query_field(p.query_sdf, q, sdf);
         for (int t = tid; t < T; t += blockDim.x) {
             const double* xq = sx + kPad + t;
-            sstate[t] = extra_state_cost(robot, sdf, extras, [&](int d) { return xq[(size_t)d * N]; }, sstate[t]);
+            sstate[t] = extra_state_cost(robot, field, extras, [&](int d) { return xq[(size_t)d * N]; }, sstate[t]);
             p.nl_state[(size_t)q * T + t] = sstate[t];
         }
         __syncthreads();

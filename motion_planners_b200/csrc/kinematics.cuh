@@ -71,6 +71,15 @@ struct SdfParams {
     double inv_h;
 };
 
+// The field local query q reads: its record in the per-query table of an engine with several scenes, else the kernel's
+// SdfParams argument.  The copy goes through a pointer to the chosen record: written as `table ? table[q] : arg` (or as a
+// member-wise copy under an if) with a __grid_constant__ argument, nvcc 12.9 takes `grid` from the argument on both paths.
+__device__ __forceinline__ SdfParams query_field(const SdfParams* table, int q, const SdfParams& arg)
+{
+    const SdfParams* src = table ? table + q : &arg;
+    return *src;
+}
+
 // Deterministic sin/cos (also run on the host for the fixed rpy rotations of stomp_b200_set_chain, so
 // that the whole FK is one arithmetic): 3-term Cody-Waite reduction by pi/2, then the degree-13 / degree-14 minimax
 // polynomials on [-pi/4, pi/4] (coefficients of Sun's fdlibm kernels; mathematical constants).
@@ -404,6 +413,11 @@ struct StateKernelArgs {
     const int32_t* static_hit;
     // floor(2^32 / T) + 1 when num_gen * T * T < 2^32 (then umulhi(idx, t_magic) == idx / T for every state index), else 0
     uint32_t t_magic;
+    // an engine with several scenes (stomp_b200_set_query_scenes): [Q] the field of each local query's scene and [Q] the
+    // scene itself (static_hit then holds one verdict per scene).  Null: every query reads the SdfParams argument and
+    // static_hit is that field's verdict
+    const SdfParams* query_sdf;
+    const int32_t* query_scene;
 };
 
 }  // namespace stomp_b200

@@ -280,6 +280,8 @@ class Problem:
     movement_duration: float = 5.0
     control_cost_weight: float = 0.001
     name: str = ""
+    scenes: list = None        # [Sdf] one field per scene (sdf is scenes[0]), or None: every query plans in `sdf`
+    query_scene: np.ndarray = None   # [Q] int32 scene of each query
 
 
 def _scene(chain, spheres, configs, n, seed, blockers=(), urdf_box=True):
@@ -327,3 +329,31 @@ def batch_problem(Q=1024, K=64, T=200, sdf_n=128, seed=1234, query_seed=4321) ->
     goal = np.stack([draw() for _ in range(Q)])
     return Problem(chain, spheres, sdf, start, goal, IIWA_NOISE_STDDEV.copy(), T, K, num_queries=Q,
                    name=f"batch_Q{Q}_K{K}_T{T}_sdf{sdf_n}")
+
+
+def batch_problem_scenes(Q=1024, K=64, T=200, sdf_n=128, num_scenes=16, seed=1234, query_seed=4321) -> Problem:
+    """Config 4 over `num_scenes` worlds: scene s is the obstacle set of seed + s as a primitive list (the engine builds the
+    fields on the device), query q plans in scene q mod num_scenes, and its start and goal are drawn within the joint limits,
+    free in its own scene: every sphere at least its radius plus one voxel from every obstacle (exact primitive distances,
+    no host grid)."""
+    chain, spheres = iiwa_chain(), iiwa_spheres()
+    keep = [(sphere_centres_numpy(chain, spheres, q), spheres.radius) for q in (IIWA_START, IIWA_GOAL)]
+    scenes = [make_sdf(sdf_n, make_obstacles(seed=seed + s, keep_clear=keep), lazy=True) for s in range(num_scenes)]
+    query_scene = (np.arange(Q) % num_scenes).astype(np.int32)
+    rng = np.random.default_rng(query_seed)
+
+    def free(q, sdf):
+        c = sphere_centres_numpy(chain, spheres, q)
+        return all(np.all(_obstacle_distance(c, kind, centre, size) >= spheres.radius + sdf.voxel)
+                   for kind, centre, size in sdf.obstacles)
+
+    def draw(sdf):
+        while True:
+            q = rng.uniform(0.9 * chain.lower, 0.9 * chain.upper)
+            if free(q, sdf):
+                return q
+
+    start = np.stack([draw(scenes[s]) for s in query_scene])
+    goal = np.stack([draw(scenes[s]) for s in query_scene])
+    return Problem(chain, spheres, scenes[0], start, goal, IIWA_NOISE_STDDEV.copy(), T, K, num_queries=Q,
+                   name=f"batch_Q{Q}_K{K}_T{T}_sdf{sdf_n}_scenes{num_scenes}", scenes=scenes, query_scene=query_scene)

@@ -44,6 +44,7 @@ int main(int argc, char** argv)
     if (getenv("NOTAIL")) opt.no_tail = atoi(getenv("NOTAIL")) != 0;
     if (getenv("LANES")) opt.rollout_lanes = true;
     if (getenv("STATIC")) opt.hoist_static = atoi(getenv("STATIC")) != 0;
+    if (getenv("FIELD")) opt.per_query_field = true;      // the field of each query read from the per-query table
     codegen::SelfPairStructure sp;
     if (dual && getenv("PAIRS")) {      // the sphere-pair rule inside the kernel: every sphere of the first arm (object included) against every one of the second
         std::vector<int> link_of((size_t)s, 0);
